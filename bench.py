@@ -2,9 +2,15 @@
 """bench.py -- structure-tensor loss fwd+bwd throughput on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c2x|c5|c1] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one forward + backward pass of the fused ST loss over one batch of synthetic
 SR/HR images (the hot path of SURVEY.md section 8).  Printed: ONE JSON line.
+
+--dump-outputs DIR writes what the timed path returned in its last step -- the loss and d loss / d sr -- as
+DIR/loss.npy and DIR/d_sr.npy (float32).  The inputs are seeded, so two builds run with the same arguments
+can be compared output for output.  A gradient larger than 60 MB (--workload c2x) is written as
+DIR/d_sr_sample.npy instead: the values at a fixed, seeded set of element indices.
 
   value      images/s with inputs resident in HBM: the two kernels (forward, backward) are enqueued
              through the C ABI on one stream, K steps captured in a CUDA graph, timed with CUDA
@@ -40,6 +46,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 METRIC = "st_loss_fwd_bwd_images_per_sec"
 UNIT = "images/s"
@@ -463,7 +470,7 @@ def run_gpu(args):
     k, _ = T.gaussian_taps(2.0)
     hbm_peak, peak_src = _peaks()
 
-    def measure(wl_name, K, Wm, with_e2e):
+    def measure(wl_name, K, Wm, with_e2e, keep_last=False):
         wl = WORKLOADS[wl_name]
         B, H, W = wl["B"], wl["H"], wl["W"]
         bytes_pair = 2 * B * 3 * H * W * 4
@@ -523,11 +530,13 @@ def run_gpu(args):
         if rank == 0:
             sampler.start()
         ms_pair = min(time_graph(g_pair) for _ in range(3))
+        # what the caller of the timed path holds after its last step (step K-1, batch (K-1) % pool_n)
+        last_step = {"loss": loss.cpu().numpy(), "d_sr": d_sr.cpu().numpy()} if keep_last else None
         ms_f = min(time_graph(g_f) for _ in range(3))
         ms_b = min(time_graph(g_b) for _ in range(3))
         loss_val = float(loss.item())
         res = dict(wl=wl, ms_step=ms_pair / K, ms_fwd=ms_f / K, ms_bwd=ms_b / K, clocks=None, pool_n=pool_n,
-                   loss=loss_val, images_per_s=world * B * K / (ms_pair * 1e-3))
+                   loss=loss_val, images_per_s=world * B * K / (ms_pair * 1e-3), last_step=last_step)
         px = B * H * W
         res["roofline_fwd"] = BYTES_FWD * px / (res["ms_fwd"] * 1e-3) / 1e9
         res["roofline_bwd"] = BYTES_BWD * px / (res["ms_bwd"] * 1e-3) / 1e9
@@ -664,7 +673,9 @@ def run_gpu(args):
         return res
 
     K, Wm = args.steps, args.warmup
-    main = measure(args.workload, K, Wm, with_e2e=True)
+    main = measure(args.workload, K, Wm, with_e2e=True, keep_last=args.dump_outputs is not None)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, main["last_step"])
     others = {}
     if not args.no_extra:
         for name in WORKLOADS:
@@ -872,7 +883,13 @@ def main():
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary workloads")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and d_sr of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
     if args.gpus > 1 and "RANK" not in os.environ and args.impl != "reference":
         # convenience: re-launch under torchrun on one node
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",
@@ -890,6 +907,20 @@ def main():
 
 
 _RESULT_FD = None
+DUMP_ARRAY_BYTES = 60 << 20   # per array; loss + d_sr stay within 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Write each array as path/<name>.npy (float32); one larger than DUMP_ARRAY_BYTES is written as
+    path/<name>_sample.npy, its values at a fixed, seeded, sorted set of flat indices."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_ARRAY_BYTES // 4, replace=False))
+            a, name = a.reshape(-1)[idx], name + "_sample"
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def emit(obj):
