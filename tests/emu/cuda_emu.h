@@ -44,10 +44,23 @@ static inline cudaError_t cudaPeekAtLastError() { return 0; }
 #define __restrict__ __restrict
 #define __launch_bounds__(...)
 #define __grid_constant__
+// Static __shared__ arrays become function-local statics of the kernels.  tests/emu/shared.ld (with -fdata-sections)
+// gathers every local static of a function named *_kernel into one range, so that launch() can poison them before
+// every block, like dynamic shared memory: a kernel that reads a static array it did not write in the same block sees
+// the poison instead of the previous block's (finite, plausible) values.  (g++ ignores a section attribute on a local
+// static of a function template, hence the linker script.)
 #define __shared__ static
 #define __align__(n) __attribute__((aligned(n)))
 
+// Bounds of that range (set by shared.ld; both null when the library was linked without it).
+extern "C" unsigned char __start_srst_emu_shared[] __attribute__((weak, visibility("hidden")));
+extern "C" unsigned char __stop_srst_emu_shared[] __attribute__((weak, visibility("hidden")));
+
 namespace emu {
+// Byte that fills dynamic and static shared memory before every block.  0xCD (the float -4.3e8) by default; 0xFF
+// makes every float a NaN and every int -1, so that a read of never-written shared memory cannot hide behind a
+// zero weight.  Set through srst_emu_set_poison().
+inline int g_smem_poison = 0xCD;
 struct BlockCtx {
   std::unique_ptr<std::barrier<>> bar;
   std::vector<std::unique_ptr<std::barrier<>>> warp_bar;
@@ -88,7 +101,9 @@ void launch(dim3 grid, dim3 block, size_t smem_bytes, F&& body) {
           ctx.warp_bar.emplace_back(std::make_unique<std::barrier<>>(lanes));
         }
         ctx.warp_xchg.assign(32 * nwarps, 0);
-        std::memset(smem_aligned, 0xCD, smem_bytes);  // poison: uninitialised reads become visible
+        std::memset(smem_aligned, g_smem_poison, smem_bytes);  // poison: uninitialised reads become visible
+        if (__start_srst_emu_shared && __stop_srst_emu_shared > __start_srst_emu_shared)
+          std::memset(__start_srst_emu_shared, g_smem_poison, __stop_srst_emu_shared - __start_srst_emu_shared);
         ctx.dyn_smem = smem_aligned;
         g_block = &ctx;
         std::vector<std::thread> ths;
@@ -135,6 +150,14 @@ inline unsigned warp_ballot(bool pred) {
   return mask;
 }
 }  // namespace emu
+
+// Test hook exported by the emulation library only (the header is compiled into exactly one translation unit):
+// the shared-memory poison byte of later launches; returns the previous one.
+extern "C" __attribute__((visibility("default"))) int srst_emu_set_poison(int byte) {
+  const int old = emu::g_smem_poison;
+  emu::g_smem_poison = byte & 0xFF;
+  return old;
+}
 
 #define threadIdx (emu::t_threadIdx)
 #define blockIdx (emu::t_blockIdx)

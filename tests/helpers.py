@@ -40,15 +40,33 @@ def emu_lib():
     libsrst.so compiled with g++ -DSRST_EMULATE; it lets the CPU suite execute the kernels' index
     logic.  The product package never loads this."""
     from srgan_st_b200 import _cabi
-    srcs = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(EMU_DIR, "cuda_emu.h"),
+    ld = os.path.join(EMU_DIR, "shared.ld")   # gathers the kernels' static __shared__ arrays for the poison fill
+    srcs = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(EMU_DIR, "cuda_emu.h"), ld,
                                                                 os.path.join(ROOT, "include", "srst.h")]
     stale = (not os.path.exists(EMU_LIB)) or any(os.path.getmtime(s) > os.path.getmtime(EMU_LIB) for s in srcs)
     if stale:
         os.makedirs(os.path.dirname(EMU_LIB), exist_ok=True)
-        cmd = ["g++", "-x", "c++", "-std=c++20", "-O2", "-DSRST_EMULATE", "-I" + EMU_DIR, "-I" + CSRC,
-               "-shared", "-fPIC", "-pthread", "-o", EMU_LIB, os.path.join(CSRC, "srst_cabi.cu")]
+        cmd = ["g++", "-x", "c++", "-std=c++20", "-O2", "-DSRST_EMULATE", "-fdata-sections", "-I" + EMU_DIR, "-I" + CSRC,
+               "-shared", "-fPIC", "-pthread", "-Wl,-T," + ld, "-o", EMU_LIB, os.path.join(CSRC, "srst_cabi.cu")]
         subprocess.run(cmd, check=True, capture_output=True)
-    return _cabi.bind(EMU_LIB)
+    lib = _cabi.bind(EMU_LIB)
+    lib.srst_emu_set_poison.restype = ctypes.c_int
+    lib.srst_emu_set_poison.argtypes = [ctypes.c_int]
+    return lib
+
+
+# Fill of the workspaces the emu_* helpers below hand to the kernels: None = all zeros; a byte value = that byte
+# everywhere but the 16-byte ticket header, which is all srst.h promises to be zero (tests/test_emu_poison.py).
+WORKSPACE_FILL = None
+FILLED_WORKSPACES = []   # every workspace filled that way, for checks that the ticket header came back zeroed
+
+
+def _workspace(nbytes):
+    ws = np.zeros(nbytes // 4 + 4, np.float32)
+    if WORKSPACE_FILL is not None:
+        ws.view(np.uint8)[16:] = WORKSPACE_FILL
+        FILLED_WORKSPACES.append(ws)
+    return ws
 
 
 def _p(a):
@@ -69,7 +87,7 @@ def emu_st(lib, sr, hr, taps, normalize=True, want_hr=False, grad_out=1.0):
     generic = lib.srst_st_supported(rs, rk) == 2   # radii beyond the compiled classes: scratch planes in the workspace
     nb = lib.srst_st_workspace_bytes_r(B, H, W, rs, rk)
     assert nb >= lib.srst_st_workspace_bytes(B, H, W) and (generic or nb == lib.srst_st_workspace_bytes(B, H, W))
-    ws = np.zeros(nb // 4 + 4, np.float32)
+    ws = _workspace(nb)
     nbb = lib.srst_st_backward_workspace_bytes(B, H, W, rs, rk)
     assert (nbb > 0) == generic
     bws = np.full(nbb // 4 + 4, np.nan, np.float32)
@@ -115,7 +133,7 @@ def emu_bb(lib, sr, gt, gt2=None, gt4=None, alpha=1.0, beta=1.0, criterion=0, gr
     B, _, H, W = sr.shape
     N = (H // 3) * (W // 3)
     nb = lib.srst_bb_workspace_bytes(B, H, W)
-    ws = np.zeros(nb // 4 + 4, np.float32)
+    ws = _workspace(nb)
     idx = np.full((B, N), -1, np.int64)
     loss = np.zeros(1, np.float32)
     go = np.full(1, grad_out, np.float32)
@@ -146,7 +164,7 @@ def emu_stpx(lib, sr, hr, taps, grad_st=1.0, grad_px=1.0):
     B, _, H, W = sr.shape
     g, dg, k = [np.ascontiguousarray(t, np.float32) for t in taps]
     nb = lib.srst_st_workspace_bytes(B, H, W)
-    ws = np.zeros(nb // 4 + 4, np.float32)
+    ws = _workspace(nb)
     both = np.zeros(2, np.float32)
     ds_sr = np.full_like(sr, np.nan)
     ixy_sr = np.full(lib.srst_st_ixy_floats(B, H, W), np.nan, np.float32)
@@ -170,7 +188,7 @@ def emu_patch_gt(lib, sr, gt, idx, gt2=None, gt4=None, criterion=0, grad_out=1.0
     idx = np.ascontiguousarray(idx, np.int64)
     B, _, H, W = sr.shape
     nb = lib.srst_bb_workspace_bytes(B, H, W)
-    ws = np.zeros(nb // 4 + 4, np.float32)
+    ws = _workspace(nb)
     go = np.full(1, grad_out, np.float32)
     d_gt = np.full_like(gt, np.nan)
     if taps is not None:
@@ -195,7 +213,7 @@ def emu_bbg(lib, sr, gt, ksize, pad, stride, gt2=None, gt4=None, alpha=1.0, beta
     N = lib.srst_bbg_num_patches(H, W, ksize, pad, stride)
     nb = lib.srst_bbg_workspace_bytes(B, H, W, ksize, pad, stride)
     assert N > 0 and nb > 0
-    ws = np.zeros(nb // 4 + 4, np.float32)
+    ws = _workspace(nb)
     idx = np.full((B, N), -1, np.int64)
     loss = np.zeros(1, np.float32)
     go = np.full(1, grad_out, np.float32)
