@@ -694,27 +694,54 @@ int srst_bb_pyramid(const float* gt, int B, int H, int W, float* out2, float* ou
 
 }  // extern "C"
 
+// Splits the search norm off `criterion` (dist_norm, utils.py:166-172; the backward entry points ignore it): what is
+// left must be L1 or L2.
+static int bb_criterion(int& criterion, bool& dist_l1) {
+  dist_l1 = (criterion & SRST_BB_DIST_L1) != 0;
+  criterion &= ~SRST_BB_DIST_L1;
+  return (criterion == SRST_BB_L1 || criterion == SRST_BB_L2) ? 0 : SRST_E_INVALID;
+}
+
+// Arguments of the default-geometry patch entry points, after their NULL / B <= 0 check: criterion, shape, then the
+// gt2 / gt4 pairing.
+static int bb_check(int& criterion, bool& dist_l1, int B, int H, int W, const float* gt2, const float* gt4) {
+  if (const int e = bb_criterion(criterion, dist_l1)) return e;
+  if (H < 12 || W < 12 || B > 65535) return SRST_E_SHAPE;
+  return (gt2 == nullptr) != (gt4 == nullptr) ? SRST_E_INVALID : 0;
+}
+
+// The caller's coarse levels of gt, or the library's own built into pyr2 / pyr4 (workspace).
+static int bb_levels(const float* gt, const BbGeom& g, const float*& gt2, const float*& gt4, float* pyr2, float* pyr4,
+                     void* stream) {
+  if (gt2) return 0;
+  gt2 = pyr2;
+  gt4 = pyr4;
+  return bb_launch_pyramid(gt, g, pyr2, pyr4, stream);
+}
+
+static int zero_fill(float* p, size_t n, void* stream) {
+#ifdef SRST_EMULATE
+  std::memset(p, 0, sizeof(float) * n);
+  return 0;
+#else
+  return (int)cudaMemsetAsync(p, 0, sizeof(float) * n, (cudaStream_t)stream);
+#endif
+}
+
 template <int MODE>
 static int bb_forward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W,
                            float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out, void* workspace,
                            size_t workspace_bytes, void* stream, const PstTaps& tp = PstTaps{}) {
   constexpr int D = BbDesc<MODE>::D;
   if (!sr || !gt || !idx_out || !loss_out || B <= 0) return SRST_E_INVALID;
-  const bool dist_l1 = (criterion & SRST_BB_DIST_L1) != 0;  // dist_norm of the search (utils.py:166-172)
-  criterion &= ~SRST_BB_DIST_L1;
-  if (criterion != SRST_BB_L1 && criterion != SRST_BB_L2) return SRST_E_INVALID;
-  if (H < 12 || W < 12 || B > 65535) return SRST_E_SHAPE;
-  if ((gt2 == nullptr) != (gt4 == nullptr)) return SRST_E_INVALID;
+  bool dist_l1;
+  int e = bb_check(criterion, dist_l1, B, H, W, gt2, gt4);
+  if (e) return e;
   const BbGeom g = bb_geom(B, H, W);
   if (!workspace || !aligned16(workspace)) return SRST_E_WORKSPACE;
   const BbWorkspace w = bb_carve(workspace, g, D);
   if (workspace_bytes < w.total_bytes) return SRST_E_WORKSPACE;
-  int e;
-  if (!gt2) {
-    if ((e = bb_launch_pyramid(gt, g, w.pyr2, w.pyr4, stream)) != 0) return e;
-    gt2 = w.pyr2;
-    gt4 = w.pyr4;
-  }
+  if ((e = bb_levels(gt, g, gt2, gt4, w.pyr2, w.pyr4, stream)) != 0) return e;
   const int npack = g.Npad > g.Mpad ? g.Npad : g.Mpad;
   SRST_LAUNCH(bb_pack_kernel<MODE>, dim3((npack + 255) / 256, B), dim3(256), 0, stream, sr, gt, gt2, gt4, w.mats,
               w.per_image, g, tp);
@@ -769,6 +796,38 @@ static int pst_taps(const float* g, const float* dg, int r_sigma, const float* k
   return 0;
 }
 
+template <int MODE>
+static int patch_backward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
+                               const float* grad_out, int B, int H, int W, int criterion, float* d_sr, void* workspace,
+                               size_t workspace_bytes, void* stream, const PstTaps& tp = PstTaps{}) {
+  if (!sr || !gt || !idx || !grad_out || !d_sr || B <= 0) return SRST_E_INVALID;
+  bool dist_l1;
+  int e = bb_check(criterion, dist_l1, B, H, W, gt2, gt4);
+  if (e) return e;
+  const BbGeom g = bb_geom(B, H, W);
+  if (!gt2) {  // the workspace only has to hold the library's own pyramid levels
+    if (!workspace || !aligned16(workspace)) return SRST_E_WORKSPACE;
+    const BbWorkspace w = bb_carve(workspace, g);
+    if (workspace_bytes < w.total_bytes) return SRST_E_WORKSPACE;
+    if ((e = bb_levels(gt, g, gt2, gt4, w.pyr2, w.pyr4, stream)) != 0) return e;
+  }
+  if constexpr (MODE == 0) {  // one thread per pixel of d_sr
+    const size_t total = (size_t)B * 3 * H * W;
+    SRST_LAUNCH(bb_backward_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
+                grad_out, g, criterion, d_sr);
+  } else {  // one thread per patch: pixels outside every patch keep a zero gradient
+    if ((H % 3 != 0 || W % 3 != 0) && (e = zero_fill(d_sr, (size_t)B * 3 * H * W, stream)) != 0) return e;
+    const size_t total = (size_t)B * g.N;
+    if constexpr (MODE == 1)
+      SRST_LAUNCH(gram_backward_kernel<false>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4,
+                  idx, grad_out, g, criterion, d_sr, nullptr, nullptr);
+    else
+      SRST_LAUNCH(pst_backward_kernel<false>, dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt, gt2, gt4,
+                  idx, grad_out, g, tp, criterion, d_sr, nullptr, nullptr);
+  }
+  return (int)cudaGetLastError();
+}
+
 extern "C" {
 
 int srst_pst_forward(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W,
@@ -782,69 +841,29 @@ int srst_pst_forward(const float* sr, const float* gt, const float* gt2, const f
                             workspace_bytes, stream, tp);
 }
 
-int srst_pst_backward(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
-                      const float* grad_out, int B, int H, int W, const float* g, const float* dg, int r_sigma,
-                      const float* k, int r_rho, int criterion, float* d_sr, void* workspace, size_t workspace_bytes,
-                      void* stream) {
-  if (!sr || !gt || !idx || !grad_out || !d_sr || B <= 0) return SRST_E_INVALID;
-  criterion &= ~SRST_BB_DIST_L1;  // the search norm does not matter to the backward
-  if (criterion != SRST_BB_L1 && criterion != SRST_BB_L2) return SRST_E_INVALID;
-  if (H < 12 || W < 12 || B > 65535) return SRST_E_SHAPE;
-  if ((gt2 == nullptr) != (gt4 == nullptr)) return SRST_E_INVALID;
-  PstTaps tp;
-  int e = pst_taps(g, dg, r_sigma, k, r_rho, tp);
-  if (e) return e;
-  const BbGeom gm = bb_geom(B, H, W);
-  if (!gt2) {
-    if (!workspace || !aligned16(workspace)) return SRST_E_WORKSPACE;
-    const BbWorkspace w = bb_carve(workspace, gm);
-    if (workspace_bytes < w.total_bytes) return SRST_E_WORKSPACE;
-    if ((e = bb_launch_pyramid(gt, gm, w.pyr2, w.pyr4, stream)) != 0) return e;
-    gt2 = w.pyr2;
-    gt4 = w.pyr4;
-  }
-  if (H % 3 != 0 || W % 3 != 0) {  // pixels outside every patch keep a zero gradient
-#ifdef SRST_EMULATE
-    std::memset(d_sr, 0, sizeof(float) * (size_t)B * 3 * H * W);
-#else
-    if ((e = (int)cudaMemsetAsync(d_sr, 0, sizeof(float) * (size_t)B * 3 * H * W, (cudaStream_t)stream)) != 0) return e;
-#endif
-  }
-  const size_t total = (size_t)B * gm.N;
-  SRST_LAUNCH(pst_backward_kernel<false>, dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt, gt2, gt4, idx,
-              grad_out, gm, tp, criterion, d_sr, nullptr, nullptr);
-  return (int)cudaGetLastError();
+int srst_bb_backward(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
+                     const float* grad_out, int B, int H, int W, int criterion, float* d_sr, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+  return patch_backward_impl<0>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace, workspace_bytes,
+                                stream);
 }
 
 int srst_gram_backward(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
                        const float* grad_out, int B, int H, int W, int criterion, float* d_sr, void* workspace,
                        size_t workspace_bytes, void* stream) {
-  if (!sr || !gt || !idx || !grad_out || !d_sr || B <= 0) return SRST_E_INVALID;
-  criterion &= ~SRST_BB_DIST_L1;  // the search norm does not matter to the backward
-  if (criterion != SRST_BB_L1 && criterion != SRST_BB_L2) return SRST_E_INVALID;
-  if (H < 12 || W < 12 || B > 65535) return SRST_E_SHAPE;
-  if ((gt2 == nullptr) != (gt4 == nullptr)) return SRST_E_INVALID;
-  const BbGeom g = bb_geom(B, H, W);
-  int e;
-  if (!gt2) {
-    if (!workspace || !aligned16(workspace)) return SRST_E_WORKSPACE;
-    const BbWorkspace w = bb_carve(workspace, g);
-    if (workspace_bytes < w.total_bytes) return SRST_E_WORKSPACE;
-    if ((e = bb_launch_pyramid(gt, g, w.pyr2, w.pyr4, stream)) != 0) return e;
-    gt2 = w.pyr2;
-    gt4 = w.pyr4;
-  }
-  if (H % 3 != 0 || W % 3 != 0) {  // pixels outside every patch keep a zero gradient
-#ifdef SRST_EMULATE
-    std::memset(d_sr, 0, sizeof(float) * (size_t)B * 3 * H * W);
-#else
-    if ((e = (int)cudaMemsetAsync(d_sr, 0, sizeof(float) * (size_t)B * 3 * H * W, (cudaStream_t)stream)) != 0) return e;
-#endif
-  }
-  const size_t total = (size_t)B * g.N;
-  SRST_LAUNCH(gram_backward_kernel<false>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
-              grad_out, g, criterion, d_sr, nullptr, nullptr);
-  return (int)cudaGetLastError();
+  return patch_backward_impl<1>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace, workspace_bytes,
+                                stream);
+}
+
+int srst_pst_backward(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
+                      const float* grad_out, int B, int H, int W, const float* g, const float* dg, int r_sigma,
+                      const float* k, int r_rho, int criterion, float* d_sr, void* workspace, size_t workspace_bytes,
+                      void* stream) {
+  PstTaps tp;
+  const int e = pst_taps(g, dg, r_sigma, k, r_rho, tp);
+  if (e) return e;
+  return patch_backward_impl<2>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace, workspace_bytes,
+                                stream, tp);
 }
 
 int srst_patch_backward_gt(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
@@ -852,25 +871,16 @@ int srst_patch_backward_gt(int mode, const float* sr, const float* gt, const flo
                            int r_sigma, const float* k, int r_rho, int criterion, float* d_gt, void* workspace,
                            size_t workspace_bytes, void* stream) {
   if (!sr || !gt || !idx || !grad_out || !d_gt || B <= 0 || mode < 0 || mode > 2) return SRST_E_INVALID;
-  criterion &= ~SRST_BB_DIST_L1;  // the search norm does not matter to the backward
-  if (criterion != SRST_BB_L1 && criterion != SRST_BB_L2) return SRST_E_INVALID;
-  if (H < 12 || W < 12 || B > 65535) return SRST_E_SHAPE;
-  if ((gt2 == nullptr) != (gt4 == nullptr)) return SRST_E_INVALID;
+  bool dist_l1;
+  int e = bb_check(criterion, dist_l1, B, H, W, gt2, gt4);
+  if (e) return e;
   PstTaps tp = {};
-  int e;
-  if (mode == 2) {
-    if (!g || !dg || !k) return SRST_E_INVALID;
-    if ((e = pst_taps(g, dg, r_sigma, k, r_rho, tp)) != 0) return e;
-  }
+  if (mode == 2 && (e = pst_taps(g, dg, r_sigma, k, r_rho, tp)) != 0) return e;
   const BbGeom gm = bb_geom(B, H, W);
   if (!workspace || !aligned16(workspace)) return SRST_E_WORKSPACE;
   const BbWorkspace w = bb_carve(workspace, gm);
   if (workspace_bytes < w.total_bytes) return SRST_E_WORKSPACE;
-  if (!gt2) {
-    if ((e = bb_launch_pyramid(gt, gm, w.pyr2, w.pyr4, stream)) != 0) return e;
-    gt2 = w.pyr2;
-    gt4 = w.pyr4;
-  }
+  if ((e = bb_levels(gt, gm, gt2, gt4, w.pyr2, w.pyr4, stream)) != 0) return e;
   // gradient images of the two coarse levels: in the descriptor-matrix region of the workspace (dead after the forward)
   const size_t n0 = (size_t)B * 3 * H * W, n2 = (size_t)B * 3 * gm.H2 * gm.W2, n4 = (size_t)B * 3 * gm.H4 * gm.W4;
   float* d2 = w.mats;
@@ -893,30 +903,6 @@ int srst_patch_backward_gt(int mode, const float* sr, const float* gt, const flo
   return (int)cudaGetLastError();
 }
 
-int srst_bb_backward(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
-                     const float* grad_out, int B, int H, int W, int criterion, float* d_sr, void* workspace,
-                     size_t workspace_bytes, void* stream) {
-  if (!sr || !gt || !idx || !grad_out || !d_sr || B <= 0) return SRST_E_INVALID;
-  criterion &= ~SRST_BB_DIST_L1;  // the search norm does not matter to the backward
-  if (criterion != SRST_BB_L1 && criterion != SRST_BB_L2) return SRST_E_INVALID;
-  if (H < 12 || W < 12 || B > 65535) return SRST_E_SHAPE;
-  if ((gt2 == nullptr) != (gt4 == nullptr)) return SRST_E_INVALID;
-  const BbGeom g = bb_geom(B, H, W);
-  int e;
-  if (!gt2) {
-    if (!workspace || !aligned16(workspace)) return SRST_E_WORKSPACE;
-    const BbWorkspace w = bb_carve(workspace, g);
-    if (workspace_bytes < w.total_bytes) return SRST_E_WORKSPACE;
-    if ((e = bb_launch_pyramid(gt, g, w.pyr2, w.pyr4, stream)) != 0) return e;
-    gt2 = w.pyr2;
-    gt4 = w.pyr4;
-  }
-  const size_t total = (size_t)B * 3 * H * W;
-  SRST_LAUNCH(bb_backward_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
-              grad_out, g, criterion, d_sr);
-  return (int)cudaGetLastError();
-}
-
 }  // extern "C"
 
 // ---- Best-Buddy loss, arbitrary patch geometry (bb_generic.cuh) -----------------------------------------------
@@ -926,13 +912,7 @@ static int bbg_prepare(const float* gt, const float*& gt2, const float*& gt4, in
   w = bbg_carve(workspace, g);
   if (workspace_bytes < w.total_bytes) return SRST_E_WORKSPACE;
   if ((gt2 == nullptr) != (gt4 == nullptr)) return SRST_E_INVALID;
-  if (!gt2) {
-    const int e = bb_launch_pyramid(gt, bb_geom(B, H, W), w.pyr2, w.pyr4, stream);
-    if (e) return e;
-    gt2 = w.pyr2;
-    gt4 = w.pyr4;
-  }
-  return 0;
+  return bb_levels(gt, bb_geom(B, H, W), gt2, gt4, w.pyr2, w.pyr4, stream);
 }
 
 extern "C" {
@@ -955,15 +935,14 @@ int srst_bbg_forward(const float* sr, const float* gt, const float* gt2, const f
                      int pad, int stride, float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out,
                      void* workspace, size_t workspace_bytes, void* stream) {
   if (!sr || !gt || !idx_out || !loss_out || B <= 0) return SRST_E_INVALID;
-  const int dist_l1 = (criterion & SRST_BB_DIST_L1) ? 1 : 0;
-  criterion &= ~SRST_BB_DIST_L1;
-  if (criterion != SRST_BB_L1 && criterion != SRST_BB_L2) return SRST_E_INVALID;
+  bool dist_l1;
+  int e = bb_criterion(criterion, dist_l1);
+  if (e) return e;
   if (!srst_bbg_supported(ksize, pad, stride)) return SRST_E_UNSUPPORTED;
   if (!bbg_geom_ok(B, H, W, ksize, pad, stride)) return SRST_E_SHAPE;
   const BbgGeom g = bbg_geom(B, H, W, ksize, pad, stride);
   BbgWorkspace w;
-  int e = bbg_prepare(gt, gt2, gt4, B, H, W, g, workspace, workspace_bytes, w, stream);
-  if (e) return e;
+  if ((e = bbg_prepare(gt, gt2, gt4, B, H, W, g, workspace, workspace_bytes, w, stream)) != 0) return e;
   struct BbgSearchTag {};
   const size_t dyn = bbg_search_smem(3 * BBG_MAXK * BBG_MAXK);  // one opt-in covers every ksize
   if ((e = ensure_smem<BbgSearchTag>(bbg_search_kernel, dyn)) != 0) return e;
@@ -971,7 +950,7 @@ int srst_bbg_forward(const float* sr, const float* gt, const float* gt2, const f
               w.ymat, w.y_per_image, w.Mpad);
   if ((e = (int)cudaGetLastError()) != 0) return e;
   SRST_LAUNCH(bbg_search_kernel, dim3((unsigned)((g.N + BBG_QT - 1) / BBG_QT), (unsigned)B), dim3(BBG_NT),
-              bbg_search_smem(g.D), stream, sr, gt, w.ymat, w.y_per_image, w.Mpad, g, alpha, beta, dist_l1, idx_out);
+              bbg_search_smem(g.D), stream, sr, gt, w.ymat, w.y_per_image, w.Mpad, g, alpha, beta, dist_l1 ? 1 : 0, idx_out);
   if ((e = (int)cudaGetLastError()) != 0) return e;
   const unsigned nl = (unsigned)(((size_t)B * g.N + BBG_NT - 1) / BBG_NT);
   SRST_LAUNCH(bbg_loss_kernel, dim3(nl), dim3(BBG_NT), 0, stream, sr, gt, gt2, gt4, g, idx_out, criterion, w.partials,
@@ -983,14 +962,14 @@ int srst_bbg_backward(const float* sr, const float* gt, const float* gt2, const 
                       const float* grad_out, int B, int H, int W, int ksize, int pad, int stride, int criterion,
                       float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
   if (!sr || !gt || !idx || !grad_out || (!d_sr && !d_gt) || B <= 0) return SRST_E_INVALID;
-  criterion &= ~SRST_BB_DIST_L1;  // the search norm does not matter to the backward
-  if (criterion != SRST_BB_L1 && criterion != SRST_BB_L2) return SRST_E_INVALID;
+  bool dist_l1;
+  int e = bb_criterion(criterion, dist_l1);
+  if (e) return e;
   if (!srst_bbg_supported(ksize, pad, stride)) return SRST_E_UNSUPPORTED;
   if (!bbg_geom_ok(B, H, W, ksize, pad, stride)) return SRST_E_SHAPE;
   const BbgGeom g = bbg_geom(B, H, W, ksize, pad, stride);
   BbgWorkspace w;
-  int e = bbg_prepare(gt, gt2, gt4, B, H, W, g, workspace, workspace_bytes, w, stream);
-  if (e) return e;
+  if ((e = bbg_prepare(gt, gt2, gt4, B, H, W, g, workspace, workspace_bytes, w, stream)) != 0) return e;
   const size_t n0 = (size_t)B * 3 * H * W;
   if (d_sr) {
     SRST_LAUNCH(bbg_backward_kernel, dim3((unsigned)((n0 + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,

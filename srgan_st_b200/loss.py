@@ -338,150 +338,139 @@ class StructureTensorPixelLoss(nn.Module):
                 f"pixel_weight={self.pixel_weight}")
 
 
-def _patch_backward_gt(mode: int, sr, gt, gt2, gt4, idx, grad_out, taps, criterion: int, stream: int):
-    """d loss / d gt of a patch loss (include/srst.h, srst_patch_backward_gt): the reference's gather of the selected
-    candidates is differentiable in p2_cat (loss.py:136-139), so a gt that requires grad gets one."""
-    lib = _cabi.lib()
+def _hr_pyramid(gt, pyramid: str):
+    """(gt2, gt4), the x1/2 and x1/4 HR levels of the patch losses: the reference's own op for "aten" (loss.py:123,127,
+    :353,356); None, None for "fused", where libsrst builds them (srst_bb_pyramid taps)."""
+    if pyramid != "aten":
+        return None, None
+    with torch.no_grad():
+        return tuple(torch.nn.functional.interpolate(gt, scale_factor=s, mode="bicubic", align_corners=False).contiguous()
+                     for s in (0.5, 0.25))
+
+
+_PST_TAPS: Dict[Tuple[float, float], tuple] = {}
+
+
+def _pst_taps(sigma: float, rho: float):
+    """(g*, dg*, r_sigma, k*, r_rho, arrays) of PatchwiseStructureTensorLoss as ready-made ctypes arguments, cached per
+    (sigma, rho).  No radius limit as in _st_taps: a 3x3 patch image only sees the five central taps, and the PST entry
+    points take radii up to 4096."""
+    key = (float(sigma), float(rho))
+    t = _PST_TAPS.get(key)
+    if t is None:
+        g, dg = _taps.gaussian_taps(key[0])
+        k, _ = _taps.gaussian_taps(key[1])
+        t = (_taps.as_c(g), _taps.as_c(dg), len(g) // 2, _taps.as_c(k), len(k) // 2, (g, dg, k))  # keep the arrays alive
+        _PST_TAPS[key] = t
+    return t
+
+
+_NO_TAPS = (None, None, 0, None, 0)
+
+
+def _patch_backward_gt(mode: int, sr, gt, gt2, gt4, idx, grad_out, taps, criterion: int, d_gt, ws, stream: int):
+    """d loss / d gt of a default-geometry patch loss (include/srst.h, srst_patch_backward_gt): the reference's gather of
+    the selected candidates is differentiable in p2_cat (loss.py:136-139), so a gt that requires grad gets one."""
     B, _, H, W = sr.shape
-    d_gt = torch.empty_like(gt)
-    ws = _workspace("bb", sr.device, stream, lib.srst_bb_workspace_bytes(B, H, W))
-    if taps is not None:
-        g, dg, k = taps
-        tp = (_taps.as_c(g), _taps.as_c(dg), len(g) // 2, _taps.as_c(k), len(k) // 2)
-    else:
-        tp = (None, None, 0, None, 0)
-    rc = lib.srst_patch_backward_gt(mode, _ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H, W,
-                                    *tp, criterion, _ptr(d_gt), _ptr(ws), ws.numel(), stream)
+    rc = _cabi.lib().srst_patch_backward_gt(mode, _ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H,
+                                            W, *taps[:5], criterion, _ptr(d_gt), _ptr(ws), ws.numel(), stream)
     _cabi.check(rc, "srst_patch_backward_gt")
-    return d_gt
 
 
-class _BestBuddyLossFn(torch.autograd.Function):
-    """autograd boundary of the Best-Buddy loss.  Only the final criterion is differentiable: w.r.t. the SR patches
-    and, through the gather of the selected candidates, w.r.t. gt (reference loss.py:135-139); the argmin is not."""
+class _PatchLossFn(torch.autograd.Function):
+    """autograd boundary of the three patch losses.  Only the final criterion is differentiable: w.r.t. the SR patches
+    and, through the gather of the selected candidates, w.r.t. gt (reference loss.py:135-139, :219-222, :369-371); the
+    argmin is not.  `loss_cls` is the module class: its _plan / _fwd / _bwd make the C ABI calls that differ per loss.
+    `args` holds what they take from the module (weights, criterion, taps, geometry), fixed at forward time: a module
+    changed between forward and backward does not change the gradient."""
 
     @staticmethod
-    def forward(ctx, sr, gt, alpha, beta, criterion, pyramid, mode="patch"):
-        lib = _cabi.lib()
-        fwd = lib.srst_bb_forward if mode == "patch" else lib.srst_gram_forward
+    def forward(ctx, sr, gt, loss_cls, args, pyramid):
         sr = sr.contiguous()
         gt = gt.contiguous()
         B, _, H, W = sr.shape
+        n, kind, nbytes = loss_cls._plan(args, B, H, W)
+        with _on_device(sr.device):
+            stream = _raw_stream(sr.device)
+            gt2, gt4 = _hr_pyramid(gt, pyramid)
+            idx = torch.empty((B, n), dtype=torch.int64, device=sr.device)
+            loss = torch.empty((), dtype=torch.float32, device=sr.device)
+            loss_cls._fwd(args, sr, gt, gt2, gt4, idx, loss, _workspace(kind, sr.device, stream, nbytes), stream)
+        ctx.save_for_backward(sr, gt, gt2, gt4, idx)
+        ctx.meta = (loss_cls, args, kind, nbytes)
+        ctx.mark_non_differentiable(idx)
+        return loss, idx
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out, _grad_idx):
+        need_sr, need_gt = ctx.needs_input_grad[:2]
+        if not (need_sr or need_gt):
+            return None, None, None, None, None
+        sr, gt, gt2, gt4, idx = ctx.saved_tensors
+        loss_cls, args, kind, nbytes = ctx.meta
+        grad_out = grad_out.to(torch.float32).contiguous()
+        with _on_device(sr.device):
+            stream = _raw_stream(sr.device)
+            d_sr = torch.empty_like(sr) if need_sr else None
+            d_gt = torch.empty_like(gt) if need_gt else None
+            loss_cls._bwd(args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, _workspace(kind, sr.device, stream, nbytes),
+                          stream)
+        return d_sr, d_gt, None, None, None
+
+
+class _PatchLoss(nn.Module):
+    """What BestBuddyLoss, GramLoss and PatchwiseStructureTensorLoss share: the reference's constructor arguments
+    `alpha`, `beta`, `ksize`, `dist_norm`, `criterion` and the `pyramid` choice, the call through _PatchLossFn, and
+    ``last_indices``, the argmin indices ``[B,N]`` (int64) of the most recent call.  A subclass supplies the C ABI calls
+    (_args, _fwd, _bwd) and checks its patch geometry (_check_geometry)."""
+
+    _criterion_error = "%s criterion has not been implmented."   # the reference's message (loss.py:113, :178)
+
+    def __init__(self, alpha, beta, ksize, dist_norm, criterion, pyramid, pad=0, stride=3):
+        super().__init__()
+        self.alpha = alpha
+        self.beta = beta
+        self.ksize = ksize
+        self.dist_norm = dist_norm
+        if criterion == "l1":
+            self.criterion = torch.nn.L1Loss()   # kept for repr/config parity (config.py:133-139)
+            self._crit = 0
+        elif criterion == "l2" or criterion == "mse":
+            self.criterion = torch.nn.MSELoss()
+            self._crit = 1
+        else:
+            raise NotImplementedError(self._criterion_error % criterion)
+        if dist_norm not in ("l1", "l2"):
+            raise NotImplementedError("%s norm has not been supported." % dist_norm)        # utils.py:189
+        self._check_geometry(ksize, pad, stride)
+        if dist_norm == "l1":
+            self._crit |= _DIST_L1
+        if pyramid not in ("aten", "fused"):
+            raise ValueError("pyramid must be 'aten' or 'fused'")
+        self.pyramid = pyramid
+        self.last_indices = None
+        _cabi.lib()
+
+    def _check_geometry(self, ksize, pad, stride):
+        if ksize != 3:
+            raise NotImplementedError(f"{type(self).__name__}: libsrst.so implements ksize=3 only")
+
+    def forward(self, x, gt):
+        _check_pair(x, gt, type(self).__name__)
+        loss, idx = _PatchLossFn.apply(x, gt, type(self), self._args(), self.pyramid)
+        self.last_indices = idx
+        return loss
+
+    @classmethod
+    def _plan(cls, args, B, H, W):
+        """(patches per image, workspace kind, workspace bytes) of the default 3x3 / stride-3 patch grid."""
         if H < 12 or W < 12:
-            raise ValueError(f"BestBuddyLoss: images must be at least 12x12 (got {H}x{W})")
-        with _on_device(sr.device):
-            stream = _raw_stream(sr.device)
-            if pyramid == "aten":
-                # the reference's own op for the HR pyramid (loss.py:123,127)
-                with torch.no_grad():
-                    gt2 = torch.nn.functional.interpolate(gt, scale_factor=0.5, mode="bicubic",
-                                                          align_corners=False).contiguous()
-                    gt4 = torch.nn.functional.interpolate(gt, scale_factor=0.25, mode="bicubic",
-                                                          align_corners=False).contiguous()
-            else:
-                gt2 = gt4 = None  # libsrst computes them (srst_bb_pyramid taps)
-            N = (H // 3) * (W // 3)
-            idx = torch.empty((B, N), dtype=torch.int64, device=sr.device)
-            loss = torch.empty((), dtype=torch.float32, device=sr.device)
-            nbytes = lib.srst_bb_workspace_bytes(B, H, W)
-            ws = _workspace("bb", sr.device, stream, nbytes)
-            rc = fwd(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, float(alpha), float(beta),
-                                     int(criterion), _ptr(idx), _ptr(loss), _ptr(ws), ws.numel(),
-                                     stream)
-        _cabi.check(rc, "srst_bb_forward" if mode == "patch" else "srst_gram_forward")
-        ctx.save_for_backward(sr, gt, gt2, gt4, idx)
-        ctx.criterion = int(criterion)
-        ctx.mode = mode
-        ctx.mark_non_differentiable(idx)
-        return loss, idx
-
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_out, _grad_idx):
-        lib = _cabi.lib()
-        sr, gt, gt2, gt4, idx = ctx.saved_tensors
-        B, _, H, W = sr.shape
-        bwd = lib.srst_bb_backward if ctx.mode == "patch" else lib.srst_gram_backward
-        if not (ctx.needs_input_grad[0] or ctx.needs_input_grad[1]):
-            return None, None, None, None, None, None, None
-        grad_out = grad_out.to(torch.float32).contiguous()
-        d_sr = d_gt = None
-        with _on_device(sr.device):
-            stream = _raw_stream(sr.device)
-            if ctx.needs_input_grad[0]:
-                d_sr = torch.empty_like(sr)
-                nbytes = lib.srst_bb_workspace_bytes(B, H, W)
-                ws = _workspace("bb", sr.device, stream, nbytes)
-                rc = bwd(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H, W,
-                         ctx.criterion, _ptr(d_sr), _ptr(ws), ws.numel(), stream)
-                _cabi.check(rc, "srst_bb_backward" if ctx.mode == "patch" else "srst_gram_backward")
-            if ctx.needs_input_grad[1]:
-                d_gt = _patch_backward_gt(0 if ctx.mode == "patch" else 1, sr, gt, gt2, gt4, idx, grad_out, None,
-                                          ctx.criterion, stream)
-        return d_sr, d_gt, None, None, None, None, None
+            raise ValueError(f"{cls.__name__}: images must be at least 12x12 (got {H}x{W})")
+        return (H // 3) * (W // 3), "bb", _cabi.lib().srst_bb_workspace_bytes(B, H, W)
 
 
-class _BestBuddyGeometryFn(torch.autograd.Function):
-    """BestBuddyLoss with a non-default (ksize, pad, stride): the exact all-pairs path of libsrst (include/srst.h,
-    srst_bbg_forward / srst_bbg_backward).  Differentiable w.r.t. the SR patches (folded back over overlapping patches)
-    and, through the gather of the selected candidates, w.r.t. gt (loss.py:135-139); the argmin is not."""
-
-    @staticmethod
-    def forward(ctx, sr, gt, alpha, beta, criterion, pyramid, geom):
-        lib = _cabi.lib()
-        sr = sr.contiguous()
-        gt = gt.contiguous()
-        B, _, H, W = sr.shape
-        ks, pad, st = geom
-        N = lib.srst_bbg_num_patches(H, W, ks, pad, st)
-        nbytes = lib.srst_bbg_workspace_bytes(B, H, W, ks, pad, st)
-        if N <= 0 or nbytes == 0:
-            raise ValueError(f"BestBuddyLoss: a {H}x{W} image has a pyramid level without a single "
-                             f"ksize={ks}, pad={pad}, stride={st} patch (F.unfold would raise too)")
-        with _on_device(sr.device):
-            stream = _raw_stream(sr.device)
-            if pyramid == "aten":
-                with torch.no_grad():
-                    gt2 = torch.nn.functional.interpolate(gt, scale_factor=0.5, mode="bicubic",
-                                                          align_corners=False).contiguous()
-                    gt4 = torch.nn.functional.interpolate(gt, scale_factor=0.25, mode="bicubic",
-                                                          align_corners=False).contiguous()
-            else:
-                gt2 = gt4 = None
-            idx = torch.empty((B, N), dtype=torch.int64, device=sr.device)
-            loss = torch.empty((), dtype=torch.float32, device=sr.device)
-            ws = _workspace("bbg", sr.device, stream, nbytes)
-            rc = lib.srst_bbg_forward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, ks, pad, st, float(alpha),
-                                      float(beta), int(criterion), _ptr(idx), _ptr(loss), _ptr(ws), ws.numel(), stream)
-        _cabi.check(rc, "srst_bbg_forward")
-        ctx.save_for_backward(sr, gt, gt2, gt4, idx)
-        ctx.criterion = int(criterion)
-        ctx.geom = geom
-        ctx.mark_non_differentiable(idx)
-        return loss, idx
-
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_out, _grad_idx):
-        lib = _cabi.lib()
-        sr, gt, gt2, gt4, idx = ctx.saved_tensors
-        if not (ctx.needs_input_grad[0] or ctx.needs_input_grad[1]):
-            return None, None, None, None, None, None, None
-        B, _, H, W = sr.shape
-        ks, pad, st = ctx.geom
-        grad_out = grad_out.to(torch.float32).contiguous()
-        with _on_device(sr.device):
-            stream = _raw_stream(sr.device)
-            d_sr = torch.empty_like(sr) if ctx.needs_input_grad[0] else None
-            d_gt = torch.empty_like(gt) if ctx.needs_input_grad[1] else None
-            ws = _workspace("bbg", sr.device, stream, lib.srst_bbg_workspace_bytes(B, H, W, ks, pad, st))
-            rc = lib.srst_bbg_backward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H, W,
-                                       ks, pad, st, ctx.criterion, _ptr(d_sr), _ptr(d_gt), _ptr(ws), ws.numel(), stream)
-        _cabi.check(rc, "srst_bbg_backward")
-        return d_sr, d_gt, None, None, None, None, None
-
-
-class BestBuddyLoss(nn.Module):
+class BestBuddyLoss(_PatchLoss):
     """Best-Buddy loss; same signature and semantics as reference loss.py:78-141.
 
     ``forward(x, gt)``: for every 3x3 SR patch pick the HR candidate patch (three pyramid levels)
@@ -500,23 +489,11 @@ class BestBuddyLoss(nn.Module):
 
     def __init__(self, alpha: float = 1.0, beta: float = 1.0, ksize: int = 3, pad: int = 0, stride: int = 3,
                  dist_norm: str = "l2", criterion: str = "l1", pyramid: str = "fused"):
-        super().__init__()
-        self.alpha = alpha
-        self.beta = beta
-        self.ksize = ksize
+        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid, pad, stride)
         self.pad = pad
         self.stride = stride
-        self.dist_norm = dist_norm
-        if criterion == "l1":
-            self.criterion = torch.nn.L1Loss()   # kept for repr/config parity (config.py:133-139)
-            self._crit = 0
-        elif criterion == "l2" or criterion == "mse":
-            self.criterion = torch.nn.MSELoss()
-            self._crit = 1
-        else:
-            raise NotImplementedError("%s criterion has not been implmented." % criterion)  # loss.py:113
-        if dist_norm not in ("l1", "l2"):
-            raise NotImplementedError("%s norm has not been supported." % dist_norm)        # utils.py:189
+
+    def _check_geometry(self, ksize, pad, stride):
         self._geom = None   # None: the tuned (3, 0, 3) kernels; else the generic-geometry path
         if (ksize, pad, stride) != (3, 0, 3):
             if not all(isinstance(v, int) and not isinstance(v, bool) for v in (ksize, pad, stride)):
@@ -526,165 +503,119 @@ class BestBuddyLoss(nn.Module):
                     f"BestBuddyLoss: libsrst.so has kernels for 1 <= ksize <= 8, pad >= 0, stride >= 1 "
                     f"(got ksize={ksize}, pad={pad}, stride={stride})")
             self._geom = (ksize, pad, stride)
-        if dist_norm == "l1":
-            self._crit |= _DIST_L1
-        if pyramid not in ("aten", "fused"):
-            raise ValueError("pyramid must be 'aten' or 'fused'")
-        self.pyramid = pyramid
-        self.last_indices = None
-        _cabi.lib()
 
-    def forward(self, x, gt):
-        _check_pair(x, gt, "BestBuddyLoss")
-        if self._geom is not None:
-            loss, idx = _BestBuddyGeometryFn.apply(x, gt, self.alpha, self.beta, self._crit, self.pyramid, self._geom)
+    def _args(self):
+        return float(self.alpha), float(self.beta), int(self._crit), self._geom
+
+    @classmethod
+    def _plan(cls, args, B, H, W):
+        if args[3] is None:
+            return super()._plan(args, B, H, W)
+        lib = _cabi.lib()
+        ks, pad, st = args[3]
+        n = lib.srst_bbg_num_patches(H, W, ks, pad, st)
+        nbytes = lib.srst_bbg_workspace_bytes(B, H, W, ks, pad, st)
+        if n <= 0 or nbytes == 0:
+            raise ValueError(f"BestBuddyLoss: a {H}x{W} image has a pyramid level without a single "
+                             f"ksize={ks}, pad={pad}, stride={st} patch (F.unfold would raise too)")
+        return n, "bbg", nbytes
+
+    @staticmethod
+    def _fwd(args, sr, gt, gt2, gt4, idx, loss, ws, stream):
+        alpha, beta, crit, geom = args
+        lib = _cabi.lib()
+        B, _, H, W = sr.shape
+        if geom is None:
+            rc = lib.srst_bb_forward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, alpha, beta, crit, _ptr(idx),
+                                     _ptr(loss), _ptr(ws), ws.numel(), stream)
+            _cabi.check(rc, "srst_bb_forward")
         else:
-            loss, idx = _BestBuddyLossFn.apply(x, gt, self.alpha, self.beta, self._crit, self.pyramid)
-        self.last_indices = idx
-        return loss
+            rc = lib.srst_bbg_forward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, *geom, alpha, beta, crit,
+                                      _ptr(idx), _ptr(loss), _ptr(ws), ws.numel(), stream)
+            _cabi.check(rc, "srst_bbg_forward")
+
+    @staticmethod
+    def _bwd(args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, ws, stream):
+        crit, geom = args[2:]
+        lib = _cabi.lib()
+        B, _, H, W = sr.shape
+        if geom is not None:   # one call fills d_sr and d_gt, either of which may be None
+            rc = lib.srst_bbg_backward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H, W, *geom,
+                                       crit, _ptr(d_sr), _ptr(d_gt), _ptr(ws), ws.numel(), stream)
+            _cabi.check(rc, "srst_bbg_backward")
+            return
+        if d_sr is not None:
+            rc = lib.srst_bb_backward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H, W, crit,
+                                      _ptr(d_sr), _ptr(ws), ws.numel(), stream)
+            _cabi.check(rc, "srst_bb_backward")
+        if d_gt is not None:
+            _patch_backward_gt(0, sr, gt, gt2, gt4, idx, grad_out, _NO_TAPS, crit, d_gt, ws, stream)
 
 
-class GramLoss(nn.Module):
+class GramLoss(_PatchLoss):
     """Gram loss; same signature and semantics as reference loss.py:146-225: the best-buddy search
     and the final criterion run on the 3x3 Gram matrix of every 3x3x3 patch instead of its pixels.
     Only ``ksize=3`` has kernels (the reference's default); ``dist_norm`` may be 'l2' or 'l1'."""
 
     def __init__(self, alpha: float = 1.0, beta: float = 1.0, ksize: int = 3, dist_norm: str = "l2",
                  criterion: str = "l1", pyramid: str = "fused"):
-        super().__init__()
-        self.alpha = alpha
-        self.beta = beta
-        self.ksize = ksize
-        self.dist_norm = dist_norm
-        if criterion == "l1":
-            self.criterion = torch.nn.L1Loss()
-            self._crit = 0
-        elif criterion == "l2" or criterion == "mse":
-            self.criterion = torch.nn.MSELoss()
-            self._crit = 1
-        else:
-            raise NotImplementedError("%s criterion has not been implmented." % criterion)  # loss.py:178
-        if dist_norm not in ("l1", "l2"):
-            raise NotImplementedError("%s norm has not been supported." % dist_norm)        # utils.py:189
-        if ksize != 3:
-            raise NotImplementedError("GramLoss: libsrst.so implements ksize=3 only")
-        if dist_norm == "l1":
-            self._crit |= _DIST_L1
-        if pyramid not in ("aten", "fused"):
-            raise ValueError("pyramid must be 'aten' or 'fused'")
-        self.pyramid = pyramid
-        self.last_indices = None
-        _cabi.lib()
+        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid)
 
-    def forward(self, x, gt):
-        _check_pair(x, gt, "GramLoss")
-        loss, idx = _BestBuddyLossFn.apply(x, gt, self.alpha, self.beta, self._crit, self.pyramid, "gram")
-        self.last_indices = idx
-        return loss
-
-
-class _PatchwiseStLossFn(torch.autograd.Function):
-    """autograd boundary of the patchwise structure-tensor loss: differentiable through the final
-    criterion and the descriptors of the SR patch and of the selected candidate (argmin is not; loss.py:366-371)."""
+    def _args(self):
+        return float(self.alpha), float(self.beta), int(self._crit)
 
     @staticmethod
-    def forward(ctx, sr, gt, sigma, rho, alpha, beta, criterion, pyramid):
-        lib = _cabi.lib()
-        sr = sr.contiguous()
-        gt = gt.contiguous()
+    def _fwd(args, sr, gt, gt2, gt4, idx, loss, ws, stream):
+        alpha, beta, crit = args
         B, _, H, W = sr.shape
-        if H < 12 or W < 12:
-            raise ValueError(f"PatchwiseStructureTensorLoss: images must be at least 12x12 (got {H}x{W})")
-        g, dg = _taps.gaussian_taps(float(sigma))
-        k, _ = _taps.gaussian_taps(float(rho))
-        with _on_device(sr.device):
-            stream = _raw_stream(sr.device)
-            if pyramid == "aten":
-                with torch.no_grad():  # the reference's own op for the HR pyramid (loss.py:353,356)
-                    gt2 = torch.nn.functional.interpolate(gt, scale_factor=0.5, mode="bicubic",
-                                                          align_corners=False).contiguous()
-                    gt4 = torch.nn.functional.interpolate(gt, scale_factor=0.25, mode="bicubic",
-                                                          align_corners=False).contiguous()
-            else:
-                gt2 = gt4 = None
-            N = (H // 3) * (W // 3)
-            idx = torch.empty((B, N), dtype=torch.int64, device=sr.device)
-            loss = torch.empty((), dtype=torch.float32, device=sr.device)
-            ws = _workspace("bb", sr.device, stream, lib.srst_bb_workspace_bytes(B, H, W))
-            rc = lib.srst_pst_forward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, _taps.as_c(g), _taps.as_c(dg),
-                                      len(g) // 2, _taps.as_c(k), len(k) // 2, float(alpha), float(beta),
-                                      int(criterion), _ptr(idx), _ptr(loss), _ptr(ws), ws.numel(),
-                                      stream)
-        _cabi.check(rc, "srst_pst_forward")
-        ctx.save_for_backward(sr, gt, gt2, gt4, idx)
-        ctx.taps = (g, dg, k)
-        ctx.criterion = int(criterion)
-        ctx.mark_non_differentiable(idx)
-        return loss, idx
+        rc = _cabi.lib().srst_gram_forward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, alpha, beta, crit, _ptr(idx),
+                                           _ptr(loss), _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_gram_forward")
 
     @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_out, _grad_idx):
-        lib = _cabi.lib()
-        sr, gt, gt2, gt4, idx = ctx.saved_tensors
-        g, dg, k = ctx.taps
+    def _bwd(args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, ws, stream):
+        crit = args[2]
         B, _, H, W = sr.shape
-        if not (ctx.needs_input_grad[0] or ctx.needs_input_grad[1]):
-            return (None,) * 8
-        grad_out = grad_out.to(torch.float32).contiguous()
-        d_sr = d_gt = None
-        with _on_device(sr.device):
-            stream = _raw_stream(sr.device)
-            if ctx.needs_input_grad[0]:
-                d_sr = torch.empty_like(sr)
-                ws = _workspace("bb", sr.device, stream, lib.srst_bb_workspace_bytes(B, H, W))
-                rc = lib.srst_pst_backward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H, W,
-                                           _taps.as_c(g), _taps.as_c(dg), len(g) // 2, _taps.as_c(k), len(k) // 2,
-                                           ctx.criterion, _ptr(d_sr), _ptr(ws), ws.numel(), stream)
-                _cabi.check(rc, "srst_pst_backward")
-            if ctx.needs_input_grad[1]:
-                d_gt = _patch_backward_gt(2, sr, gt, gt2, gt4, idx, grad_out, (g, dg, k), ctx.criterion, stream)
-        return (d_sr, d_gt) + (None,) * 6
+        if d_sr is not None:
+            rc = _cabi.lib().srst_gram_backward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H, W,
+                                                crit, _ptr(d_sr), _ptr(ws), ws.numel(), stream)
+            _cabi.check(rc, "srst_gram_backward")
+        if d_gt is not None:
+            _patch_backward_gt(1, sr, gt, gt2, gt4, idx, grad_out, _NO_TAPS, crit, d_gt, ws, stream)
 
 
-class PatchwiseStructureTensorLoss(nn.Module):
+class PatchwiseStructureTensorLoss(_PatchLoss):
     """Patchwise structure-tensor loss; same signature and semantics as reference loss.py:292-375:
     the best-buddy search and the final criterion run on the det-normalised structure tensor of
     every 3x3 patch (seen as a 3x3 image, zero 'same' padding) instead of its pixels.
     Only ``ksize=3`` has kernels (the reference's default); ``dist_norm`` may be 'l2' or 'l1'."""
 
+    _criterion_error = "%s criterion has not been supported."   # loss.py:323
+
     def __init__(self, sigma: float = 0.5, rho: float = 2, alpha: float = 1.0, beta: float = 1.0, ksize: int = 3,
                  dist_norm: str = "l2", criterion: str = "l1", pyramid: str = "fused"):
-        super().__init__()
-        self.alpha = alpha
-        self.beta = beta
-        self.ksize = ksize
-        self.dist_norm = dist_norm
+        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid)
         self.sigma = sigma
         self.rho = rho
-        if criterion == "l1":
-            self.criterion = torch.nn.L1Loss(reduction="mean")
-            self._crit = 0
-        elif criterion == "l2" or criterion == "mse":
-            self.criterion = torch.nn.MSELoss(reduction="mean")
-            self._crit = 1
-        else:
-            raise NotImplementedError("%s criterion has not been supported." % criterion)  # loss.py:323
-        if dist_norm not in ("l1", "l2"):
-            raise NotImplementedError("%s norm has not been supported." % dist_norm)       # utils.py:189
-        if ksize != 3:
-            raise NotImplementedError("PatchwiseStructureTensorLoss: libsrst.so implements ksize=3 only")
-        if dist_norm == "l1":
-            self._crit |= _DIST_L1
-        if pyramid not in ("aten", "fused"):
-            raise ValueError("pyramid must be 'aten' or 'fused'")
-        self.pyramid = pyramid
-        self.last_indices = None
-        _cabi.lib()
 
-    def forward(self, x, gt):
-        _check_pair(x, gt, "PatchwiseStructureTensorLoss")
-        loss, idx = _PatchwiseStLossFn.apply(x, gt, self.sigma, self.rho, self.alpha, self.beta, self._crit,
-                                             self.pyramid)
-        self.last_indices = idx
-        return loss
+    def _args(self):
+        return float(self.alpha), float(self.beta), int(self._crit), _pst_taps(self.sigma, self.rho)
+
+    @staticmethod
+    def _fwd(args, sr, gt, gt2, gt4, idx, loss, ws, stream):
+        alpha, beta, crit, taps = args
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_pst_forward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, *taps[:5], alpha, beta, crit,
+                                          _ptr(idx), _ptr(loss), _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_pst_forward")
+
+    @staticmethod
+    def _bwd(args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, ws, stream):
+        crit, taps = args[2:]
+        B, _, H, W = sr.shape
+        if d_sr is not None:
+            rc = _cabi.lib().srst_pst_backward(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B, H, W,
+                                               *taps[:5], crit, _ptr(d_sr), _ptr(ws), ws.numel(), stream)
+            _cabi.check(rc, "srst_pst_backward")
+        if d_gt is not None:
+            _patch_backward_gt(2, sr, gt, gt2, gt4, idx, grad_out, taps, crit, d_gt, ws, stream)

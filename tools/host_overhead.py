@@ -1,5 +1,6 @@
-"""Where the eager module path spends host time: cProfile of StructureTensorLoss fwd+bwd at batch 64 x 96x96 with
-device-resident inputs (kernels take ~31 us; everything else is Python / torch / ctypes overhead).
+"""Where the eager module path spends host time: host enqueue and wall time per fwd+bwd of every loss module, then a
+cProfile of StructureTensorLoss fwd+bwd, at batch 64 x 96x96 with device-resident inputs (the ST kernels take ~31 us;
+everything else is Python / torch / ctypes overhead).
     python tools/host_overhead.py > gpurun_out/host_overhead.log"""
 import cProfile
 import os
@@ -10,7 +11,8 @@ import time
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from srgan_st_b200 import StructureTensorLoss, StructureTensorPixelLoss  # noqa: E402
+from srgan_st_b200 import (BestBuddyLoss, GramLoss, PatchwiseStructureTensorLoss, StructureTensorLoss,  # noqa: E402
+                           StructureTensorPixelLoss)
 
 torch.manual_seed(0)
 y = torch.rand(64, 3, 96, 96, device="cuda")
@@ -32,7 +34,9 @@ def bench(m, n=300):
     return t_enq * 1e6, t_all * 1e6
 
 
-for name, m in (("StructureTensorLoss", StructureTensorLoss()), ("StructureTensorPixelLoss", StructureTensorPixelLoss())):
+for name, m in (("StructureTensorLoss", StructureTensorLoss()), ("StructureTensorPixelLoss", StructureTensorPixelLoss()),
+                ("BestBuddyLoss", BestBuddyLoss()), ("BestBuddyLoss(ksize=4, stride=4)", BestBuddyLoss(ksize=4, stride=4)),
+                ("GramLoss", GramLoss()), ("PatchwiseStructureTensorLoss", PatchwiseStructureTensorLoss())):
     enq, tot = bench(m)
     print(f"{name}: host enqueue {enq:.1f} us per fwd+bwd, wall {tot:.1f} us per fwd+bwd (device-resident inputs, eager)")
 m = StructureTensorLoss()
