@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define SRST_VERSION 204 /* major*100 + minor: the major number changes whenever an argument list changes */
+#define SRST_VERSION 205 /* major*100 + minor: the major number changes whenever an argument list changes */
 
 #define SRST_E_INVALID (-1)     /* null pointer / non-positive size / bad enum */
 #define SRST_E_UNSUPPORTED (-2) /* filter radius or patch geometry not compiled in */
@@ -122,6 +122,27 @@ int srst_st_backward_ws(const float* ixy, const float* ds, const float* grad_out
                         const float* g, const float* dg, int r_sigma,
                         const float* k, int r_rho,
                         float* d_img, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Per-image reduction (reduction='none'; the reference's vmap(st_loss)(x, gt) before its .mean(), loss.py:411-413).
+ * Same arguments, checks, return codes, workspace and saved buffers as srst_st_forward / srst_st_backward_ws, for the
+ * compiled radius classes and the generic-radius path alike, but
+ *   srst_st_forward_per_image:  loss_out[b] = mean over the H*W pixels of image b   (device, B floats)
+ *   srst_st_backward_per_image: grad_out = device [B], the upstream gradient of each loss_out[b] (any values, e.g.
+ *                               all equal after .sum()); d_img of image b = grad_out[b]/(H*W) * dLoss_b/dimg
+ * The tile shapes are the ones srst_st_forward / srst_st_backward pick, and each image's pixels are reduced in double
+ * in a fixed order, so results are deterministic; d_img of image b is bit-identical to srst_st_backward_ws on that
+ * image alone (B = 1) with grad_out[b]. */
+int srst_st_forward_per_image(const float* sr, const float* hr, int B, int H, int W,
+                              const float* g, const float* dg, int r_sigma,
+                              const float* k, int r_rho,
+                              int normalize, float eps,
+                              float* loss_out, float* ds_sr, float* ds_hr, float* ixy_sr, float* ixy_hr,
+                              void* workspace, size_t workspace_bytes, void* stream);
+int srst_st_backward_per_image(const float* ixy, const float* ds, const float* grad_out,
+                               int B, int H, int W,
+                               const float* g, const float* dg, int r_sigma,
+                               const float* k, int r_rho,
+                               float* d_img, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Structure-tensor FEATURES of one image tensor (diagnostic output; BASELINE.json north_star: "closed-form 2x2
  * eigendecomposition giving orientation, coherence and eigenvalues").  The reference computes these only in an
@@ -256,6 +277,31 @@ int srst_patch_backward_gt(int mode, const float* sr, const float* gt, const flo
                            int criterion,
                            float* d_gt, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Per-image reduction (reduction='none') of the three default-geometry patch losses.
+ *   mode: 0 = BestBuddyLoss, 1 = GramLoss, 2 = PatchwiseStructureTensorLoss (g, dg, k as for srst_pst_forward;
+ *         ignored, may be NULL, for modes 0 and 1); any other mode: SRST_E_INVALID.
+ * srst_patch_forward_per_image: the arguments of srst_bb_forward / srst_gram_forward / srst_pst_forward (criterion with
+ *   SRST_BB_DIST_L1, gt2 / gt4, workspace: srst_bb_workspace_bytes), but loss_out[b] = the mean over image b's N*D
+ *   criterion terms (device, B floats): the reference module applied to image b alone.  idx_out is the same as there.
+ * srst_patch_backward_per_image: grad_out = device [B]; d_sr = the srst_*_backward result with image b scaled by
+ *   grad_out[b]/(N*D) instead of grad_out[0]/(B*N*D) (bit-identical to the scalar entry point on image b alone), d_gt
+ *   = the srst_patch_backward_gt result likewise (atomicAdd: last bits may vary).  Either of d_sr / d_gt may be NULL,
+ *   not both.  The workspace is required whenever d_gt is given or gt2 / gt4 are NULL.
+ * Return codes as the scalar entry points; the per-image forward may overwrite the x1/2 pyramid level it built in the
+ * workspace (the backward entry points rebuild it). */
+int srst_patch_forward_per_image(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                                 int B, int H, int W,
+                                 const float* g, const float* dg, int r_sigma, const float* k, int r_rho,
+                                 float alpha, float beta, int criterion,
+                                 int64_t* idx_out, float* loss_out,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+int srst_patch_backward_per_image(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                                  const int64_t* idx, const float* grad_out,
+                                  int B, int H, int W,
+                                  const float* g, const float* dg, int r_sigma, const float* k, int r_rho,
+                                  int criterion,
+                                  float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Best-Buddy loss with an arbitrary patch geometry: BestBuddyLoss(ksize, pad, stride) of the reference
  * (loss.py:86; F.unfold(kernel_size=ksize, padding=pad, stride=stride) at loss.py:116-129) for everything
@@ -285,6 +331,20 @@ int srst_bbg_backward(const float* sr, const float* gt, const float* gt2, const 
                       int B, int H, int W, int ksize, int pad, int stride, int criterion,
                       float* d_sr, float* d_gt,
                       void* workspace, size_t workspace_bytes, void* stream);
+
+/* Per-image reduction (reduction='none') of the arbitrary-geometry path: the arguments, checks and workspace of
+ * srst_bbg_forward / srst_bbg_backward, but loss_out[b] = the mean over image b's N*D terms (device, B floats) and
+ * grad_out = device [B] (image b's gradients scaled by grad_out[b]/(N*D)). */
+int srst_bbg_forward_per_image(const float* sr, const float* gt, const float* gt2, const float* gt4,
+                               int B, int H, int W, int ksize, int pad, int stride,
+                               float alpha, float beta, int criterion,
+                               int64_t* idx_out, float* loss_out,
+                               void* workspace, size_t workspace_bytes, void* stream);
+int srst_bbg_backward_per_image(const float* sr, const float* gt, const float* gt2, const float* gt4,
+                                const int64_t* idx, const float* grad_out,
+                                int B, int H, int W, int ksize, int pad, int stride, int criterion,
+                                float* d_sr, float* d_gt,
+                                void* workspace, size_t workspace_bytes, void* stream);
 
 /* The HR pyramid on its own (exposed for tests): out2 [B,3,H/2,W/2], out4 [B,3,H/4,W/4]. */
 int srst_bb_pyramid(const float* gt, int B, int H, int W, float* out2, float* out4, void* stream);

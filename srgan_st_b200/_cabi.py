@@ -39,6 +39,13 @@ SIGNATURES = {
     "srst_st_backward_ws": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                            c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
                                            vp, vp, ctypes.c_size_t, vp]),
+    "srst_st_forward_per_image": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                 c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                                 ctypes.c_int, ctypes.c_float, vp, vp, vp, vp, vp,
+                                                 vp, ctypes.c_size_t, vp]),
+    "srst_st_backward_per_image": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                  c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                                  vp, vp, ctypes.c_size_t, vp]),
     "srst_st_features": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                         c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int, vp, vp, vp, vp, vp]),
     "srst_stpx_forward": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
@@ -67,6 +74,13 @@ SIGNATURES = {
     "srst_patch_backward_gt": (ctypes.c_int, [ctypes.c_int, vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                               c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
                                               ctypes.c_int, vp, vp, ctypes.c_size_t, vp]),
+    "srst_patch_forward_per_image": (ctypes.c_int, [ctypes.c_int, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                    c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                                    ctypes.c_float, ctypes.c_float, ctypes.c_int, vp, vp,
+                                                    vp, ctypes.c_size_t, vp]),
+    "srst_patch_backward_per_image": (ctypes.c_int, [ctypes.c_int, vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int,
+                                                     ctypes.c_int, c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                                     ctypes.c_int, vp, vp, vp, ctypes.c_size_t, vp]),
     "srst_bbg_supported": (ctypes.c_int, [ctypes.c_int] * 3),
     "srst_bbg_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int] * 6),
     "srst_bbg_num_patches": (ctypes.c_longlong, [ctypes.c_int] * 5),
@@ -77,6 +91,13 @@ SIGNATURES = {
     "srst_bbg_backward": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                          ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp,
                                          vp, ctypes.c_size_t, vp]),
+    "srst_bbg_forward_per_image": (ctypes.c_int, [vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                  ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                  ctypes.c_float, ctypes.c_float, ctypes.c_int, vp, vp,
+                                                  vp, ctypes.c_size_t, vp]),
+    "srst_bbg_backward_per_image": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                   ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp,
+                                                   vp, ctypes.c_size_t, vp]),
     "srst_bb_pyramid": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp, vp]),
 }
 

@@ -261,7 +261,25 @@ bbg_search_kernel(const float* __restrict__ sr, const float* __restrict__ gt, co
   }
 }
 
-// one thread per query patch
+// criterion term (sum over the D patch elements) of query i of image b against its selected candidate
+SRST_DEV float bbg_loss_term(const float* sr, const float* gt, const float* gt2, const float* gt4, const BbgGeom& g,
+                             int criterion, int b, int i, int j) {
+  j = min(max(j, 0), g.M - 1);
+  const BbgPatch P1 = bbg_patch_of(sr + (size_t)b * 3 * g.L[0].H * g.L[0].W, g.L[0], g.p, g.s, i);
+  const BbgPatch Pc = bbg_candidate(gt, gt2, gt4, g, b, j);
+  float acc = 0.f;
+  for (int c = 0; c < 3; ++c)
+    for (int ky = 0; ky < g.k; ++ky)
+      for (int kx = 0; kx < g.k; ++kx) {
+        const float d = bbg_value(P1, c, ky, kx) - bbg_value(Pc, c, ky, kx);
+        acc += (criterion == 0) ? fabsf(d) : d * d;
+      }
+  return acc;
+}
+
+// one thread per query patch.  PER_IMG: reduction='none' -- ceil(N / BBG_NT) CTAs per image, image-major, so no CTA
+// spans two images; loss_out[b] = the mean over image b's N*D terms.
+template <bool PER_IMG = false>
 __global__ void __launch_bounds__(BBG_NT)
 bbg_loss_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                 const float* __restrict__ gt4, BbgGeom g, const int64_t* __restrict__ idx, int criterion, float* partials,
@@ -271,18 +289,13 @@ bbg_loss_kernel(const float* __restrict__ sr, const float* __restrict__ gt, cons
   const int tid = threadIdx.x;
   const size_t t = (size_t)blockIdx.x * BBG_NT + tid;
   float acc = 0.f;
-  if (t < (size_t)g.B * g.N) {
+  if constexpr (PER_IMG) {
+    const unsigned int per = gridDim.x / g.B, b = blockIdx.x / per;
+    const int i = (int)(blockIdx.x - b * per) * BBG_NT + tid;
+    if (i < g.N) acc = bbg_loss_term(sr, gt, gt2, gt4, g, criterion, (int)b, i, (int)idx[(size_t)b * g.N + i]);
+  } else if (t < (size_t)g.B * g.N) {
     const int b = (int)(t / g.N), i = (int)(t - (size_t)b * g.N);
-    int j = (int)idx[t];
-    j = min(max(j, 0), g.M - 1);
-    const BbgPatch P1 = bbg_patch_of(sr + (size_t)b * 3 * g.L[0].H * g.L[0].W, g.L[0], g.p, g.s, i);
-    const BbgPatch Pc = bbg_candidate(gt, gt2, gt4, g, b, j);
-    for (int c = 0; c < 3; ++c)
-      for (int ky = 0; ky < g.k; ++ky)
-        for (int kx = 0; kx < g.k; ++kx) {
-          const float d = bbg_value(P1, c, ky, kx) - bbg_value(Pc, c, ky, kx);
-          acc += (criterion == 0) ? fabsf(d) : d * d;
-        }
+    acc = bbg_loss_term(sr, gt, gt2, gt4, g, criterion, b, i, (int)idx[t]);
   }
   acc = warp_sum(acc);
   if ((tid & 31) == 0) s_red[tid >> 5] = acc;
@@ -295,7 +308,13 @@ bbg_loss_kernel(const float* __restrict__ sr, const float* __restrict__ gt, cons
     s_last = (atomicAdd(ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
   }
   __syncthreads();
-  if (s_last && tid < 32) {
+  if constexpr (PER_IMG) {
+    if (s_last) {
+      __threadfence();
+      reduce_partials_per_image(partials, g.B, gridDim.x / g.B, 1.0 / ((double)g.N * g.D), loss_out);
+      if (tid == 0) *ticket = 0u;
+    }
+  } else if (s_last && tid < 32) {
     __threadfence();
     double tot = 0.0;
     for (unsigned int i = tid; i < gridDim.x; i += 32) { tot += (double)__ldcg(partials + i); partials[i] = 0.f; }
@@ -312,7 +331,9 @@ SRST_DEV float bbg_crit_grad(float d, int criterion, float scale) {
   return (criterion == 0) ? ((d > 0.f) ? scale : ((d < 0.f) ? -scale : 0.f)) : 2.0f * d * scale;
 }
 
-// one thread per SR pixel: the patches py in [ceil((y + p - k + 1)/s), floor((y + p)/s)] x likewise px cover it
+// one thread per SR pixel: the patches py in [ceil((y + p - k + 1)/s), floor((y + p)/s)] x likewise px cover it.
+// PER_IMG: reduction='none', grad_out is [B] and image b scales by grad_out[b] / (N D)
+template <bool PER_IMG = false>
 __global__ void __launch_bounds__(256)
 bbg_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                     const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -324,7 +345,7 @@ bbg_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, 
   const int y = (int)((t / W) % H);
   const int c = (int)((t / ((size_t)W * H)) % 3);
   const int b = (int)(t / ((size_t)3 * W * H));
-  const float scale = __ldg(grad_out) / ((float)g.B * (float)g.N * (float)g.D);
+  const float scale = __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : g.B) * (float)g.N * (float)g.D);
   const float v = __ldg(sr + t);
   const int ylo = y + g.p - g.k + 1, xlo = x + g.p - g.k + 1;
   const int py0 = ylo <= 0 ? 0 : (ylo + g.s - 1) / g.s, py1 = min((y + g.p) / g.s, g.L[0].ny - 1);
@@ -342,6 +363,8 @@ bbg_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, 
 }
 
 // one thread per (query patch, channel): minus the SR-side gradient lands on the selected candidate's pixels
+// (PER_IMG: reduction='none', grad_out is [B] and image b scales by grad_out[b] / (N D))
+template <bool PER_IMG = false>
 __global__ void __launch_bounds__(256)
 bbg_backward_gt_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                        const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -353,7 +376,7 @@ bbg_backward_gt_kernel(const float* __restrict__ sr, const float* __restrict__ g
   const int b = (int)(bi / g.N), i = (int)(bi - (size_t)b * g.N);
   int j = (int)idx[bi];
   j = min(max(j, 0), g.M - 1);
-  const float scale = __ldg(grad_out) / ((float)g.B * (float)g.N * (float)g.D);
+  const float scale = __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : g.B) * (float)g.N * (float)g.D);
   const BbgPatch P1 = bbg_patch_of(sr + (size_t)b * 3 * g.L[0].H * g.L[0].W, g.L[0], g.p, g.s, i);
   const BbgPatch Pc = bbg_candidate(gt, gt2, gt4, g, b, j);
   const int l = j < g.L[0].n ? 0 : (j < g.L[0].n + g.L[1].n ? 1 : 2);

@@ -798,7 +798,29 @@ bb_search_l1_kernel(const float* __restrict__ mats, size_t per_image, BbGeom g, 
 }
 
 // ---- loss ---------------------------------------------------------------------------------------
+// criterion term (sum over the D descriptor elements) of query i of image b against its selected candidate j
 template <int D>
+SRST_DEV float bb_loss_term(const float* mats, size_t per_image, const BbGeom& g, int b, int i, int j, int criterion) {
+  const BbPtrs P = bb_image_ptrs(mats, per_image, b, g.Npad, g.Mpad, D);
+  float acc = 0.f;
+#pragma unroll
+  for (int k = 0; k < D; ++k) {
+    const float d = __ldg(P.q1 + (size_t)k * g.Npad + i) - __ldg(P.y + (size_t)k * g.Mpad + j);
+    acc += (criterion == 0) ? fabsf(d) : d * d;
+  }
+  return acc;
+}
+
+// Criterion-gradient scale of a term of image b over `D` elements: grad_out[0] / (B N D) for the batch mean,
+// grad_out[b] / (N D) per image (reduction='none': grad_out is [B]).
+template <bool PER_IMG>
+SRST_DEV float patch_grad_scale(const float* __restrict__ grad_out, int b, int B, int N, float D) {
+  return __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : B) * (float)N * D);
+}
+
+// PER_IMG: reduction='none' -- ceil(N / BB_NT) CTAs per image, image-major, so no CTA spans two images;
+// loss_out[b] = the mean over image b's N*D terms.
+template <int D, bool PER_IMG = false>
 __global__ void __launch_bounds__(BB_NT)
 bb_loss_kernel(const float* __restrict__ mats, size_t per_image, BbGeom g, const int64_t* __restrict__ idx,
                int criterion, float* partials, unsigned int* ticket, float* loss_out) {
@@ -807,15 +829,13 @@ bb_loss_kernel(const float* __restrict__ mats, size_t per_image, BbGeom g, const
   const int tid = threadIdx.x;
   const size_t t = (size_t)blockIdx.x * BB_NT + tid;
   float acc = 0.f;
-  if (t < (size_t)g.B * g.N) {
+  if constexpr (PER_IMG) {
+    const unsigned int per = gridDim.x / g.B, b = blockIdx.x / per;
+    const int i = (int)(blockIdx.x - b * per) * BB_NT + tid;
+    if (i < g.N) acc = bb_loss_term<D>(mats, per_image, g, (int)b, i, (int)idx[(size_t)b * g.N + i], criterion);
+  } else if (t < (size_t)g.B * g.N) {
     const int b = (int)(t / g.N), i = (int)(t - (size_t)b * g.N);
-    const BbPtrs P = bb_image_ptrs(mats, per_image, b, g.Npad, g.Mpad, D);
-    const int j = (int)idx[t];
-#pragma unroll
-    for (int k = 0; k < D; ++k) {
-      const float d = __ldg(P.q1 + (size_t)k * g.Npad + i) - __ldg(P.y + (size_t)k * g.Mpad + j);
-      acc += (criterion == 0) ? fabsf(d) : d * d;
-    }
+    acc = bb_loss_term<D>(mats, per_image, g, b, i, (int)idx[t], criterion);
   }
   acc = warp_sum(acc);
   if ((tid & 31) == 0) s_red[tid >> 5] = acc;
@@ -828,7 +848,13 @@ bb_loss_kernel(const float* __restrict__ mats, size_t per_image, BbGeom g, const
     s_last = (atomicAdd(ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
   }
   __syncthreads();
-  if (s_last && tid < 32) {
+  if constexpr (PER_IMG) {
+    if (s_last) {
+      __threadfence();
+      reduce_partials_per_image(partials, g.B, gridDim.x / g.B, 1.0 / ((double)g.N * D), loss_out);
+      if (tid == 0) *ticket = 0u;
+    }
+  } else if (s_last && tid < 32) {
     __threadfence();
     double tot = 0.0;
     for (unsigned int i = tid; i < gridDim.x; i += 32) { tot += (double)__ldcg(partials + i); partials[i] = 0.f; }
@@ -852,6 +878,8 @@ SRST_DEV float bb_candidate_value(const float* gt, const float* gt2, const float
   return __ldg(img + ((size_t)c * H + 3 * py + ky) * W + 3 * px + kx);
 }
 
+// PER_IMG: reduction='none', grad_out is [B] (patch_grad_scale)
+template <bool PER_IMG = false>
 __global__ void __launch_bounds__(256)
 bb_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                    const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -870,7 +898,7 @@ bb_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, c
     const int j = (int)idx[(size_t)b * g.N + i];
     const float sel = bb_candidate_value(gt, gt2, gt4, g, b, j, c, y - 3 * py, x - 3 * px);
     const float d = __ldg(sr + t) - sel;
-    const float scale = __ldg(grad_out) / ((float)g.B * (float)g.N * (float)BB_D);
+    const float scale = patch_grad_scale<PER_IMG>(grad_out, b, g.B, g.N, (float)BB_D);
     out = (criterion == 0) ? ((d > 0.f) ? scale : ((d < 0.f) ? -scale : 0.f)) : 2.0f * d * scale;
   }
   d_sr[t] = out;
@@ -909,7 +937,8 @@ __global__ void __launch_bounds__(256) bb_fill_zero_kernel(float* __restrict__ p
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = 0.f;
 }
 
-// BestBuddyLoss: one thread per query patch
+// BestBuddyLoss: one thread per query patch (PER_IMG: grad_out is [B], patch_grad_scale)
+template <bool PER_IMG = false>
 __global__ void __launch_bounds__(256)
 bb_backward_gt_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                       const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -921,7 +950,7 @@ bb_backward_gt_kernel(const float* __restrict__ sr, const float* __restrict__ gt
   float v[BB_D], w[BB_D];
   bb_read_patch(sr + (size_t)b * 3 * g.H * g.W, g.H, g.W, g.n0x, i, v);
   bb_read_candidate(gt, gt2, gt4, g, b, j, w);
-  const float scale = __ldg(grad_out) / ((float)g.B * (float)g.N * (float)BB_D);
+  const float scale = patch_grad_scale<PER_IMG>(grad_out, b, g.B, g.N, (float)BB_D);
 #pragma unroll
   for (int e = 0; e < BB_D; ++e) {
     const float d = w[e] - v[e];
@@ -968,7 +997,8 @@ bb_pyramid_adjoint_kernel(const float* __restrict__ d2, const float* __restrict_
 // One thread per patch; every pixel covered by a patch belongs to exactly one, the rest stay 0.
 // TO_GT: the same formula with the roles swapped (v = the selected candidate, differentiated; w = the SR patch), the
 // result accumulated into the candidate's level image (d_sr = level 0 = d_gt, d2, d4).
-template <bool TO_GT = false>
+// PER_IMG: reduction='none', grad_out is [B] (patch_grad_scale)
+template <bool TO_GT = false, bool PER_IMG = false>
 __global__ void __launch_bounds__(256)
 gram_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                      const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -988,7 +1018,7 @@ gram_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt,
   }
   bb_gram(v, g1);
   bb_gram(w, gs);
-  const float scale = __ldg(grad_out) / ((float)g.B * (float)g.N * 9.0f);
+  const float scale = patch_grad_scale<PER_IMG>(grad_out, b, g.B, g.N, 9.0f);
   float dG[9];
 #pragma unroll
   for (int k = 0; k < 9; ++k) {
@@ -1017,7 +1047,8 @@ gram_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt,
 //   dJxx = dDxx/q + ddet*Jyy , dJyy = dDyy/q + ddet*Jxx , dJxy = dDxy/q - 2 ddet*Jxy
 // then the adjoint 3x3 smoothing, the product rule dIx = 2 Ix dPxx + Iy dPxy, dIy = 2 Iy dPyy + Ix dPxy,
 // the adjoint derivative filters and the grayscale weights.  One thread per patch.
-template <bool TO_GT = false>  // TO_GT: roles swapped and scatter-add into the candidate's level image, as in gram_backward_kernel
+// TO_GT: roles swapped and scatter-add into the candidate's level image, as in gram_backward_kernel; PER_IMG: as there
+template <bool TO_GT = false, bool PER_IMG = false>
 __global__ void __launch_bounds__(128)
 pst_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                     const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -1038,7 +1069,7 @@ pst_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, 
   pst_descriptor(w, tp, dsel);
   PstState S;
   pst_state(v, tp, S);
-  const float scale = __ldg(grad_out) / ((float)g.B * (float)g.N * (float)BB_D);
+  const float scale = patch_grad_scale<PER_IMG>(grad_out, b, g.B, g.N, (float)BB_D);
   float dJ[3][9];
 #pragma unroll
   for (int p = 0; p < 9; ++p) {

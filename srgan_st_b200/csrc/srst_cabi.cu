@@ -194,10 +194,11 @@ static bool make_plane_map(SrstTmap* map, const float* base, long long planes, i
 #endif
 }
 
-template <class C, bool PX, bool HR> struct FwdTag {};  // once-flag tag per forward instantiation
-template <class C, bool PX> struct BwdTag {};
+// once-flag tag per forward / backward instantiation (PI: the per-image reduction, reduction='none')
+template <class C, bool PX, bool HR, bool PI = false> struct FwdTag {};
+template <class C, bool PX, bool PI = false> struct BwdTag {};
 
-template <class C, bool PX = false>
+template <class C, bool PX = false, bool PI = false>
 static int launch_st_forward(StFwdParams<C::RG, C::RK>& P, void* stream) {
   P.tiles_x = (P.W + C::TW - 1) / C::TW;
   P.tiles_y = (P.H + C::TH - 1) / C::TH;
@@ -205,11 +206,11 @@ static int launch_st_forward(StFwdParams<C::RG, C::RK>& P, void* stream) {
   if (ntiles <= 0 || ntiles > 0x7fffffffLL) return SRST_E_SHAPE;
   int e;
   if (P.ds_hr) {
-    if ((e = ensure_smem<FwdTag<C, PX, true>>(st_forward_kernel<C, PX, true>, C::SMEM_BYTES)) != 0) return e;
-    SRST_LAUNCH_PDL((st_forward_kernel<C, PX, true>), dim3((unsigned)ntiles), dim3(C::NT), C::SMEM_BYTES, stream, P);
+    if ((e = ensure_smem<FwdTag<C, PX, true, PI>>(st_forward_kernel<C, PX, true, PI>, C::SMEM_BYTES)) != 0) return e;
+    SRST_LAUNCH_PDL((st_forward_kernel<C, PX, true, PI>), dim3((unsigned)ntiles), dim3(C::NT), C::SMEM_BYTES, stream, P);
   } else {
-    if ((e = ensure_smem<FwdTag<C, PX, false>>(st_forward_kernel<C, PX, false>, C::SMEM_BYTES)) != 0) return e;
-    SRST_LAUNCH_PDL((st_forward_kernel<C, PX, false>), dim3((unsigned)ntiles), dim3(C::NT), C::SMEM_BYTES, stream, P);
+    if ((e = ensure_smem<FwdTag<C, PX, false, PI>>(st_forward_kernel<C, PX, false, PI>, C::SMEM_BYTES)) != 0) return e;
+    SRST_LAUNCH_PDL((st_forward_kernel<C, PX, false, PI>), dim3((unsigned)ntiles), dim3(C::NT), C::SMEM_BYTES, stream, P);
   }
   return (int)cudaGetLastError();
 }
@@ -218,8 +219,8 @@ static int launch_st_forward(StFwdParams<C::RG, C::RK>& P, void* stream) {
 // tiled shape).  Chunking: whole strips when B * strips already fills the machine, otherwise each strip is cut
 // into as many row chunks as there are idle SMs (a chunk costs one extra 16-row block of gradient + horizontal work).
 constexpr int kMarchUnusable = -1000;
-template <class C, bool PX, bool HR> struct MarchTag {};
-template <class C, bool PX = false>
+template <class C, bool PX, bool HR, bool PI = false> struct MarchTag {};
+template <class C, bool PX = false, bool PI = false>
 static int launch_st_march(const StFwdParams<C::RG, C::RK>& F, void* stream) {
   static thread_local StMarchParams<C::RG, C::RK> MP_tls;
   auto& MP = MP_tls;  // a plain reference: the emulation's kernel threads must see THIS thread's instance
@@ -243,16 +244,16 @@ static int launch_st_march(const StFwdParams<C::RG, C::RK>& F, void* stream) {
   if (grid <= 0 || grid > 0x7fffffffLL) return SRST_E_SHAPE;
   int e;
   if (F.ds_hr) {
-    if ((e = ensure_smem<MarchTag<C, PX, true>>(st_forward_march_kernel<C, PX, true>, C::SMEM_BYTES)) != 0) return e;
-    SRST_LAUNCH_PDL((st_forward_march_kernel<C, PX, true>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, MP);
+    if ((e = ensure_smem<MarchTag<C, PX, true, PI>>(st_forward_march_kernel<C, PX, true, PI>, C::SMEM_BYTES)) != 0) return e;
+    SRST_LAUNCH_PDL((st_forward_march_kernel<C, PX, true, PI>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, MP);
   } else {
-    if ((e = ensure_smem<MarchTag<C, PX, false>>(st_forward_march_kernel<C, PX, false>, C::SMEM_BYTES)) != 0) return e;
-    SRST_LAUNCH_PDL((st_forward_march_kernel<C, PX, false>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, MP);
+    if ((e = ensure_smem<MarchTag<C, PX, false, PI>>(st_forward_march_kernel<C, PX, false, PI>, C::SMEM_BYTES)) != 0) return e;
+    SRST_LAUNCH_PDL((st_forward_march_kernel<C, PX, false, PI>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, MP);
   }
   return (int)cudaGetLastError();
 }
 
-template <class C, bool PX = false>
+template <class C, bool PX = false, bool PI = false>
 static int launch_st_backward(StBwdParams<C::RG, C::RK>& P, void* stream) {
   static const bool tma_env = env_int_once("SRST_ST_BWD_TMA", 1) != 0;
   const int Hp = (P.H + 1) / 2;
@@ -263,14 +264,14 @@ static int launch_st_backward(StBwdParams<C::RG, C::RK>& P, void* stream) {
   P.tiles_y = (P.H + C::TH - 1) / C::TH;
   const long long nblk = (long long)P.B * P.tiles_x * P.tiles_y;
   if (nblk <= 0 || nblk > 0x7fffffffLL) return SRST_E_SHAPE;
-  int e = ensure_smem<BwdTag<C, PX>>(st_backward_kernel<C, PX>, C::SMEM_BYTES);
+  int e = ensure_smem<BwdTag<C, PX, PI>>(st_backward_kernel<C, PX, PI>, C::SMEM_BYTES);
   if (e) return e;
   long long grid = nblk;
   if (C::PIPE && P.use_tma) {  // persistent: one wave of resident CTAs, each looping over tiles
     const long long slots = (long long)sm_count() * C::MINB;
     if (grid > slots) grid = slots;
   }
-  SRST_LAUNCH_PDL((st_backward_kernel<C, PX>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, P);
+  SRST_LAUNCH_PDL((st_backward_kernel<C, PX, PI>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, P);
   return (int)cudaGetLastError();
 }
 
@@ -396,6 +397,7 @@ struct StCall {
   const float *sr = nullptr, *hr = nullptr, *ixy = nullptr, *ds = nullptr, *grad_out = nullptr;
   float *ds_sr = nullptr, *ds_hr = nullptr, *ixy_sr = nullptr, *ixy_hr = nullptr, *loss_out = nullptr, *d_img = nullptr;
   int px = 0;                                            // forward: also reduce the fused Pixel (MSE) term into loss_out[1]
+  int per_image = 0;                                     // reduction='none': loss_out / grad_out are [B] (no Pixel term)
   const float *px_img = nullptr, *px_other = nullptr, *grad_px = nullptr;  // backward: image pair + upstream gradient of the MSE term
   int B = 0, H = 0, W = 0, normalize = 1, vec4 = 0;
   float eps = 0.f;
@@ -416,18 +418,28 @@ static int st_forward_rr(const StCall& c) {
   P.loss_out = c.loss_out;
   P.B = c.B; P.H = c.H; P.W = c.W; P.tiles_x = P.tiles_y = 0;
   P.normalize = c.normalize; P.vec4 = c.vec4; P.eps = c.eps;
-  P.inv_count = (float)(1.0 / ((double)c.B * c.H * c.W));
+  P.inv_count = (float)(1.0 / ((double)(c.per_image ? 1 : c.B) * c.H * c.W));
   P.taps = cached_taps<RG, RK>(c.g, c.dg, c.rs, c.k, c.rk);
   if constexpr (RG == 2 && RK == 8) {
     const int mcfg = pick_march_cfg(c.W);
     if (mcfg >= 0) {
       int e;
-      if (mcfg == kFwdMarch96) e = c.px ? launch_st_march<March96, true>(P, c.stream) : launch_st_march<March96>(P, c.stream);
+      if (c.per_image)
+        e = mcfg == kFwdMarch96 ? launch_st_march<March96, false, true>(P, c.stream)
+                                : launch_st_march<March112, false, true>(P, c.stream);
+      else if (mcfg == kFwdMarch96) e = c.px ? launch_st_march<March96, true>(P, c.stream) : launch_st_march<March96>(P, c.stream);
       else e = c.px ? launch_st_march<March112, true>(P, c.stream) : launch_st_march<March112>(P, c.stream);
       if (e != kMarchUnusable) return e;
     }
     int cfg = pick_fwd_cfg(c.B, c.H, c.W);
     if (cfg >= kFwdMarch96) cfg = (c.W <= 96) ? 1 : 0;  // a marching shape was forced but TMA cannot fetch these tensors
+    if (c.per_image) {
+      switch (cfg) {
+        case 1: return launch_st_forward<Fwd1, false, true>(P, c.stream);
+        case 2: return launch_st_forward<Fwd2, false, true>(P, c.stream);
+        default: return launch_st_forward<Fwd0, false, true>(P, c.stream);
+      }
+    }
     if (c.px) {  // the fused Pixel term is compiled into the two default tile shapes only
       if (cfg != 0 && c.W <= 96) return launch_st_forward<Fwd1, true>(P, c.stream);
       return launch_st_forward<Fwd0, true>(P, c.stream);
@@ -439,6 +451,7 @@ static int st_forward_rr(const StCall& c) {
     }
   } else {
     using G = StFwdCfg<32, 64, 16, 4, RG, RK, (RK <= 8 ? 2 : 1), 0>;
+    if (c.per_image) return launch_st_forward<G, false, true>(P, c.stream);
     return c.px ? launch_st_forward<G, true>(P, c.stream) : launch_st_forward<G>(P, c.stream);
   }
 }
@@ -451,17 +464,19 @@ static int st_backward_rr(const StCall& c) {
   P.img = c.px_img; P.px_other = c.px_other; P.grad_px = c.grad_px;
   P.B = c.B; P.H = c.H; P.W = c.W; P.tiles_x = P.tiles_y = 0;
   P.vec4 = c.vec4;
-  P.inv_count = (float)(1.0 / ((double)c.B * c.H * c.W));
+  P.inv_count = (float)(1.0 / ((double)(c.per_image ? 1 : c.B) * c.H * c.W));
   P.taps = cached_taps<RG, RK>(c.g, c.dg, c.rs, c.k, c.rk);
   if constexpr (RG == 2 && RK == 8) {
     if (c.px_other) {  // the fused Pixel term is compiled into the two default tile shapes
       if (c.W <= 96) return launch_st_backward<Bwd1, true>(P, c.stream);
       return launch_st_backward<Bwd0, true>(P, c.stream);
     }
-    if (pick_bwd_cfg(c.B, c.H, c.W) == 1) return launch_st_backward<Bwd1>(P, c.stream);
-    return launch_st_backward<Bwd0>(P, c.stream);
+    if (pick_bwd_cfg(c.B, c.H, c.W) == 1)
+      return c.per_image ? launch_st_backward<Bwd1, false, true>(P, c.stream) : launch_st_backward<Bwd1>(P, c.stream);
+    return c.per_image ? launch_st_backward<Bwd0, false, true>(P, c.stream) : launch_st_backward<Bwd0>(P, c.stream);
   } else {
     using G = StBwdCfg<24, 64, (24 + 2 * RG) / 2, 256, RG, RK, (RK <= 8 ? 2 : 1), 4>;
+    if (c.per_image) return launch_st_backward<G, false, true>(P, c.stream);
     return c.px_other ? launch_st_backward<G, true>(P, c.stream) : launch_st_backward<G>(P, c.stream);
   }
 }
@@ -508,9 +523,24 @@ static int st_forward_generic(const StCall& c, size_t workspace_bytes) {
   Q.s1 = S[0]; Q.s2 = S[1]; Q.ds_sr = c.ds_sr; Q.ds_hr = c.ds_hr; Q.partials = partials;
   Q.ticket = reinterpret_cast<unsigned int*>(c.workspace); Q.loss_out = c.loss_out;
   Q.B = c.B; Q.H = c.H; Q.W = c.W; Q.normalize = c.normalize; Q.eps = c.eps;
+  if (c.per_image) {
+    // CTAs that each stay inside one image, image-major; their partials go where the compiled classes keep theirs
+    // (B * ceil(H/16) * ceil(W/48) slots after the ticket), so any B fits
+    const size_t plane_blocks = ((size_t)c.H * c.W + kGenNT - 1) / kGenNT;
+    const size_t slots = (size_t)((c.H + kMinFwdTH - 1) / kMinFwdTH) * ((c.W + kMinFwdTW - 1) / kMinFwdTW);
+    size_t per = (size_t)kGenMaxPartials / (size_t)c.B;
+    per = per < 1 ? 1 : per;
+    per = per < plane_blocks ? per : plane_blocks;
+    per = per < slots ? per : slots;
+    if ((size_t)c.B * per > 0x7fffffffULL) return SRST_E_SHAPE;
+    Q.partials = reinterpret_cast<float*>(c.workspace) + 4;
+    Q.inv_count = (float)(1.0 / ((double)c.H * c.W));
+    SRST_LAUNCH(gen_chain_kernel<true>, dim3((unsigned)(c.B * per)), dim3(kGenNT), 0, c.stream, Q);
+    return (int)cudaGetLastError();
+  }
   Q.inv_count = (float)(1.0 / ((double)c.B * c.H * c.W));
   const unsigned ngrid = nblk < (unsigned)kGenMaxPartials ? nblk : (unsigned)kGenMaxPartials;
-  SRST_LAUNCH(gen_chain_kernel, dim3(ngrid), dim3(kGenNT), 0, c.stream, Q);
+  SRST_LAUNCH(gen_chain_kernel<false>, dim3(ngrid), dim3(kGenNT), 0, c.stream, Q);
   return (int)cudaGetLastError();
 }
 
@@ -527,7 +557,7 @@ static int st_backward_generic(const StCall& c, void* workspace, size_t workspac
   static thread_local StGenParams P_tls;
   StGenParams& P = P_tls;
   P.B = c.B; P.H = c.H; P.W = c.W;
-  P.scale = (float)(1.0 / ((double)c.B * c.H * c.W));
+  P.scale = (float)(1.0 / ((double)(c.per_image ? 1 : c.B) * c.H * c.W));
   gen_fill_taps(P.taps, c);
   const unsigned nblk = (unsigned)((npix + kGenNT - 1) / kGenNT);
   P.in0 = c.ds; P.in1 = P.in2 = nullptr; P.out0 = V; P.out1 = nullptr;
@@ -537,7 +567,8 @@ static int st_backward_generic(const StCall& c, void* workspace, size_t workspac
   P.in0 = DI; P.in1 = nullptr; P.out0 = V;
   SRST_LAUNCH(gen_bwd_gh_kernel, dim3(nblk), dim3(kGenNT), 0, c.stream, P);
   P.in0 = V; P.in1 = c.grad_out; P.out0 = c.d_img;
-  SRST_LAUNCH(gen_bwd_gv_kernel, dim3(nblk), dim3(kGenNT), 0, c.stream, P);
+  if (c.per_image) SRST_LAUNCH(gen_bwd_gv_kernel<true>, dim3(nblk), dim3(kGenNT), 0, c.stream, P);
+  else SRST_LAUNCH(gen_bwd_gv_kernel<false>, dim3(nblk), dim3(kGenNT), 0, c.stream, P);
   return (int)cudaGetLastError();
 }
 
@@ -553,12 +584,11 @@ static int st_dispatch(const StCall& c, bool forward) {
 
 }  // namespace srst
 
-extern "C" {
-
-int srst_st_forward(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
-                    int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss_out,
-                    float* ds_sr, float* ds_hr, float* ixy_sr, float* ixy_hr, void* workspace,
-                    size_t workspace_bytes, void* stream) {
+// srst_st_forward and srst_st_forward_per_image: the same checks and dispatch; per_image selects the [B] reduction
+static int st_forward_entry(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
+                            int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss_out,
+                            float* ds_sr, float* ds_hr, float* ixy_sr, float* ixy_hr, void* workspace,
+                            size_t workspace_bytes, void* stream, int per_image) {
   if (!sr || !hr || !g || !dg || !k || !loss_out || B <= 0 || H <= 0 || W <= 0) return SRST_E_INVALID;
   if (!srst_st_supported(r_sigma, r_rho)) return SRST_E_UNSUPPORTED;
   if (!workspace || !aligned16(workspace) || workspace_bytes < srst_st_workspace_bytes(B, H, W))
@@ -569,13 +599,14 @@ int srst_st_forward(const float* sr, const float* hr, int B, int H, int W, const
   c.vec4 = (W % 4 == 0 && aligned16(sr) && aligned16(hr) && (!ds_sr || aligned16(ds_sr)) &&
             (!ds_hr || aligned16(ds_hr)) && (!ixy_sr || aligned16(ixy_sr)) && (!ixy_hr || aligned16(ixy_hr))) ? 1 : 0;
   c.workspace = workspace; c.g = g; c.dg = dg; c.k = k; c.rs = r_sigma; c.rk = r_rho; c.stream = stream;
+  c.per_image = per_image;
   if (!st_compiled(r_sigma, r_rho)) return st_forward_generic(c, workspace_bytes);
   return st_dispatch(c, true);
 }
 
-int srst_st_backward_ws(const float* ixy, const float* ds, const float* grad_out, int B, int H, int W,
-                        const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float* d_img,
-                        void* workspace, size_t workspace_bytes, void* stream) {
+static int st_backward_entry(const float* ixy, const float* ds, const float* grad_out, int B, int H, int W,
+                             const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float* d_img,
+                             void* workspace, size_t workspace_bytes, void* stream, int per_image) {
   if (!ixy || !ds || !grad_out || !g || !dg || !k || !d_img || B <= 0 || H <= 0 || W <= 0) return SRST_E_INVALID;
   if (!srst_st_supported(r_sigma, r_rho)) return SRST_E_UNSUPPORTED;
   StCall c;
@@ -583,8 +614,41 @@ int srst_st_backward_ws(const float* ixy, const float* ds, const float* grad_out
   c.B = B; c.H = H; c.W = W;
   c.vec4 = (W % 4 == 0 && aligned16(d_img) && aligned16(ds)) ? 1 : 0;
   c.g = g; c.dg = dg; c.k = k; c.rs = r_sigma; c.rk = r_rho; c.stream = stream;
+  c.per_image = per_image;
   if (!st_compiled(r_sigma, r_rho)) return st_backward_generic(c, workspace, workspace_bytes);
   return st_dispatch(c, false);
+}
+
+extern "C" {
+
+int srst_st_forward(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
+                    int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss_out,
+                    float* ds_sr, float* ds_hr, float* ixy_sr, float* ixy_hr, void* workspace,
+                    size_t workspace_bytes, void* stream) {
+  return st_forward_entry(sr, hr, B, H, W, g, dg, r_sigma, k, r_rho, normalize, eps, loss_out, ds_sr, ds_hr, ixy_sr,
+                          ixy_hr, workspace, workspace_bytes, stream, 0);
+}
+
+int srst_st_forward_per_image(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
+                              int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss_out,
+                              float* ds_sr, float* ds_hr, float* ixy_sr, float* ixy_hr, void* workspace,
+                              size_t workspace_bytes, void* stream) {
+  return st_forward_entry(sr, hr, B, H, W, g, dg, r_sigma, k, r_rho, normalize, eps, loss_out, ds_sr, ds_hr, ixy_sr,
+                          ixy_hr, workspace, workspace_bytes, stream, 1);
+}
+
+int srst_st_backward_ws(const float* ixy, const float* ds, const float* grad_out, int B, int H, int W,
+                        const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float* d_img,
+                        void* workspace, size_t workspace_bytes, void* stream) {
+  return st_backward_entry(ixy, ds, grad_out, B, H, W, g, dg, r_sigma, k, r_rho, d_img, workspace, workspace_bytes,
+                           stream, 0);
+}
+
+int srst_st_backward_per_image(const float* ixy, const float* ds, const float* grad_out, int B, int H, int W,
+                               const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float* d_img,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+  return st_backward_entry(ixy, ds, grad_out, B, H, W, g, dg, r_sigma, k, r_rho, d_img, workspace, workspace_bytes,
+                           stream, 1);
 }
 
 int srst_st_backward(const float* ixy, const float* ds, const float* grad_out, int B, int H, int W,
@@ -728,7 +792,8 @@ static int zero_fill(float* p, size_t n, void* stream) {
 #endif
 }
 
-template <int MODE>
+// PI: reduction='none' (srst_patch_forward_per_image): loss_out is [B]
+template <int MODE, bool PI = false>
 static int bb_forward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W,
                            float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out, void* workspace,
                            size_t workspace_bytes, void* stream, const PstTaps& tp = PstTaps{}) {
@@ -757,6 +822,16 @@ static int bb_forward_impl(const float* sr, const float* gt, const float* gt2, c
                 alpha, beta, idx_out);
   }
   if ((e = (int)cudaGetLastError()) != 0) return e;
+  if constexpr (PI) {
+    // ceil(N / BB_NT) CTAs per image, so that none spans two images.  That can be more CTAs than w.partials has slots
+    // for; their partials go over the library's own x1/2 pyramid level instead (the loss kernel reads only the
+    // descriptor matrices, and every backward entry point rebuilds that level).  It holds 3 (H/2)(W/2) >= N / 256 + 1
+    // floats per image.
+    const unsigned per = (unsigned)((g.N + BB_NT - 1) / BB_NT);
+    SRST_LAUNCH((bb_loss_kernel<D, true>), dim3(per * (unsigned)B), dim3(BB_NT), 0, stream, w.mats, w.per_image, g, idx_out,
+                criterion, w.pyr2, w.ticket, loss_out);
+    return (int)cudaGetLastError();
+  }
   const unsigned nl = (unsigned)(((size_t)B * g.N + BB_NT - 1) / BB_NT);
   SRST_LAUNCH(bb_loss_kernel<D>, dim3(nl), dim3(BB_NT), 0, stream, w.mats, w.per_image, g, idx_out, criterion,
               w.partials, w.ticket, loss_out);
@@ -796,7 +871,8 @@ static int pst_taps(const float* g, const float* dg, int r_sigma, const float* k
   return 0;
 }
 
-template <int MODE>
+// PI: reduction='none' (srst_patch_backward_per_image): grad_out is [B]
+template <int MODE, bool PI = false>
 static int patch_backward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
                                const float* grad_out, int B, int H, int W, int criterion, float* d_sr, void* workspace,
                                size_t workspace_bytes, void* stream, const PstTaps& tp = PstTaps{}) {
@@ -813,17 +889,17 @@ static int patch_backward_impl(const float* sr, const float* gt, const float* gt
   }
   if constexpr (MODE == 0) {  // one thread per pixel of d_sr
     const size_t total = (size_t)B * 3 * H * W;
-    SRST_LAUNCH(bb_backward_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
+    SRST_LAUNCH(bb_backward_kernel<PI>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
                 grad_out, g, criterion, d_sr);
   } else {  // one thread per patch: pixels outside every patch keep a zero gradient
     if ((H % 3 != 0 || W % 3 != 0) && (e = zero_fill(d_sr, (size_t)B * 3 * H * W, stream)) != 0) return e;
     const size_t total = (size_t)B * g.N;
     if constexpr (MODE == 1)
-      SRST_LAUNCH(gram_backward_kernel<false>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4,
-                  idx, grad_out, g, criterion, d_sr, nullptr, nullptr);
+      SRST_LAUNCH((gram_backward_kernel<false, PI>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2,
+                  gt4, idx, grad_out, g, criterion, d_sr, nullptr, nullptr);
     else
-      SRST_LAUNCH(pst_backward_kernel<false>, dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt, gt2, gt4,
-                  idx, grad_out, g, tp, criterion, d_sr, nullptr, nullptr);
+      SRST_LAUNCH((pst_backward_kernel<false, PI>), dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt, gt2,
+                  gt4, idx, grad_out, g, tp, criterion, d_sr, nullptr, nullptr);
   }
   return (int)cudaGetLastError();
 }
@@ -866,10 +942,14 @@ int srst_pst_backward(const float* sr, const float* gt, const float* gt2, const 
                                 stream, tp);
 }
 
-int srst_patch_backward_gt(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
-                           const int64_t* idx, const float* grad_out, int B, int H, int W, const float* g, const float* dg,
-                           int r_sigma, const float* k, int r_rho, int criterion, float* d_gt, void* workspace,
-                           size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// srst_patch_backward_gt, and the d_gt half of srst_patch_backward_per_image (PI: grad_out is [B])
+template <bool PI>
+static int patch_backward_gt_impl(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                                  const int64_t* idx, const float* grad_out, int B, int H, int W, const float* g,
+                                  const float* dg, int r_sigma, const float* k, int r_rho, int criterion, float* d_gt,
+                                  void* workspace, size_t workspace_bytes, void* stream) {
   if (!sr || !gt || !idx || !grad_out || !d_gt || B <= 0 || mode < 0 || mode > 2) return SRST_E_INVALID;
   bool dist_l1;
   int e = bb_check(criterion, dist_l1, B, H, W, gt2, gt4);
@@ -890,17 +970,72 @@ int srst_patch_backward_gt(int mode, const float* sr, const float* gt, const flo
   SRST_LAUNCH(bb_fill_zero_kernel, dim3(fill_grid((n2 + 3) / 4 * 4 + n4, 148)), dim3(256), 0, stream, d2, (n2 + 3) / 4 * 4 + n4);
   const size_t total = (size_t)B * gm.N;
   if (mode == 0)
-    SRST_LAUNCH(bb_backward_gt_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
+    SRST_LAUNCH(bb_backward_gt_kernel<PI>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
                 grad_out, gm, criterion, d_gt, d2, d4);
   else if (mode == 1)
-    SRST_LAUNCH(gram_backward_kernel<true>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4,
-                idx, grad_out, gm, criterion, d_gt, d2, d4);
+    SRST_LAUNCH((gram_backward_kernel<true, PI>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2,
+                gt4, idx, grad_out, gm, criterion, d_gt, d2, d4);
   else
-    SRST_LAUNCH(pst_backward_kernel<true>, dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt, gt2, gt4,
-                idx, grad_out, gm, tp, criterion, d_gt, d2, d4);
+    SRST_LAUNCH((pst_backward_kernel<true, PI>), dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt, gt2,
+                gt4, idx, grad_out, gm, tp, criterion, d_gt, d2, d4);
   SRST_LAUNCH(bb_pyramid_adjoint_kernel, dim3((unsigned)((n2 + n4 + 255) / 256)), dim3(256), 0, stream, d2, d4, d_gt, B * 3,
               H, W, gm.H2, gm.W2, gm.H4, gm.W4);
   return (int)cudaGetLastError();
+}
+
+extern "C" {
+
+int srst_patch_backward_gt(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                           const int64_t* idx, const float* grad_out, int B, int H, int W, const float* g, const float* dg,
+                           int r_sigma, const float* k, int r_rho, int criterion, float* d_gt, void* workspace,
+                           size_t workspace_bytes, void* stream) {
+  return patch_backward_gt_impl<false>(mode, sr, gt, gt2, gt4, idx, grad_out, B, H, W, g, dg, r_sigma, k, r_rho, criterion,
+                                       d_gt, workspace, workspace_bytes, stream);
+}
+
+int srst_patch_forward_per_image(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4, int B,
+                                 int H, int W, const float* g, const float* dg, int r_sigma, const float* k, int r_rho,
+                                 float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out,
+                                 void* workspace, size_t workspace_bytes, void* stream) {
+  switch (mode) {
+    case 0:
+      return bb_forward_impl<0, true>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
+                                      workspace_bytes, stream);
+    case 1:
+      return bb_forward_impl<1, true>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
+                                      workspace_bytes, stream);
+    case 2: {
+      PstTaps tp;
+      const int e = pst_taps(g, dg, r_sigma, k, r_rho, tp);
+      if (e) return e;
+      return bb_forward_impl<2, true>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
+                                      workspace_bytes, stream, tp);
+    }
+    default: return SRST_E_INVALID;
+  }
+}
+
+int srst_patch_backward_per_image(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                                  const int64_t* idx, const float* grad_out, int B, int H, int W, const float* g,
+                                  const float* dg, int r_sigma, const float* k, int r_rho, int criterion, float* d_sr,
+                                  float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
+  if ((!d_sr && !d_gt) || mode < 0 || mode > 2) return SRST_E_INVALID;
+  int e = 0;
+  if (d_sr) {
+    PstTaps tp;
+    if (mode == 2 && (e = pst_taps(g, dg, r_sigma, k, r_rho, tp)) != 0) return e;
+    if (mode == 0) e = patch_backward_impl<0, true>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace,
+                                                    workspace_bytes, stream);
+    else if (mode == 1) e = patch_backward_impl<1, true>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace,
+                                                         workspace_bytes, stream);
+    else e = patch_backward_impl<2, true>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace,
+                                          workspace_bytes, stream, tp);
+    if (e) return e;
+  }
+  if (d_gt)
+    e = patch_backward_gt_impl<true>(mode, sr, gt, gt2, gt4, idx, grad_out, B, H, W, g, dg, r_sigma, k, r_rho, criterion,
+                                     d_gt, workspace, workspace_bytes, stream);
+  return e;
 }
 
 }  // extern "C"
@@ -931,9 +1066,13 @@ long long srst_bbg_num_patches(int H, int W, int ksize, int pad, int stride) {
   return bbg_geom(1, H, W, ksize, pad, stride).N;
 }
 
-int srst_bbg_forward(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W, int ksize,
-                     int pad, int stride, float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out,
-                     void* workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// srst_bbg_forward / srst_bbg_forward_per_image (PI: loss_out is [B])
+template <bool PI>
+static int bbg_forward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W,
+                            int ksize, int pad, int stride, float alpha, float beta, int criterion, int64_t* idx_out,
+                            float* loss_out, void* workspace, size_t workspace_bytes, void* stream) {
   if (!sr || !gt || !idx_out || !loss_out || B <= 0) return SRST_E_INVALID;
   bool dist_l1;
   int e = bb_criterion(criterion, dist_l1);
@@ -952,15 +1091,25 @@ int srst_bbg_forward(const float* sr, const float* gt, const float* gt2, const f
   SRST_LAUNCH(bbg_search_kernel, dim3((unsigned)((g.N + BBG_QT - 1) / BBG_QT), (unsigned)B), dim3(BBG_NT),
               bbg_search_smem(g.D), stream, sr, gt, w.ymat, w.y_per_image, w.Mpad, g, alpha, beta, dist_l1 ? 1 : 0, idx_out);
   if ((e = (int)cudaGetLastError()) != 0) return e;
+  if constexpr (PI) {
+    // ceil(N / BBG_NT) CTAs per image, so that none spans two images; their partials go over the candidate matrices,
+    // which only the search reads ((D + 1) Mpad >= N floats per image)
+    const unsigned per = (unsigned)((g.N + BBG_NT - 1) / BBG_NT);
+    SRST_LAUNCH(bbg_loss_kernel<true>, dim3(per * (unsigned)B), dim3(BBG_NT), 0, stream, sr, gt, gt2, gt4, g, idx_out,
+                criterion, w.ymat, w.ticket, loss_out);
+    return (int)cudaGetLastError();
+  }
   const unsigned nl = (unsigned)(((size_t)B * g.N + BBG_NT - 1) / BBG_NT);
-  SRST_LAUNCH(bbg_loss_kernel, dim3(nl), dim3(BBG_NT), 0, stream, sr, gt, gt2, gt4, g, idx_out, criterion, w.partials,
+  SRST_LAUNCH(bbg_loss_kernel<false>, dim3(nl), dim3(BBG_NT), 0, stream, sr, gt, gt2, gt4, g, idx_out, criterion, w.partials,
               w.ticket, loss_out);
   return (int)cudaGetLastError();
 }
 
-int srst_bbg_backward(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
-                      const float* grad_out, int B, int H, int W, int ksize, int pad, int stride, int criterion,
-                      float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
+// srst_bbg_backward / srst_bbg_backward_per_image (PI: grad_out is [B])
+template <bool PI>
+static int bbg_backward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
+                             const float* grad_out, int B, int H, int W, int ksize, int pad, int stride, int criterion,
+                             float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
   if (!sr || !gt || !idx || !grad_out || (!d_sr && !d_gt) || B <= 0) return SRST_E_INVALID;
   bool dist_l1;
   int e = bb_criterion(criterion, dist_l1);
@@ -972,7 +1121,7 @@ int srst_bbg_backward(const float* sr, const float* gt, const float* gt2, const 
   if ((e = bbg_prepare(gt, gt2, gt4, B, H, W, g, workspace, workspace_bytes, w, stream)) != 0) return e;
   const size_t n0 = (size_t)B * 3 * H * W;
   if (d_sr) {
-    SRST_LAUNCH(bbg_backward_kernel, dim3((unsigned)((n0 + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
+    SRST_LAUNCH(bbg_backward_kernel<PI>, dim3((unsigned)((n0 + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
                 grad_out, g, criterion, d_sr);
     if ((e = (int)cudaGetLastError()) != 0) return e;
   }
@@ -981,13 +1130,43 @@ int srst_bbg_backward(const float* sr, const float* gt, const float* gt2, const 
     SRST_LAUNCH(bb_fill_zero_kernel, dim3(fill_grid(n0, 592)), dim3(256), 0, stream, d_gt, n0);
     SRST_LAUNCH(bb_fill_zero_kernel, dim3(fill_grid((n2 + 3) / 4 * 4 + n4, 148)), dim3(256), 0, stream, w.d2, (n2 + 3) / 4 * 4 + n4);
     const size_t total = (size_t)B * g.N * 3;
-    SRST_LAUNCH(bbg_backward_gt_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
+    SRST_LAUNCH(bbg_backward_gt_kernel<PI>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
                 grad_out, g, criterion, d_gt, w.d2, w.d4);
     SRST_LAUNCH(bb_pyramid_adjoint_kernel, dim3((unsigned)((n2 + n4 + 255) / 256)), dim3(256), 0, stream, w.d2, w.d4, d_gt,
                 B * 3, H, W, g.L[1].H, g.L[1].W, g.L[2].H, g.L[2].W);
     if ((e = (int)cudaGetLastError()) != 0) return e;
   }
   return 0;
+}
+
+extern "C" {
+
+int srst_bbg_forward(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W, int ksize,
+                     int pad, int stride, float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out,
+                     void* workspace, size_t workspace_bytes, void* stream) {
+  return bbg_forward_impl<false>(sr, gt, gt2, gt4, B, H, W, ksize, pad, stride, alpha, beta, criterion, idx_out, loss_out,
+                                 workspace, workspace_bytes, stream);
+}
+
+int srst_bbg_forward_per_image(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W,
+                               int ksize, int pad, int stride, float alpha, float beta, int criterion, int64_t* idx_out,
+                               float* loss_out, void* workspace, size_t workspace_bytes, void* stream) {
+  return bbg_forward_impl<true>(sr, gt, gt2, gt4, B, H, W, ksize, pad, stride, alpha, beta, criterion, idx_out, loss_out,
+                                workspace, workspace_bytes, stream);
+}
+
+int srst_bbg_backward(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
+                      const float* grad_out, int B, int H, int W, int ksize, int pad, int stride, int criterion,
+                      float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
+  return bbg_backward_impl<false>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, ksize, pad, stride, criterion, d_sr, d_gt,
+                                  workspace, workspace_bytes, stream);
+}
+
+int srst_bbg_backward_per_image(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
+                                const float* grad_out, int B, int H, int W, int ksize, int pad, int stride, int criterion,
+                                float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
+  return bbg_backward_impl<true>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, ksize, pad, stride, criterion, d_sr, d_gt,
+                                 workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

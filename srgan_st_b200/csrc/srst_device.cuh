@@ -291,4 +291,23 @@ SRST_DEV float warp_sum(float v) {
   return v;
 }
 
+// Per-image form of the deterministic loss reduction (reduction='none'), run by every thread of the CTA that drew
+// the last ticket.  The grid is laid out image-major, so partials[b * per .. (b + 1) * per) are image b's CTAs: one
+// warp per image sums them in double in a fixed order (lane-strided, then a fixed shuffle tree), zeroes them again and
+// writes out[b] = sum * scale.
+SRST_DEV void reduce_partials_per_image(float* partials, int B, unsigned int per, double scale, float* out) {
+  const int lane = threadIdx.x & 31;
+  for (int b = threadIdx.x >> 5; b < B; b += blockDim.x >> 5) {
+    float* p = partials + (size_t)b * per;
+    double acc = 0.0;
+    for (unsigned int i = lane; i < per; i += 32) {
+      acc += (double)__ldcg(p + i);
+      p[i] = 0.f;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (lane == 0) out[b] = (float)(acc * scale);
+  }
+}
+
 }  // namespace srst

@@ -142,24 +142,38 @@ struct StGenChainParams {
   float eps, inv_count;
 };
 
+// chain of pixel i (flat over [B][H][W]): adds its distance to lsum, writes its ds_sr / ds_hr
+SRST_DEV void gen_chain_pixel(const StGenChainParams& P, size_t i, size_t plane, float& lsum) {
+  const size_t b = i / plane, o = b * 3 * plane + (i - b * plane);
+  const float a = __ldg(P.s1 + o), bb = __ldg(P.s1 + o + plane), c = __ldg(P.s1 + o + 2 * plane);
+  const float e = __ldg(P.s2 + o), f = __ldg(P.s2 + o + plane), h = __ldg(P.s2 + o + 2 * plane);
+  StPixelGrad2 G;
+  G.da = G.db = G.dc = G.de = G.df = G.dh = make_float2(0.f, 0.f);
+  const float2 d = st_pixel2_raw<true, true>(bcast2(a), bcast2(bb), bcast2(c), bcast2(e), bcast2(f), bcast2(h),
+                                            P.normalize != 0, P.eps, G);
+  lsum += d.x;
+  if (P.ds_sr) { P.ds_sr[o] = G.da.x; P.ds_sr[o + plane] = G.db.x; P.ds_sr[o + 2 * plane] = G.dc.x; }
+  if (P.ds_hr) { P.ds_hr[o] = G.de.x; P.ds_hr[o + plane] = G.df.x; P.ds_hr[o + 2 * plane] = G.dh.x; }
+}
+
 // per-pixel chain (utils.py:236-279) and its adjoint on both tensors; deterministic loss reduction (CTA partial ->
-// workspace, last CTA sums in a fixed order in double and hands the ticket back zeroed)
+// workspace, last CTA sums in a fixed order in double and hands the ticket back zeroed).
+// PER_IMG: reduction='none' -- the grid is gridDim.x / B CTAs per image, image-major, each striding over its own
+// image only; loss_out[b] = the mean over image b's pixels (P.inv_count = 1 / (H W)).
+template <bool PER_IMG = false>
 __global__ void __launch_bounds__(kGenNT) gen_chain_kernel(const __grid_constant__ StGenChainParams P) {
   __shared__ float s_red[kGenNT / 32];
   __shared__ unsigned int s_last;
   const size_t plane = (size_t)P.H * P.W, npix = (size_t)P.B * plane;
   float lsum = 0.f;
-  for (size_t i = (size_t)blockIdx.x * kGenNT + threadIdx.x; i < npix; i += (size_t)gridDim.x * kGenNT) {
-    const size_t b = i / plane, o = b * 3 * plane + (i - b * plane);
-    const float a = __ldg(P.s1 + o), bb = __ldg(P.s1 + o + plane), c = __ldg(P.s1 + o + 2 * plane);
-    const float e = __ldg(P.s2 + o), f = __ldg(P.s2 + o + plane), h = __ldg(P.s2 + o + 2 * plane);
-    StPixelGrad2 G;
-    G.da = G.db = G.dc = G.de = G.df = G.dh = make_float2(0.f, 0.f);
-    const float2 d = st_pixel2_raw<true, true>(bcast2(a), bcast2(bb), bcast2(c), bcast2(e), bcast2(f), bcast2(h),
-                                              P.normalize != 0, P.eps, G);
-    lsum += d.x;
-    if (P.ds_sr) { P.ds_sr[o] = G.da.x; P.ds_sr[o + plane] = G.db.x; P.ds_sr[o + 2 * plane] = G.dc.x; }
-    if (P.ds_hr) { P.ds_hr[o] = G.de.x; P.ds_hr[o + plane] = G.df.x; P.ds_hr[o + 2 * plane] = G.dh.x; }
+  if constexpr (PER_IMG) {
+    const unsigned int per = gridDim.x / P.B, b = blockIdx.x / per;
+    const size_t end = (size_t)(b + 1) * plane;
+    for (size_t i = (size_t)b * plane + (size_t)(blockIdx.x - b * per) * kGenNT + threadIdx.x; i < end; i += (size_t)per * kGenNT)
+      gen_chain_pixel(P, i, plane, lsum);
+  } else {
+    for (size_t i = (size_t)blockIdx.x * kGenNT + threadIdx.x; i < npix; i += (size_t)gridDim.x * kGenNT)
+      gen_chain_pixel(P, i, plane, lsum);
   }
   lsum = warp_sum(lsum);
   if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = lsum;
@@ -173,7 +187,13 @@ __global__ void __launch_bounds__(kGenNT) gen_chain_kernel(const __grid_constant
     s_last = (tk == gridDim.x - 1) ? 1u : 0u;
   }
   __syncthreads();
-  if (s_last && threadIdx.x < 32) {
+  if constexpr (PER_IMG) {
+    if (s_last) {
+      __threadfence();
+      reduce_partials_per_image(P.partials, P.B, gridDim.x / P.B, (double)P.inv_count, P.loss_out);
+      if (threadIdx.x == 0) *P.ticket = 0u;
+    }
+  } else if (s_last && threadIdx.x < 32) {
     __threadfence();
     double acc = 0.0;
     for (unsigned int i = threadIdx.x; i < gridDim.x; i += 32) acc += (double)__ldcg(P.partials + i);
@@ -247,7 +267,9 @@ __global__ void __launch_bounds__(kGenNT) gen_bwd_gh_kernel(const __grid_constan
 
 // backward: in0 = U1, U2; in1 = grad_out (device scalar) -> out0 = d_img [B,3,H,W]:
 // dgray = -(Ch(dg) U1 + Ch(g) U2) (g symmetric, dg antisymmetric: the adjoint flips the taps), times the upstream
-// gradient / (B H W), spread over the channels with the grayscale weights
+// gradient / (B H W), spread over the channels with the grayscale weights.
+// PER_IMG: in1 = grad_out [B]; pixel of image b scales by grad_out[b] (P.scale = 1 / (H W))
+template <bool PER_IMG = false>
 __global__ void __launch_bounds__(kGenNT) gen_bwd_gv_kernel(const __grid_constant__ StGenParams P) {
   const size_t i = (size_t)blockIdx.x * kGenNT + threadIdx.x;
   int b, y, x;
@@ -261,7 +283,7 @@ __global__ void __launch_bounds__(kGenNT) gen_bwd_gv_kernel(const __grid_constan
     acc = fmaf(P.taps.dg[t + r], __ldg(q), acc);
     acc = fmaf(P.taps.g[t + r], __ldg(q + plane), acc);
   }
-  const float dgr = acc * (-__ldg(P.in1) * P.scale);
+  const float dgr = acc * (-__ldg(P.in1 + (PER_IMG ? b : 0)) * P.scale);
   float* o = P.out0 + (size_t)b * 3 * plane + (size_t)y * P.W + x;
   o[0] = kGrayR * dgr;
   o[plane] = kGrayG * dgr;

@@ -688,9 +688,12 @@ SRST_DEV void st_unit_tensor(float* smem, const float* __restrict__ base, float*
   }
 }
 
-template <class C, bool PX = false, bool WANT_HR = false>
+// PER_IMG: reduction='none' -- loss_out[b] is the mean over image b's pixels (P.inv_count = 1 / (H W)) instead of
+// loss_out[0] over the batch; no fused Pixel term
+template <class C, bool PX = false, bool WANT_HR = false, bool PER_IMG = false>
 __global__ void __launch_bounds__(C::NT, C::MINB)
 st_forward_kernel(const __grid_constant__ StFwdParams<C::RG, C::RK> P) {
+  static_assert(!(PX && PER_IMG), "the fused Pixel term has no per-image reduction");
   SRST_DYN_SMEM(float, smem);
   __shared__ float s_red[32];
   __shared__ unsigned int s_last;
@@ -825,7 +828,13 @@ st_forward_kernel(const __grid_constant__ StFwdParams<C::RG, C::RK> P) {
   }
   __syncthreads();
   SRST_STAMP(10);  // every warp of the CTA is done
-  if (s_last) {
+  if constexpr (PER_IMG) {
+    if (s_last) {  // image-major grid: image b owns tiles_y * tiles_x consecutive CTAs
+      __threadfence();
+      reduce_partials_per_image(P.partials, P.B, gridDim.x / P.B, (double)P.inv_count, P.loss_out);
+      if (tid == 0) *P.ticket = 0u;
+    }
+  } else if (s_last) {
     __threadfence();
     if (tid < 32) {
       double acc = 0.0;
@@ -965,7 +974,9 @@ struct StBwdCfg {
   static_assert((CSD == 4 || CSD == 8) && EW % CSD == 0, "bad phase-D' item width");
 };
 
-template <class C, bool PX = false>
+// PER_IMG: reduction='none' -- grad_out is [B] and the tile of image b scales by grad_out[b] / (H W)
+// (P.inv_count = 1 / (H W)) instead of grad_out[0] / (B H W)
+template <class C, bool PX = false, bool PER_IMG = false>
 __global__ void __launch_bounds__(C::NT, C::MINB)
 st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
   SRST_DYN_SMEM(float, smem);
@@ -1122,7 +1133,7 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
   // correlation with flipped taps; g is symmetric and dg antisymmetric, so
   //   dgray = -[ (dIx * dg|) * g-  +  (dIy * g|) * dg- ]
   // i.e. the forward gradient operators applied to dIx and dIy, negated.
-  const float scale = -__ldg(P.grad_out) * P.inv_count;
+  const float scale = -__ldg(P.grad_out + (PER_IMG ? b : 0)) * P.inv_count;
   [[maybe_unused]] const float px_scale = PX ? __ldg(P.grad_px) * P.inv_count * (2.0f / 3.0f) : 0.f;
   for (int it = tid; it < C::MapE::SLOTS; it += C::NT) {
     int q, seg;

@@ -3,7 +3,8 @@
 ``StructureTensorLoss``, ``BestBuddyLoss``, ``GramLoss`` and ``PatchwiseStructureTensorLoss`` keep the reference's constructor signatures,
 attributes and ``criterion(sr, gt) -> 0-dim fp32 tensor`` contract (reference loss.py:380-413 and
 loss.py:78-141; called from train.py:138 and warmup.py:91), so they register through
-``config.add_g_criterion(name, module, weight)`` (config.py:122-125) unchanged.  Underneath, each is
+``config.add_g_criterion(name, module, weight)`` (config.py:122-125) unchanged.  With the extra keyword
+``reduction='none'`` they return the per-image losses ``[B]`` instead, reduced on the device by the same kernels.  Underneath, each is
 a ``torch.autograd.Function`` whose forward/backward enqueue hand-written CUDA kernels on the
 current stream through the C ABI of ``include/srst.h``.
 
@@ -59,6 +60,17 @@ def _no_gt_grad(gt: torch.Tensor, who: str) -> None:
     the training loops never ask for it (gt comes from the data loader) and libsrst has no kernel for it."""
     if gt.requires_grad and torch.is_grad_enabled():
         raise NotImplementedError(f"{who}: gradient w.r.t. gt is not implemented (pass gt.detach())")
+
+
+def _check_reduction(reduction, who: str) -> str:
+    """'mean' (the reference's batch mean) or 'none' (one loss per image, [B]); anything else raises."""
+    if reduction not in ("mean", "none"):
+        raise ValueError(f"{who}: reduction must be 'mean' or 'none' (got {reduction!r})")
+    return reduction
+
+
+def _reduction_repr(reduction: str) -> str:
+    return "" if reduction == "mean" else f"reduction='{reduction}'"
 
 
 def _ptr(t):
@@ -135,10 +147,11 @@ def _st_taps(sigma: float, rho: float, who: str, compiled_only: bool = False):
 class _StructureTensorLossFn(torch.autograd.Function):
     """autograd boundary of the fused ST loss (the reference lets autograd differentiate ~100
     ATen ops instead; loss.py:399-413).  Saved for backward: per image that needs a gradient, ONE buffer
-    holding the ds planes (12 B/px) followed by the Ix, Iy planes (8 B/px); the images themselves are not."""
+    holding the ds planes (12 B/px) followed by the Ix, Iy planes (8 B/px); the images themselves are not.
+    `per_image`: reduction='none' -- the loss is [B] and the upstream gradient [B] (the *_per_image entry points)."""
 
     @staticmethod
-    def forward(ctx, sr, hr, sigma, rho, normalize):
+    def forward(ctx, sr, hr, sigma, rho, normalize, per_image=False):
         lib = _cabi.lib()
         sr = sr.contiguous()
         hr = hr.contiguous()
@@ -148,26 +161,27 @@ class _StructureTensorLossFn(torch.autograd.Function):
         n_ds, n_ixy, ws_bytes, bws_bytes = _st_sizes(B, H, W, tp[2], tp[4])   # n_ds is padded: the ixy part stays 16-byte aligned
         with _on_device(sr.device):
             stream = _raw_stream(sr.device)
-            loss = torch.empty((), dtype=torch.float32, device=sr.device)
+            loss = torch.empty((B,) if per_image else (), dtype=torch.float32, device=sr.device)
             saved = [torch.empty(n_ds + n_ixy, dtype=torch.float32, device=sr.device) if n else None for n in need[:2]]
             ds = [t.data_ptr() if t is not None else None for t in saved]
             ixy = [p + 4 * n_ds if p is not None else None for p in ds]
             ws = _workspace("st", sr.device, stream, ws_bytes)
-            rc = lib.srst_st_forward(sr.data_ptr(), hr.data_ptr(), B, H, W, tp[0], tp[1], tp[2], tp[3], tp[4],
-                                     int(bool(normalize)), 1e-12, loss.data_ptr(), ds[0], ds[1], ixy[0], ixy[1],
-                                     ws.data_ptr(), ws.numel(), stream)
+            fwd = lib.srst_st_forward_per_image if per_image else lib.srst_st_forward
+            rc = fwd(sr.data_ptr(), hr.data_ptr(), B, H, W, tp[0], tp[1], tp[2], tp[3], tp[4],
+                     int(bool(normalize)), 1e-12, loss.data_ptr(), ds[0], ds[1], ixy[0], ixy[1],
+                     ws.data_ptr(), ws.numel(), stream)
         if rc:
-            _cabi.check(rc, "srst_st_forward")
+            _cabi.check(rc, "srst_st_forward_per_image" if per_image else "srst_st_forward")
         ctx.save_for_backward(saved[0], saved[1])
-        ctx.meta = (tp, B, H, W, n_ds, bws_bytes)
+        ctx.meta = (tp, B, H, W, n_ds, bws_bytes, per_image)
         return loss
 
     @staticmethod
     @once_differentiable
     def backward(ctx, grad_out):
         lib = _cabi.lib()
-        tp, B, H, W, n_ds, bws_bytes = ctx.meta
-        if grad_out.dtype != torch.float32 or not grad_out.is_contiguous():
+        tp, B, H, W, n_ds, bws_bytes, per_image = ctx.meta
+        if grad_out.dtype != torch.float32 or not grad_out.is_contiguous():   # also the stride-0 [B] of .sum() / .mean()
             grad_out = grad_out.to(torch.float32).contiguous()
         outs = [None, None]
         dev = grad_out.device
@@ -177,7 +191,12 @@ class _StructureTensorLossFn(torch.autograd.Function):
                 if saved is None or not ctx.needs_input_grad[i]:
                     continue
                 d_img = torch.empty((B, 3, H, W), dtype=torch.float32, device=dev)
-                if bws_bytes:  # generic-radius path: five scratch planes
+                if per_image:  # one entry point for both paths; the compiled classes need no workspace
+                    ws = _workspace("st_bwd", dev, stream, bws_bytes) if bws_bytes else None
+                    rc = lib.srst_st_backward_per_image(saved.data_ptr() + 4 * n_ds, saved.data_ptr(), grad_out.data_ptr(), B,
+                                                        H, W, tp[0], tp[1], tp[2], tp[3], tp[4], d_img.data_ptr(), _ptr(ws),
+                                                        ws.numel() if ws is not None else 0, stream)
+                elif bws_bytes:  # generic-radius path: five scratch planes
                     ws = _workspace("st_bwd", dev, stream, bws_bytes)
                     rc = lib.srst_st_backward_ws(saved.data_ptr() + 4 * n_ds, saved.data_ptr(), grad_out.data_ptr(), B, H, W,
                                                  tp[0], tp[1], tp[2], tp[3], tp[4], d_img.data_ptr(), ws.data_ptr(),
@@ -188,7 +207,7 @@ class _StructureTensorLossFn(torch.autograd.Function):
                 if rc:
                     _cabi.check(rc, "srst_st_backward")
                 outs[i] = d_img
-        return outs[0], outs[1], None, None, None
+        return outs[0], outs[1], None, None, None, None
 
 
 class StructureTensorLoss(nn.Module):
@@ -196,13 +215,16 @@ class StructureTensorLoss(nn.Module):
 
     ``forward(x, gt)``: x = SR ``[B,3,H,W]``, gt = HR, both fp32 CUDA; returns the mean over all
     pixels of the affine-invariant distance between the det-normalised structure tensors.
+    ``reduction='none'`` returns the ``[B]`` per-image means instead (the reference's ``vmap(st_loss)(x, gt)``
+    before its ``.mean()``, loss.py:411-413), differentiable w.r.t. x and gt.
     """
 
-    def __init__(self, sigma: float = 0.5, rho: float = 2.0, normalize: bool = True):
+    def __init__(self, sigma: float = 0.5, rho: float = 2.0, normalize: bool = True, reduction: str = "mean"):
         super().__init__()
         self.sigma = sigma
         self.rho = rho
         self.normalize = normalize
+        self.reduction = _check_reduction(reduction, "StructureTensorLoss")
         _cabi.lib()  # fail at construction time if the CUDA library is missing
 
     def st_loss(self, x, gt):
@@ -211,10 +233,13 @@ class StructureTensorLoss(nn.Module):
 
     def forward(self, x, gt):
         _check_pair(x, gt, "StructureTensorLoss")
+        if self.reduction == "none":
+            return _StructureTensorLossFn.apply(x, gt, self.sigma, self.rho, self.normalize, True)
         return _StructureTensorLossFn.apply(x, gt, self.sigma, self.rho, self.normalize)
 
     def extra_repr(self) -> str:
-        return f"sigma={self.sigma}, rho={self.rho}, normalize={self.normalize}"
+        r = f"sigma={self.sigma}, rho={self.rho}, normalize={self.normalize}"
+        return r if self.reduction == "mean" else f"{r}, {_reduction_repr(self.reduction)}"
 
 
 def structure_tensor_features(img: torch.Tensor, sigma: float = 0.5, rho: float = 2.0):
@@ -382,10 +407,11 @@ class _PatchLossFn(torch.autograd.Function):
     and, through the gather of the selected candidates, w.r.t. gt (reference loss.py:135-139, :219-222, :369-371); the
     argmin is not.  `loss_cls` is the module class: its _plan / _fwd / _bwd make the C ABI calls that differ per loss.
     `args` holds what they take from the module (weights, criterion, taps, geometry), fixed at forward time: a module
-    changed between forward and backward does not change the gradient."""
+    changed between forward and backward does not change the gradient.  `per_image`: reduction='none' -- the loss and
+    the upstream gradient are [B], and _fwd_none / _bwd_none make the calls."""
 
     @staticmethod
-    def forward(ctx, sr, gt, loss_cls, args, pyramid):
+    def forward(ctx, sr, gt, loss_cls, args, pyramid, per_image=False):
         sr = sr.contiguous()
         gt = gt.contiguous()
         B, _, H, W = sr.shape
@@ -394,10 +420,11 @@ class _PatchLossFn(torch.autograd.Function):
             stream = _raw_stream(sr.device)
             gt2, gt4 = _hr_pyramid(gt, pyramid)
             idx = torch.empty((B, n), dtype=torch.int64, device=sr.device)
-            loss = torch.empty((), dtype=torch.float32, device=sr.device)
-            loss_cls._fwd(args, sr, gt, gt2, gt4, idx, loss, _workspace(kind, sr.device, stream, nbytes), stream)
+            loss = torch.empty((B,) if per_image else (), dtype=torch.float32, device=sr.device)
+            fwd = loss_cls._fwd_none if per_image else loss_cls._fwd
+            fwd(args, sr, gt, gt2, gt4, idx, loss, _workspace(kind, sr.device, stream, nbytes), stream)
         ctx.save_for_backward(sr, gt, gt2, gt4, idx)
-        ctx.meta = (loss_cls, args, kind, nbytes)
+        ctx.meta = (loss_cls, args, kind, nbytes, per_image)
         ctx.mark_non_differentiable(idx)
         return loss, idx
 
@@ -406,29 +433,35 @@ class _PatchLossFn(torch.autograd.Function):
     def backward(ctx, grad_out, _grad_idx):
         need_sr, need_gt = ctx.needs_input_grad[:2]
         if not (need_sr or need_gt):
-            return None, None, None, None, None
+            return None, None, None, None, None, None
         sr, gt, gt2, gt4, idx = ctx.saved_tensors
-        loss_cls, args, kind, nbytes = ctx.meta
-        grad_out = grad_out.to(torch.float32).contiguous()
+        loss_cls, args, kind, nbytes, per_image = ctx.meta
+        grad_out = grad_out.to(torch.float32).contiguous()   # also the stride-0 [B] of .sum() / .mean()
         with _on_device(sr.device):
             stream = _raw_stream(sr.device)
             d_sr = torch.empty_like(sr) if need_sr else None
             d_gt = torch.empty_like(gt) if need_gt else None
-            loss_cls._bwd(args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, _workspace(kind, sr.device, stream, nbytes),
-                          stream)
-        return d_sr, d_gt, None, None, None
+            bwd = loss_cls._bwd_none if per_image else loss_cls._bwd
+            bwd(args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, _workspace(kind, sr.device, stream, nbytes), stream)
+        return d_sr, d_gt, None, None, None, None
 
 
 class _PatchLoss(nn.Module):
     """What BestBuddyLoss, GramLoss and PatchwiseStructureTensorLoss share: the reference's constructor arguments
-    `alpha`, `beta`, `ksize`, `dist_norm`, `criterion` and the `pyramid` choice, the call through _PatchLossFn, and
-    ``last_indices``, the argmin indices ``[B,N]`` (int64) of the most recent call.  A subclass supplies the C ABI calls
-    (_args, _fwd, _bwd) and checks its patch geometry (_check_geometry)."""
+    `alpha`, `beta`, `ksize`, `dist_norm`, `criterion`, the `pyramid` and `reduction` choices, the call through
+    _PatchLossFn, and ``last_indices``, the argmin indices ``[B,N]`` (int64) of the most recent call.  A subclass supplies
+    the C ABI calls (_args, _fwd, _bwd; _MODE and _taps_of for the per-image entry points) and checks its patch geometry
+    (_check_geometry).
+
+    ``reduction='none'`` returns ``[B]``: entry b is the mean over image b's criterion terms, i.e. the reference module
+    applied to ``(x[b:b+1], gt[b:b+1])``; the search and ``last_indices`` are the same as with 'mean'."""
 
     _criterion_error = "%s criterion has not been implmented."   # the reference's message (loss.py:113, :178)
+    _MODE = 0   # `mode` of srst_patch_forward_per_image / srst_patch_backward_per_image
 
-    def __init__(self, alpha, beta, ksize, dist_norm, criterion, pyramid, pad=0, stride=3):
+    def __init__(self, alpha, beta, ksize, dist_norm, criterion, pyramid, pad=0, stride=3, reduction="mean"):
         super().__init__()
+        self.reduction = _check_reduction(reduction, type(self).__name__)
         self.alpha = alpha
         self.beta = beta
         self.ksize = ksize
@@ -458,9 +491,38 @@ class _PatchLoss(nn.Module):
 
     def forward(self, x, gt):
         _check_pair(x, gt, type(self).__name__)
-        loss, idx = _PatchLossFn.apply(x, gt, type(self), self._args(), self.pyramid)
+        if self.reduction == "none":
+            loss, idx = _PatchLossFn.apply(x, gt, type(self), self._args(), self.pyramid, True)
+        else:
+            loss, idx = _PatchLossFn.apply(x, gt, type(self), self._args(), self.pyramid)
         self.last_indices = idx
         return loss
+
+    def extra_repr(self) -> str:
+        return _reduction_repr(self.reduction)
+
+    @staticmethod
+    def _taps_of(args):
+        return _NO_TAPS
+
+    @classmethod
+    def _fwd_none(cls, args, sr, gt, gt2, gt4, idx, loss, ws, stream):
+        """reduction='none' forward of the default 3x3 / stride-3 patch grid: loss is [B]."""
+        alpha, beta, crit = args[:3]
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_patch_forward_per_image(cls._MODE, _ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W,
+                                                      *cls._taps_of(args)[:5], alpha, beta, crit, _ptr(idx), _ptr(loss),
+                                                      _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_patch_forward_per_image")
+
+    @classmethod
+    def _bwd_none(cls, args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, ws, stream):
+        """reduction='none' backward: grad_out is [B]; one call fills d_sr and d_gt, either of which may be None."""
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_patch_backward_per_image(cls._MODE, _ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx),
+                                                       _ptr(grad_out), B, H, W, *cls._taps_of(args)[:5], args[2], _ptr(d_sr),
+                                                       _ptr(d_gt), _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_patch_backward_per_image")
 
     @classmethod
     def _plan(cls, args, B, H, W):
@@ -485,11 +547,12 @@ class BestBuddyLoss(_PatchLoss):
     ``F.interpolate(mode='bicubic', align_corners=False)`` (equal to 2e-7; 0.03 ms instead of 0.43 ms at
     batch 64 x 192x192); "aten" calls the reference's own op.
     ``last_indices`` holds the argmin indices ``[B,N]`` (int64) of the most recent call.
+    ``reduction='none'`` returns the ``[B]`` per-image losses (every geometry).
     """
 
     def __init__(self, alpha: float = 1.0, beta: float = 1.0, ksize: int = 3, pad: int = 0, stride: int = 3,
-                 dist_norm: str = "l2", criterion: str = "l1", pyramid: str = "fused"):
-        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid, pad, stride)
+                 dist_norm: str = "l2", criterion: str = "l1", pyramid: str = "fused", reduction: str = "mean"):
+        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid, pad, stride, reduction)
         self.pad = pad
         self.stride = stride
 
@@ -551,15 +614,38 @@ class BestBuddyLoss(_PatchLoss):
         if d_gt is not None:
             _patch_backward_gt(0, sr, gt, gt2, gt4, idx, grad_out, _NO_TAPS, crit, d_gt, ws, stream)
 
+    @classmethod
+    def _fwd_none(cls, args, sr, gt, gt2, gt4, idx, loss, ws, stream):
+        alpha, beta, crit, geom = args
+        if geom is None:
+            return super()._fwd_none(args, sr, gt, gt2, gt4, idx, loss, ws, stream)
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_bbg_forward_per_image(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, *geom, alpha, beta,
+                                                    crit, _ptr(idx), _ptr(loss), _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_bbg_forward_per_image")
+
+    @classmethod
+    def _bwd_none(cls, args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, ws, stream):
+        crit, geom = args[2:]
+        if geom is None:
+            return super()._bwd_none(args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, ws, stream)
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_bbg_backward_per_image(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B,
+                                                     H, W, *geom, crit, _ptr(d_sr), _ptr(d_gt), _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_bbg_backward_per_image")
+
 
 class GramLoss(_PatchLoss):
     """Gram loss; same signature and semantics as reference loss.py:146-225: the best-buddy search
     and the final criterion run on the 3x3 Gram matrix of every 3x3x3 patch instead of its pixels.
-    Only ``ksize=3`` has kernels (the reference's default); ``dist_norm`` may be 'l2' or 'l1'."""
+    Only ``ksize=3`` has kernels (the reference's default); ``dist_norm`` may be 'l2' or 'l1'.
+    ``reduction='none'`` returns the ``[B]`` per-image losses."""
+
+    _MODE = 1
 
     def __init__(self, alpha: float = 1.0, beta: float = 1.0, ksize: int = 3, dist_norm: str = "l2",
-                 criterion: str = "l1", pyramid: str = "fused"):
-        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid)
+                 criterion: str = "l1", pyramid: str = "fused", reduction: str = "mean"):
+        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid, reduction=reduction)
 
     def _args(self):
         return float(self.alpha), float(self.beta), int(self._crit)
@@ -588,18 +674,24 @@ class PatchwiseStructureTensorLoss(_PatchLoss):
     """Patchwise structure-tensor loss; same signature and semantics as reference loss.py:292-375:
     the best-buddy search and the final criterion run on the det-normalised structure tensor of
     every 3x3 patch (seen as a 3x3 image, zero 'same' padding) instead of its pixels.
-    Only ``ksize=3`` has kernels (the reference's default); ``dist_norm`` may be 'l2' or 'l1'."""
+    Only ``ksize=3`` has kernels (the reference's default); ``dist_norm`` may be 'l2' or 'l1'.
+    ``reduction='none'`` returns the ``[B]`` per-image losses."""
 
     _criterion_error = "%s criterion has not been supported."   # loss.py:323
+    _MODE = 2
 
     def __init__(self, sigma: float = 0.5, rho: float = 2, alpha: float = 1.0, beta: float = 1.0, ksize: int = 3,
-                 dist_norm: str = "l2", criterion: str = "l1", pyramid: str = "fused"):
-        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid)
+                 dist_norm: str = "l2", criterion: str = "l1", pyramid: str = "fused", reduction: str = "mean"):
+        super().__init__(alpha, beta, ksize, dist_norm, criterion, pyramid, reduction=reduction)
         self.sigma = sigma
         self.rho = rho
 
     def _args(self):
         return float(self.alpha), float(self.beta), int(self._crit), _pst_taps(self.sigma, self.rho)
+
+    @staticmethod
+    def _taps_of(args):
+        return args[3]
 
     @staticmethod
     def _fwd(args, sr, gt, gt2, gt4, idx, loss, ws, stream):
