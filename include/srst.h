@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define SRST_VERSION 205 /* major*100 + minor: the major number changes whenever an argument list changes */
+#define SRST_VERSION 206 /* major*100 + minor: the major number changes whenever an argument list changes */
 
 #define SRST_E_INVALID (-1)     /* null pointer / non-positive size / bad enum */
 #define SRST_E_UNSUPPORTED (-2) /* filter radius or patch geometry not compiled in */
@@ -182,6 +182,28 @@ int srst_stpx_backward(const float* sr, const float* hr, const float* ixy, const
                        const float* g, const float* dg, int r_sigma,
                        const float* k, int r_rho,
                        float* d_sr, void* stream);
+
+/* Per-image reduction (reduction='none') of the fused criterion.  Same arguments, checks, return codes, workspace and
+ * saved buffers as srst_stpx_forward / srst_stpx_backward (generic radii: SRST_E_UNSUPPORTED), but
+ *   srst_stpx_forward_per_image:  loss2_out = device [2][B]: loss2_out[b] = mean of the ST distance over image b's
+ *                                 H*W pixels (as srst_st_forward_per_image), loss2_out[B + b] = mean((sr_b - hr_b)^2)
+ *                                 over its 3*H*W values
+ *   srst_stpx_backward_per_image: grad_st, grad_px = device [B] each (any values); d_sr of image b =
+ *                                 grad_st[b]/(H*W) * dST_b/dsr + grad_px[b] * 2 (sr_b - hr_b) / (3*H*W)
+ * The tile shapes are the ones the scalar entry points pick and each image's terms are reduced in double in a fixed
+ * order; d_sr of image b is bit-identical to srst_stpx_backward on that image alone with (grad_st[b], grad_px[b]). */
+int srst_stpx_forward_per_image(const float* sr, const float* hr, int B, int H, int W,
+                                const float* g, const float* dg, int r_sigma,
+                                const float* k, int r_rho,
+                                int normalize, float eps,
+                                float* loss2_out, float* ds_sr, float* ixy_sr,
+                                void* workspace, size_t workspace_bytes, void* stream);
+int srst_stpx_backward_per_image(const float* sr, const float* hr, const float* ixy, const float* ds,
+                                 const float* grad_st, const float* grad_px,
+                                 int B, int H, int W,
+                                 const float* g, const float* dg, int r_sigma,
+                                 const float* k, int r_rho,
+                                 float* d_sr, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Best-Buddy loss.   Replaces

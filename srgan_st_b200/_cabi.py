@@ -53,6 +53,11 @@ SIGNATURES = {
                                          ctypes.c_int, ctypes.c_float, vp, vp, vp, vp, ctypes.c_size_t, vp]),
     "srst_stpx_backward": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                           c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int, vp, vp]),
+    "srst_stpx_forward_per_image": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                   c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                                   ctypes.c_int, ctypes.c_float, vp, vp, vp, vp, ctypes.c_size_t, vp]),
+    "srst_stpx_backward_per_image": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                    c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int, vp, vp]),
     "srst_bb_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int] * 3),
     "srst_bb_forward": (ctypes.c_int, [vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                        ctypes.c_float, ctypes.c_float, ctypes.c_int, vp, vp,

@@ -397,7 +397,8 @@ struct StCall {
   const float *sr = nullptr, *hr = nullptr, *ixy = nullptr, *ds = nullptr, *grad_out = nullptr;
   float *ds_sr = nullptr, *ds_hr = nullptr, *ixy_sr = nullptr, *ixy_hr = nullptr, *loss_out = nullptr, *d_img = nullptr;
   int px = 0;                                            // forward: also reduce the fused Pixel (MSE) term into loss_out[1]
-  int per_image = 0;                                     // reduction='none': loss_out / grad_out are [B] (no Pixel term)
+  int per_image = 0;                                     // reduction='none': loss_out / grad_out / grad_px are [B], and
+                                                         // the MSE terms go to loss_out[B .. 2B)
   const float *px_img = nullptr, *px_other = nullptr, *grad_px = nullptr;  // backward: image pair + upstream gradient of the MSE term
   int B = 0, H = 0, W = 0, normalize = 1, vec4 = 0;
   float eps = 0.f;
@@ -406,6 +407,20 @@ struct StCall {
   int rs = 0, rk = 0;
   void* stream = nullptr;
 };
+
+// one tile shape with the batch or the per-image reduction (c.per_image); PX: the fused Pixel term
+template <class C, bool PX, int RG, int RK>
+static int tiled_fwd(StFwdParams<RG, RK>& P, const StCall& c) {
+  return c.per_image ? launch_st_forward<C, PX, true>(P, c.stream) : launch_st_forward<C, PX>(P, c.stream);
+}
+template <class C, bool PX>
+static int march_fwd(const StFwdParams<C::RG, C::RK>& P, const StCall& c) {
+  return c.per_image ? launch_st_march<C, PX, true>(P, c.stream) : launch_st_march<C, PX>(P, c.stream);
+}
+template <class C, bool PX, int RG, int RK>
+static int tiled_bwd(StBwdParams<RG, RK>& P, const StCall& c) {
+  return c.per_image ? launch_st_backward<C, PX, true>(P, c.stream) : launch_st_backward<C, PX>(P, c.stream);
+}
 
 template <int RG, int RK>
 static int st_forward_rr(const StCall& c) {
@@ -424,35 +439,24 @@ static int st_forward_rr(const StCall& c) {
     const int mcfg = pick_march_cfg(c.W);
     if (mcfg >= 0) {
       int e;
-      if (c.per_image)
-        e = mcfg == kFwdMarch96 ? launch_st_march<March96, false, true>(P, c.stream)
-                                : launch_st_march<March112, false, true>(P, c.stream);
-      else if (mcfg == kFwdMarch96) e = c.px ? launch_st_march<March96, true>(P, c.stream) : launch_st_march<March96>(P, c.stream);
-      else e = c.px ? launch_st_march<March112, true>(P, c.stream) : launch_st_march<March112>(P, c.stream);
+      if (mcfg == kFwdMarch96) e = c.px ? march_fwd<March96, true>(P, c) : march_fwd<March96, false>(P, c);
+      else e = c.px ? march_fwd<March112, true>(P, c) : march_fwd<March112, false>(P, c);
       if (e != kMarchUnusable) return e;
     }
     int cfg = pick_fwd_cfg(c.B, c.H, c.W);
     if (cfg >= kFwdMarch96) cfg = (c.W <= 96) ? 1 : 0;  // a marching shape was forced but TMA cannot fetch these tensors
-    if (c.per_image) {
-      switch (cfg) {
-        case 1: return launch_st_forward<Fwd1, false, true>(P, c.stream);
-        case 2: return launch_st_forward<Fwd2, false, true>(P, c.stream);
-        default: return launch_st_forward<Fwd0, false, true>(P, c.stream);
-      }
-    }
     if (c.px) {  // the fused Pixel term is compiled into the two default tile shapes only
-      if (cfg != 0 && c.W <= 96) return launch_st_forward<Fwd1, true>(P, c.stream);
-      return launch_st_forward<Fwd0, true>(P, c.stream);
+      if (cfg != 0 && c.W <= 96) return tiled_fwd<Fwd1, true>(P, c);
+      return tiled_fwd<Fwd0, true>(P, c);
     }
     switch (cfg) {
-      case 1: return launch_st_forward<Fwd1>(P, c.stream);
-      case 2: return launch_st_forward<Fwd2>(P, c.stream);
-      default: return launch_st_forward<Fwd0>(P, c.stream);
+      case 1: return tiled_fwd<Fwd1, false>(P, c);
+      case 2: return tiled_fwd<Fwd2, false>(P, c);
+      default: return tiled_fwd<Fwd0, false>(P, c);
     }
   } else {
     using G = StFwdCfg<32, 64, 16, 4, RG, RK, (RK <= 8 ? 2 : 1), 0>;
-    if (c.per_image) return launch_st_forward<G, false, true>(P, c.stream);
-    return c.px ? launch_st_forward<G, true>(P, c.stream) : launch_st_forward<G>(P, c.stream);
+    return c.px ? tiled_fwd<G, true>(P, c) : tiled_fwd<G, false>(P, c);
   }
 }
 
@@ -468,16 +472,14 @@ static int st_backward_rr(const StCall& c) {
   P.taps = cached_taps<RG, RK>(c.g, c.dg, c.rs, c.k, c.rk);
   if constexpr (RG == 2 && RK == 8) {
     if (c.px_other) {  // the fused Pixel term is compiled into the two default tile shapes
-      if (c.W <= 96) return launch_st_backward<Bwd1, true>(P, c.stream);
-      return launch_st_backward<Bwd0, true>(P, c.stream);
+      if (c.W <= 96) return tiled_bwd<Bwd1, true>(P, c);
+      return tiled_bwd<Bwd0, true>(P, c);
     }
-    if (pick_bwd_cfg(c.B, c.H, c.W) == 1)
-      return c.per_image ? launch_st_backward<Bwd1, false, true>(P, c.stream) : launch_st_backward<Bwd1>(P, c.stream);
-    return c.per_image ? launch_st_backward<Bwd0, false, true>(P, c.stream) : launch_st_backward<Bwd0>(P, c.stream);
+    if (pick_bwd_cfg(c.B, c.H, c.W) == 1) return tiled_bwd<Bwd1, false>(P, c);
+    return tiled_bwd<Bwd0, false>(P, c);
   } else {
     using G = StBwdCfg<24, 64, (24 + 2 * RG) / 2, 256, RG, RK, (RK <= 8 ? 2 : 1), 4>;
-    if (c.per_image) return launch_st_backward<G, false, true>(P, c.stream);
-    return c.px_other ? launch_st_backward<G, true>(P, c.stream) : launch_st_backward<G>(P, c.stream);
+    return c.px_other ? tiled_bwd<G, true>(P, c) : tiled_bwd<G, false>(P, c);
   }
 }
 
@@ -657,9 +659,13 @@ int srst_st_backward(const float* ixy, const float* ds, const float* grad_out, i
   return srst_st_backward_ws(ixy, ds, grad_out, B, H, W, g, dg, r_sigma, k, r_rho, d_img, nullptr, 0, stream);
 }
 
-int srst_stpx_forward(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
-                      int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss2_out, float* ds_sr,
-                      float* ixy_sr, void* workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// srst_stpx_forward and srst_stpx_forward_per_image: the same checks and dispatch; per_image selects the [2][B] output
+static int stpx_forward_entry(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
+                              int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss2_out,
+                              float* ds_sr, float* ixy_sr, void* workspace, size_t workspace_bytes, void* stream,
+                              int per_image) {
   if (!sr || !hr || !g || !dg || !k || !loss2_out || B <= 0 || H <= 0 || W <= 0) return SRST_E_INVALID;
   if (!st_compiled(r_sigma, r_rho)) return SRST_E_UNSUPPORTED;  // the generic-radius path has no fused / feature variant
   if (!workspace || !aligned16(workspace) || workspace_bytes < srst_st_workspace_bytes(B, H, W))
@@ -670,12 +676,13 @@ int srst_stpx_forward(const float* sr, const float* hr, int B, int H, int W, con
   c.vec4 = (W % 4 == 0 && aligned16(sr) && aligned16(hr) && (!ds_sr || aligned16(ds_sr)) &&
             (!ixy_sr || aligned16(ixy_sr))) ? 1 : 0;
   c.workspace = workspace; c.g = g; c.dg = dg; c.k = k; c.rs = r_sigma; c.rk = r_rho; c.stream = stream;
+  c.per_image = per_image;
   return st_dispatch(c, true);
 }
 
-int srst_stpx_backward(const float* sr, const float* hr, const float* ixy, const float* ds, const float* grad_st,
-                       const float* grad_px, int B, int H, int W, const float* g, const float* dg, int r_sigma,
-                       const float* k, int r_rho, float* d_sr, void* stream) {
+static int stpx_backward_entry(const float* sr, const float* hr, const float* ixy, const float* ds, const float* grad_st,
+                               const float* grad_px, int B, int H, int W, const float* g, const float* dg, int r_sigma,
+                               const float* k, int r_rho, float* d_sr, void* stream, int per_image) {
   if (!sr || !hr || !ixy || !ds || !grad_st || !grad_px || !g || !dg || !k || !d_sr || B <= 0 || H <= 0 || W <= 0)
     return SRST_E_INVALID;
   if (!st_compiled(r_sigma, r_rho)) return SRST_E_UNSUPPORTED;  // the generic-radius path has no fused / feature variant
@@ -684,7 +691,36 @@ int srst_stpx_backward(const float* sr, const float* hr, const float* ixy, const
   c.B = B; c.H = H; c.W = W;
   c.vec4 = (W % 4 == 0 && aligned16(sr) && aligned16(hr) && aligned16(d_sr) && aligned16(ds)) ? 1 : 0;
   c.g = g; c.dg = dg; c.k = k; c.rs = r_sigma; c.rk = r_rho; c.stream = stream;
+  c.per_image = per_image;
   return st_dispatch(c, false);
+}
+
+extern "C" {
+
+int srst_stpx_forward(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
+                      int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss2_out, float* ds_sr,
+                      float* ixy_sr, void* workspace, size_t workspace_bytes, void* stream) {
+  return stpx_forward_entry(sr, hr, B, H, W, g, dg, r_sigma, k, r_rho, normalize, eps, loss2_out, ds_sr, ixy_sr,
+                            workspace, workspace_bytes, stream, 0);
+}
+
+int srst_stpx_forward_per_image(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
+                                int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss2_out,
+                                float* ds_sr, float* ixy_sr, void* workspace, size_t workspace_bytes, void* stream) {
+  return stpx_forward_entry(sr, hr, B, H, W, g, dg, r_sigma, k, r_rho, normalize, eps, loss2_out, ds_sr, ixy_sr,
+                            workspace, workspace_bytes, stream, 1);
+}
+
+int srst_stpx_backward(const float* sr, const float* hr, const float* ixy, const float* ds, const float* grad_st,
+                       const float* grad_px, int B, int H, int W, const float* g, const float* dg, int r_sigma,
+                       const float* k, int r_rho, float* d_sr, void* stream) {
+  return stpx_backward_entry(sr, hr, ixy, ds, grad_st, grad_px, B, H, W, g, dg, r_sigma, k, r_rho, d_sr, stream, 0);
+}
+
+int srst_stpx_backward_per_image(const float* sr, const float* hr, const float* ixy, const float* ds,
+                                 const float* grad_st, const float* grad_px, int B, int H, int W, const float* g,
+                                 const float* dg, int r_sigma, const float* k, int r_rho, float* d_sr, void* stream) {
+  return stpx_backward_entry(sr, hr, ixy, ds, grad_st, grad_px, B, H, W, g, dg, r_sigma, k, r_rho, d_sr, stream, 1);
 }
 
 }  // extern "C"

@@ -689,11 +689,10 @@ SRST_DEV void st_unit_tensor(float* smem, const float* __restrict__ base, float*
 }
 
 // PER_IMG: reduction='none' -- loss_out[b] is the mean over image b's pixels (P.inv_count = 1 / (H W)) instead of
-// loss_out[0] over the batch; no fused Pixel term
+// loss_out[0] over the batch; with PX, loss_out[B + b] is image b's mean squared difference over its 3 H W values
 template <class C, bool PX = false, bool WANT_HR = false, bool PER_IMG = false>
 __global__ void __launch_bounds__(C::NT, C::MINB)
 st_forward_kernel(const __grid_constant__ StFwdParams<C::RG, C::RK> P) {
-  static_assert(!(PX && PER_IMG), "the fused Pixel term has no per-image reduction");
   SRST_DYN_SMEM(float, smem);
   __shared__ float s_red[32];
   __shared__ unsigned int s_last;
@@ -832,6 +831,8 @@ st_forward_kernel(const __grid_constant__ StFwdParams<C::RG, C::RK> P) {
     if (s_last) {  // image-major grid: image b owns tiles_y * tiles_x consecutive CTAs
       __threadfence();
       reduce_partials_per_image(P.partials, P.B, gridDim.x / P.B, (double)P.inv_count, P.loss_out);
+      if constexpr (PX)
+        reduce_partials_per_image(P.px_partials, P.B, gridDim.x / P.B, (double)P.inv_count / 3.0, P.loss_out + P.B);
       if (tid == 0) *P.ticket = 0u;
     }
   } else if (s_last) {
@@ -974,7 +975,7 @@ struct StBwdCfg {
   static_assert((CSD == 4 || CSD == 8) && EW % CSD == 0, "bad phase-D' item width");
 };
 
-// PER_IMG: reduction='none' -- grad_out is [B] and the tile of image b scales by grad_out[b] / (H W)
+// PER_IMG: reduction='none' -- grad_out (and with PX grad_px) is [B] and the tile of image b scales by grad_out[b] / (H W)
 // (P.inv_count = 1 / (H W)) instead of grad_out[0] / (B H W)
 template <class C, bool PX = false, bool PER_IMG = false>
 __global__ void __launch_bounds__(C::NT, C::MINB)
@@ -1134,7 +1135,7 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
   //   dgray = -[ (dIx * dg|) * g-  +  (dIy * g|) * dg- ]
   // i.e. the forward gradient operators applied to dIx and dIy, negated.
   const float scale = -__ldg(P.grad_out + (PER_IMG ? b : 0)) * P.inv_count;
-  [[maybe_unused]] const float px_scale = PX ? __ldg(P.grad_px) * P.inv_count * (2.0f / 3.0f) : 0.f;
+  [[maybe_unused]] const float px_scale = PX ? __ldg(P.grad_px + (PER_IMG ? b : 0)) * P.inv_count * (2.0f / 3.0f) : 0.f;
   for (int it = tid; it < C::MapE::SLOTS; it += C::NT) {
     int q, seg;
     if (!C::MapE::decode(it, q, seg)) continue;

@@ -178,11 +178,10 @@ SRST_DEV float2 st_pixel2_raw(float2 a, float2 b, float2 c, float2 e, float2 f, 
 }
 
 // PER_IMG: reduction='none' -- loss_out[b] is the mean over image b's pixels (P.inv_count = 1 / (H W)) instead of
-// loss_out[0] over the batch; no fused Pixel term
+// loss_out[0] over the batch; with PX, loss_out[B + b] is image b's mean squared difference over its 3 H W values
 template <class C, bool PX = false, bool WANT_HR = false, bool PER_IMG = false>
 __global__ void __launch_bounds__(C::NT, C::MINB)
 st_forward_march_kernel(const __grid_constant__ StMarchParams<C::RG, C::RK> MP) {
-  static_assert(!(PX && PER_IMG), "the fused Pixel term has no per-image reduction");
   SRST_DYN_SMEM(float, smem);
   __shared__ float s_red[32];
   __shared__ unsigned int s_last;
@@ -619,6 +618,8 @@ st_forward_march_kernel(const __grid_constant__ StMarchParams<C::RG, C::RK> MP) 
     if (s_last) {  // image-major grid: image b owns nchunks * nstrips consecutive CTAs
       __threadfence();
       reduce_partials_per_image(P.partials, P.B, gridDim.x / P.B, (double)P.inv_count, P.loss_out);
+      if constexpr (PX)
+        reduce_partials_per_image(P.px_partials, P.B, gridDim.x / P.B, (double)P.inv_count / 3.0, P.loss_out + P.B);
       if (tid == 0) *P.ticket = 0u;
     }
   } else if (s_last) {

@@ -271,10 +271,12 @@ def structure_tensor_features(img: torch.Tensor, sigma: float = 0.5, rho: float 
 
 class _StructureTensorPixelLossFn(torch.autograd.Function):
     """ST loss and the "Pixel" MSE criterion from ONE pass over (sr, gt) per direction (SURVEY 8f rank 4).
-    Returns the two unweighted terms as one 2-vector [st, mse]; gt carries no gradient."""
+    Returns the two unweighted terms as one 2-vector [st, mse]; gt carries no gradient.
+    `per_image`: reduction='none' -- the terms are [2, B] (row 0 ST, row 1 MSE) and so is the upstream gradient
+    (the *_per_image entry points)."""
 
     @staticmethod
-    def forward(ctx, sr, hr, sigma, rho, normalize):
+    def forward(ctx, sr, hr, sigma, rho, normalize, per_image=False):
         lib = _cabi.lib()
         sr = sr.contiguous()
         hr = hr.contiguous()
@@ -284,17 +286,18 @@ class _StructureTensorPixelLossFn(torch.autograd.Function):
         n_ds, n_ixy, ws_bytes, _ = _st_sizes(B, H, W)
         with _on_device(sr.device):
             stream = _raw_stream(sr.device)
-            both = torch.empty(2, dtype=torch.float32, device=sr.device)
+            both = torch.empty((2, B) if per_image else 2, dtype=torch.float32, device=sr.device)
             saved = torch.empty(n_ds + n_ixy, dtype=torch.float32, device=sr.device) if need_sr else None
             p = saved.data_ptr() if need_sr else None
             ws = _workspace("st", sr.device, stream, ws_bytes)
-            rc = lib.srst_stpx_forward(sr.data_ptr(), hr.data_ptr(), B, H, W, tp[0], tp[1], tp[2], tp[3], tp[4],
-                                       int(bool(normalize)), 1e-12, both.data_ptr(), p,
-                                       p + 4 * n_ds if need_sr else None, ws.data_ptr(), ws.numel(), stream)
+            fwd = lib.srst_stpx_forward_per_image if per_image else lib.srst_stpx_forward
+            rc = fwd(sr.data_ptr(), hr.data_ptr(), B, H, W, tp[0], tp[1], tp[2], tp[3], tp[4],
+                     int(bool(normalize)), 1e-12, both.data_ptr(), p,
+                     p + 4 * n_ds if need_sr else None, ws.data_ptr(), ws.numel(), stream)
         if rc:
-            _cabi.check(rc, "srst_stpx_forward")
+            _cabi.check(rc, "srst_stpx_forward_per_image" if per_image else "srst_stpx_forward")
         ctx.save_for_backward(sr, hr, saved)
-        ctx.meta = (tp, n_ds)
+        ctx.meta = (tp, n_ds, per_image)
         return both
 
     @staticmethod
@@ -302,21 +305,23 @@ class _StructureTensorPixelLossFn(torch.autograd.Function):
     def backward(ctx, grad_both):
         lib = _cabi.lib()
         sr, hr, saved = ctx.saved_tensors
-        tp, n_ds = ctx.meta
+        tp, n_ds, per_image = ctx.meta
         if saved is None or not ctx.needs_input_grad[0]:
-            return None, None, None, None, None
+            return None, None, None, None, None, None
         B, _, H, W = sr.shape
         with _on_device(sr.device):
             stream = _raw_stream(sr.device)
-            if grad_both.dtype != torch.float32 or not grad_both.is_contiguous():
+            if grad_both.dtype != torch.float32 or not grad_both.is_contiguous():   # also the stride-0 one of .sum()
                 grad_both = grad_both.to(torch.float32).contiguous()
             d_sr = torch.empty_like(sr)
-            g = grad_both.data_ptr()                       # [d/d st, d/d mse]: two adjacent device scalars
-            rc = lib.srst_stpx_backward(sr.data_ptr(), hr.data_ptr(), saved.data_ptr() + 4 * n_ds, saved.data_ptr(),
-                                        g, g + 4, B, H, W, tp[0], tp[1], tp[2], tp[3], tp[4], d_sr.data_ptr(), stream)
+            g = grad_both.data_ptr()   # [d/d st, d/d mse]: two adjacent device scalars, or two adjacent [B] rows
+            bwd = lib.srst_stpx_backward_per_image if per_image else lib.srst_stpx_backward
+            rc = bwd(sr.data_ptr(), hr.data_ptr(), saved.data_ptr() + 4 * n_ds, saved.data_ptr(),
+                     g, g + 4 * (B if per_image else 1), B, H, W, tp[0], tp[1], tp[2], tp[3], tp[4], d_sr.data_ptr(),
+                     stream)
         if rc:
-            _cabi.check(rc, "srst_stpx_backward")
-        return d_sr, None, None, None, None
+            _cabi.check(rc, "srst_stpx_backward_per_image" if per_image else "srst_stpx_backward")
+        return d_sr, None, None, None, None, None
 
 
 class StructureTensorPixelLoss(nn.Module):
@@ -327,40 +332,51 @@ class StructureTensorPixelLoss(nn.Module):
     and evaluate them one after the other on the same two tensors (config.py:71-93, warmup.py:88-96,
     train.py:131-144).  Registering this module once, with weight 1.0, gives the same generator loss
     and gradient; the two unweighted terms of the last call stay on the device in ``last_terms`` for
-    logging without a synchronisation."""
+    logging without a synchronisation.
+
+    ``reduction='none'`` returns the ``[B]`` per-image losses ``st_weight * st[b] + pixel_weight * mse[b]`` instead:
+    ``st[b]`` is ``StructureTensorLoss(reduction='none')`` of image b, ``mse[b]`` the mean of ``(x[b] - gt[b])**2``.
+    It is differentiable w.r.t. x, still from one fused pass per direction."""
 
     def __init__(self, sigma: float = 0.5, rho: float = 2.0, normalize: bool = True, st_weight: float = 1.0,
-                 pixel_weight: float = 1.0):
+                 pixel_weight: float = 1.0, reduction: str = "mean"):
         super().__init__()
         self.sigma = sigma
         self.rho = rho
         self.normalize = normalize
         self.st_weight = st_weight
         self.pixel_weight = pixel_weight
+        self.reduction = _check_reduction(reduction, "StructureTensorPixelLoss")
         self._last = None
         self._w = None   # (device, st_weight, pixel_weight, tensor): the weights as a device 2-vector
         _cabi.lib()
 
     @property
     def last_terms(self):
-        """(st, mse) of the most recent call as two 0-dim device tensors (detached), or None."""
+        """(st, mse) of the most recent call as two device tensors (detached), or None: 0-dim, or [B] each with
+        reduction='none'."""
         return None if self._last is None else (self._last[0], self._last[1])
 
     def forward(self, x, gt):
         _check_pair(x, gt, "StructureTensorPixelLoss")
         _no_gt_grad(gt, "StructureTensorPixelLoss")
-        both = _StructureTensorPixelLossFn.apply(x, gt, self.sigma, self.rho, self.normalize)
+        per_image = self.reduction == "none"
+        if per_image:
+            both = _StructureTensorPixelLossFn.apply(x, gt, self.sigma, self.rho, self.normalize, True)
+        else:
+            both = _StructureTensorPixelLossFn.apply(x, gt, self.sigma, self.rho, self.normalize)
         self._last = both.detach()
         w = self._w
         if w is None or w[0] != x.device or w[1] != self.st_weight or w[2] != self.pixel_weight:
             w = (x.device, self.st_weight, self.pixel_weight,
                  torch.tensor([self.st_weight, self.pixel_weight], dtype=torch.float32, device=x.device))
             self._w = w
-        return torch.dot(both, w[3])
+        return w[3] @ both if per_image else torch.dot(both, w[3])
 
     def extra_repr(self) -> str:
-        return (f"sigma={self.sigma}, rho={self.rho}, normalize={self.normalize}, st_weight={self.st_weight}, "
-                f"pixel_weight={self.pixel_weight}")
+        r = (f"sigma={self.sigma}, rho={self.rho}, normalize={self.normalize}, st_weight={self.st_weight}, "
+             f"pixel_weight={self.pixel_weight}")
+        return r if self.reduction == "mean" else f"{r}, {_reduction_repr(self.reduction)}"
 
 
 def _hr_pyramid(gt, pyramid: str):

@@ -6,6 +6,9 @@ Every case is a forward + backward step.  The 'none' step backpropagates loss.me
 step), so the two differ only by the per-image kernels and the tiny reduction torch adds.  Variants of one case are
 timed alternately, R rounds of K steps each, with CUDA events; the median of the rounds is printed, with the spread.
 The card's name and power limit are printed first: the numbers belong to them.
+
+The fused ST + Pixel cases also time 'split': the per-image losses without the fused module,
+st_weight * StructureTensorLoss(reduction='none') + pixel_weight * ((x - gt)**2).mean((1, 2, 3)), same backward.
 """
 import argparse
 import os
@@ -16,7 +19,7 @@ import sys
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from srgan_st_b200 import BestBuddyLoss, StructureTensorLoss  # noqa: E402
+from srgan_st_b200 import BestBuddyLoss, StructureTensorLoss, StructureTensorPixelLoss  # noqa: E402
 
 
 def card():
@@ -38,7 +41,7 @@ def pair(B, H, W, seed=0):
 def step_fn(module, sr, gt, how):
     if how == "mean":
         return lambda: module(sr, gt).backward()
-    if how == "none":
+    if how in ("none", "split"):
         return lambda: module(sr, gt).mean().backward()
     B = sr.shape[0]   # "calls": B separate one-image calls, the workaround without reduction='none'
 
@@ -89,6 +92,18 @@ def main():
         iters = a.iters if B * H * W < 50_000_000 else max(a.iters // 4, 3)
         report(name, time_alternating({"mean": step_fn(st_mean, sr, gt, "mean"),
                                        "none": step_fn(st_none, sr, gt, "none")}, a.rounds, iters))
+        del sr, gt
+    w_st, w_px = 0.5, 2.0
+    px_mean = StructureTensorPixelLoss(st_weight=w_st, pixel_weight=w_px)
+    px_none = StructureTensorPixelLoss(st_weight=w_st, pixel_weight=w_px, reduction="none")
+
+    def split(x, y):
+        return w_st * st_none(x, y) + w_px * ((x - y) ** 2).mean((1, 2, 3))
+
+    for B, H, W, name in ((64, 96, 96, "ST+Pixel configs[1] 64x96x96"), (1, 1356, 2040, "ST+Pixel 1x1356x2040")):
+        sr, gt = pair(B, H, W)
+        report(name, time_alternating({"mean": step_fn(px_mean, sr, gt, "mean"), "none": step_fn(px_none, sr, gt, "none"),
+                                       "split": step_fn(split, sr, gt, "split")}, a.rounds, a.iters))
         del sr, gt
     sr, gt = pair(64, 192, 192)
     report("BestBuddy configs[3] 64x192x192", time_alternating(
