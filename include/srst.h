@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define SRST_VERSION 206 /* major*100 + minor: the major number changes whenever an argument list changes */
+#define SRST_VERSION 207 /* major*100 + minor: the major number changes whenever an argument list changes */
 
 #define SRST_E_INVALID (-1)     /* null pointer / non-positive size / bad enum */
 #define SRST_E_UNSUPPORTED (-2) /* filter radius or patch geometry not compiled in */
@@ -143,6 +143,34 @@ int srst_st_backward_per_image(const float* ixy, const float* ds, const float* g
                                const float* g, const float* dg, int r_sigma,
                                const float* k, int r_rho,
                                float* d_img, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Per-pixel distance map (the element-wise form of the loss: the map d = utils.compute_distance(L) that st_loss builds
+ * before its .mean(), loss.py:408-409, utils.py:269-279), e.g. for spatial weighting or masking of the loss and for
+ * loss heat maps.
+ *   srst_st_forward_map: the arguments of srst_st_forward with map_out (device [B,H,W] fp32, required) after loss_out.
+ *     Same checks, return codes and workspace (srst_st_workspace_bytes_r); compiled radius classes and the generic-radius
+ *     path.  map_out[b,y,x] = the distance of pixel (y, x) of image b.  loss_out[0], ds_* and ixy_* are bit-identical to
+ *     srst_st_forward on the same inputs (the same tile shapes are picked), so loss_out[0] = mean(map_out) up to the
+ *     order of the summation.
+ *   srst_st_backward_map: d_img = sum over pixels p of grad_map[p] * d(map_out[p])/d(img), for one image tensor.
+ *     ixy, ds as for srst_st_backward (the unscaled buffers the forward wrote; they are only read, so the call can be
+ *     repeated); grad_map: device [B,H,W], any values.  A prepass writes grad_map * ds into the workspace, then the
+ *     srst_st_backward kernels run on it with a unit upstream gradient.  The workspace is always required
+ *     (srst_st_backward_map_workspace_bytes; no zero-initialisation needed).  Ordering as for srst_st_backward.
+ *   srst_st_backward_map_workspace_bytes: the weighted ds planes (12 B/px) plus a 256-byte slot, plus
+ *     srst_st_backward_workspace_bytes on the generic-radius path; 0 for unsupported radii or non-positive sizes. */
+int srst_st_forward_map(const float* sr, const float* hr, int B, int H, int W,
+                        const float* g, const float* dg, int r_sigma,
+                        const float* k, int r_rho,
+                        int normalize, float eps,
+                        float* loss_out, float* map_out, float* ds_sr, float* ds_hr, float* ixy_sr, float* ixy_hr,
+                        void* workspace, size_t workspace_bytes, void* stream);
+size_t srst_st_backward_map_workspace_bytes(int B, int H, int W, int r_sigma, int r_rho);
+int srst_st_backward_map(const float* ixy, const float* ds, const float* grad_map,
+                         int B, int H, int W,
+                         const float* g, const float* dg, int r_sigma,
+                         const float* k, int r_rho,
+                         float* d_img, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Structure-tensor FEATURES of one image tensor (diagnostic output; BASELINE.json north_star: "closed-form 2x2
  * eigendecomposition giving orientation, coherence and eigenvalues").  The reference computes these only in an

@@ -46,6 +46,14 @@ SIGNATURES = {
     "srst_st_backward_per_image": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                   c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
                                                   vp, vp, ctypes.c_size_t, vp]),
+    "srst_st_forward_map": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                           c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                           ctypes.c_int, ctypes.c_float, vp, vp, vp, vp, vp, vp,
+                                           vp, ctypes.c_size_t, vp]),
+    "srst_st_backward_map_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int] * 5),
+    "srst_st_backward_map": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                            c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                            vp, vp, ctypes.c_size_t, vp]),
     "srst_st_features": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                         c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int, vp, vp, vp, vp, vp]),
     "srst_stpx_forward": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,

@@ -194,23 +194,24 @@ static bool make_plane_map(SrstTmap* map, const float* base, long long planes, i
 #endif
 }
 
-// once-flag tag per forward / backward instantiation (PI: the per-image reduction, reduction='none')
-template <class C, bool PX, bool HR, bool PI = false> struct FwdTag {};
+// once-flag tag per forward / backward instantiation (PI: the per-image reduction, reduction='none'; MAP: the
+// distance map)
+template <class C, bool PX, bool HR, bool PI = false, bool MAP = false> struct FwdTag {};
 template <class C, bool PX, bool PI = false> struct BwdTag {};
 
-template <class C, bool PX = false, bool PI = false>
-static int launch_st_forward(StFwdParams<C::RG, C::RK>& P, void* stream) {
+template <class C, bool PX = false, bool PI = false, bool MAP = false>
+static int launch_st_forward(StFwdParamsT<C::RG, C::RK, MAP>& P, void* stream) {
   P.tiles_x = (P.W + C::TW - 1) / C::TW;
   P.tiles_y = (P.H + C::TH - 1) / C::TH;
   const long long ntiles = (long long)P.B * P.tiles_x * P.tiles_y;
   if (ntiles <= 0 || ntiles > 0x7fffffffLL) return SRST_E_SHAPE;
   int e;
   if (P.ds_hr) {
-    if ((e = ensure_smem<FwdTag<C, PX, true, PI>>(st_forward_kernel<C, PX, true, PI>, C::SMEM_BYTES)) != 0) return e;
-    SRST_LAUNCH_PDL((st_forward_kernel<C, PX, true, PI>), dim3((unsigned)ntiles), dim3(C::NT), C::SMEM_BYTES, stream, P);
+    if ((e = ensure_smem<FwdTag<C, PX, true, PI, MAP>>(st_forward_kernel<C, PX, true, PI, MAP>, C::SMEM_BYTES)) != 0) return e;
+    SRST_LAUNCH_PDL((st_forward_kernel<C, PX, true, PI, MAP>), dim3((unsigned)ntiles), dim3(C::NT), C::SMEM_BYTES, stream, P);
   } else {
-    if ((e = ensure_smem<FwdTag<C, PX, false, PI>>(st_forward_kernel<C, PX, false, PI>, C::SMEM_BYTES)) != 0) return e;
-    SRST_LAUNCH_PDL((st_forward_kernel<C, PX, false, PI>), dim3((unsigned)ntiles), dim3(C::NT), C::SMEM_BYTES, stream, P);
+    if ((e = ensure_smem<FwdTag<C, PX, false, PI, MAP>>(st_forward_kernel<C, PX, false, PI, MAP>, C::SMEM_BYTES)) != 0) return e;
+    SRST_LAUNCH_PDL((st_forward_kernel<C, PX, false, PI, MAP>), dim3((unsigned)ntiles), dim3(C::NT), C::SMEM_BYTES, stream, P);
   }
   return (int)cudaGetLastError();
 }
@@ -219,16 +220,17 @@ static int launch_st_forward(StFwdParams<C::RG, C::RK>& P, void* stream) {
 // tiled shape).  Chunking: whole strips when B * strips already fills the machine, otherwise each strip is cut
 // into as many row chunks as there are idle SMs (a chunk costs one extra 16-row block of gradient + horizontal work).
 constexpr int kMarchUnusable = -1000;
-template <class C, bool PX, bool HR, bool PI = false> struct MarchTag {};
-template <class C, bool PX = false, bool PI = false>
-static int launch_st_march(const StFwdParams<C::RG, C::RK>& F, void* stream) {
-  static thread_local StMarchParams<C::RG, C::RK> MP_tls;
+template <class C, bool PX, bool HR, bool PI = false, bool MAP = false> struct MarchTag {};
+template <class C, bool PX = false, bool PI = false, bool MAP = false>
+static int launch_st_march(const StFwdParamsT<C::RG, C::RK, MAP>& F, void* stream) {
+  static thread_local StMarchParamsT<C::RG, C::RK, MAP> MP_tls;
   auto& MP = MP_tls;  // a plain reference: the emulation's kernel threads must see THIS thread's instance
   if (!F.vec4) return kMarchUnusable;
   if (!make_plane_map(&MP.sr_map, F.sr, (long long)F.B * 3, F.H, F.W, C::GW, C::RS, 3) ||
       !make_plane_map(&MP.hr_map, F.hr, (long long)F.B * 3, F.H, F.W, C::GW, C::RS, 3))
     return kMarchUnusable;
   MP.F = F;
+  if constexpr (MAP) MP.map_out = F.map_out;
   const int nblk = (F.H + C::RS - 1) / C::RS;
   MP.nstrips = (F.W + C::TW - 1) / C::TW;
   const long long base = (long long)F.B * MP.nstrips;
@@ -244,11 +246,13 @@ static int launch_st_march(const StFwdParams<C::RG, C::RK>& F, void* stream) {
   if (grid <= 0 || grid > 0x7fffffffLL) return SRST_E_SHAPE;
   int e;
   if (F.ds_hr) {
-    if ((e = ensure_smem<MarchTag<C, PX, true, PI>>(st_forward_march_kernel<C, PX, true, PI>, C::SMEM_BYTES)) != 0) return e;
-    SRST_LAUNCH_PDL((st_forward_march_kernel<C, PX, true, PI>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, MP);
+    if ((e = ensure_smem<MarchTag<C, PX, true, PI, MAP>>(st_forward_march_kernel<C, PX, true, PI, MAP>, C::SMEM_BYTES)) != 0)
+      return e;
+    SRST_LAUNCH_PDL((st_forward_march_kernel<C, PX, true, PI, MAP>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, MP);
   } else {
-    if ((e = ensure_smem<MarchTag<C, PX, false, PI>>(st_forward_march_kernel<C, PX, false, PI>, C::SMEM_BYTES)) != 0) return e;
-    SRST_LAUNCH_PDL((st_forward_march_kernel<C, PX, false, PI>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, MP);
+    if ((e = ensure_smem<MarchTag<C, PX, false, PI, MAP>>(st_forward_march_kernel<C, PX, false, PI, MAP>, C::SMEM_BYTES)) != 0)
+      return e;
+    SRST_LAUNCH_PDL((st_forward_march_kernel<C, PX, false, PI, MAP>), dim3((unsigned)grid), dim3(C::NT), C::SMEM_BYTES, stream, MP);
   }
   return (int)cudaGetLastError();
 }
@@ -400,6 +404,9 @@ struct StCall {
   int per_image = 0;                                     // reduction='none': loss_out / grad_out / grad_px are [B], and
                                                          // the MSE terms go to loss_out[B .. 2B)
   const float *px_img = nullptr, *px_other = nullptr, *grad_px = nullptr;  // backward: image pair + upstream gradient of the MSE term
+  float* map_out = nullptr;                              // forward: also store the per-pixel distances [B,H,W]
+  int unit_scale = 0;                                    // backward: ds already carries the upstream gradient of each
+                                                         // pixel and grad_out is a device 1.0f (no 1/(B H W))
   int B = 0, H = 0, W = 0, normalize = 1, vec4 = 0;
   float eps = 0.f;
   void* workspace = nullptr;
@@ -408,13 +415,16 @@ struct StCall {
   void* stream = nullptr;
 };
 
-// one tile shape with the batch or the per-image reduction (c.per_image); PX: the fused Pixel term
+// one tile shape with the batch or the per-image reduction (c.per_image), or the distance map (c.map_out, never
+// together with PX); PX: the fused Pixel term
 template <class C, bool PX, int RG, int RK>
-static int tiled_fwd(StFwdParams<RG, RK>& P, const StCall& c) {
+static int tiled_fwd(StFwdMapParams<RG, RK>& P, const StCall& c) {
+  if (c.map_out) return launch_st_forward<C, false, false, true>(P, c.stream);
   return c.per_image ? launch_st_forward<C, PX, true>(P, c.stream) : launch_st_forward<C, PX>(P, c.stream);
 }
 template <class C, bool PX>
-static int march_fwd(const StFwdParams<C::RG, C::RK>& P, const StCall& c) {
+static int march_fwd(const StFwdMapParams<C::RG, C::RK>& P, const StCall& c) {
+  if (c.map_out) return launch_st_march<C, false, false, true>(P, c.stream);
   return c.per_image ? launch_st_march<C, PX, true>(P, c.stream) : launch_st_march<C, PX>(P, c.stream);
 }
 template <class C, bool PX, int RG, int RK>
@@ -424,7 +434,8 @@ static int tiled_bwd(StBwdParams<RG, RK>& P, const StCall& c) {
 
 template <int RG, int RK>
 static int st_forward_rr(const StCall& c) {
-  static thread_local StFwdParams<RG, RK> P;  // ~0.5 KB of taps: filled in place, passed by reference to the launcher
+  static thread_local StFwdMapParams<RG, RK> P;  // ~0.5 KB of taps: filled in place, passed by reference to the launcher
+  P.map_out = c.map_out;
   P.sr = c.sr; P.hr = c.hr; P.ds_sr = c.ds_sr; P.ds_hr = c.ds_hr; P.ixy_sr = c.ixy_sr; P.ixy_hr = c.ixy_hr;
   P.ticket = reinterpret_cast<unsigned int*>(c.workspace);
   P.partials = reinterpret_cast<float*>(c.workspace) + 4;
@@ -468,7 +479,7 @@ static int st_backward_rr(const StCall& c) {
   P.img = c.px_img; P.px_other = c.px_other; P.grad_px = c.grad_px;
   P.B = c.B; P.H = c.H; P.W = c.W; P.tiles_x = P.tiles_y = 0;
   P.vec4 = c.vec4;
-  P.inv_count = (float)(1.0 / ((double)(c.per_image ? 1 : c.B) * c.H * c.W));
+  P.inv_count = c.unit_scale ? 1.0f : (float)(1.0 / ((double)(c.per_image ? 1 : c.B) * c.H * c.W));
   P.taps = cached_taps<RG, RK>(c.g, c.dg, c.rs, c.k, c.rk);
   if constexpr (RG == 2 && RK == 8) {
     if (c.px_other) {  // the fused Pixel term is compiled into the two default tile shapes
@@ -542,6 +553,13 @@ static int st_forward_generic(const StCall& c, size_t workspace_bytes) {
   }
   Q.inv_count = (float)(1.0 / ((double)c.B * c.H * c.W));
   const unsigned ngrid = nblk < (unsigned)kGenMaxPartials ? nblk : (unsigned)kGenMaxPartials;
+  if (c.map_out) {
+    StGenChainMapParams M;
+    static_cast<StGenChainParams&>(M) = Q;
+    M.map_out = c.map_out;
+    SRST_LAUNCH((gen_chain_kernel<false, true>), dim3(ngrid), dim3(kGenNT), 0, c.stream, M);
+    return (int)cudaGetLastError();
+  }
   SRST_LAUNCH(gen_chain_kernel<false>, dim3(ngrid), dim3(kGenNT), 0, c.stream, Q);
   return (int)cudaGetLastError();
 }
@@ -559,7 +577,7 @@ static int st_backward_generic(const StCall& c, void* workspace, size_t workspac
   static thread_local StGenParams P_tls;
   StGenParams& P = P_tls;
   P.B = c.B; P.H = c.H; P.W = c.W;
-  P.scale = (float)(1.0 / ((double)(c.per_image ? 1 : c.B) * c.H * c.W));
+  P.scale = c.unit_scale ? 1.0f : (float)(1.0 / ((double)(c.per_image ? 1 : c.B) * c.H * c.W));
   gen_fill_taps(P.taps, c);
   const unsigned nblk = (unsigned)((npix + kGenNT - 1) / kGenNT);
   P.in0 = c.ds; P.in1 = P.in2 = nullptr; P.out0 = V; P.out1 = nullptr;
@@ -587,10 +605,11 @@ static int st_dispatch(const StCall& c, bool forward) {
 }  // namespace srst
 
 // srst_st_forward and srst_st_forward_per_image: the same checks and dispatch; per_image selects the [B] reduction
+// (srst_st_forward_map: map_out set, per_image 0)
 static int st_forward_entry(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
                             int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss_out,
                             float* ds_sr, float* ds_hr, float* ixy_sr, float* ixy_hr, void* workspace,
-                            size_t workspace_bytes, void* stream, int per_image) {
+                            size_t workspace_bytes, void* stream, int per_image, float* map_out = nullptr) {
   if (!sr || !hr || !g || !dg || !k || !loss_out || B <= 0 || H <= 0 || W <= 0) return SRST_E_INVALID;
   if (!srst_st_supported(r_sigma, r_rho)) return SRST_E_UNSUPPORTED;
   if (!workspace || !aligned16(workspace) || workspace_bytes < srst_st_workspace_bytes(B, H, W))
@@ -602,13 +621,15 @@ static int st_forward_entry(const float* sr, const float* hr, int B, int H, int 
             (!ds_hr || aligned16(ds_hr)) && (!ixy_sr || aligned16(ixy_sr)) && (!ixy_hr || aligned16(ixy_hr))) ? 1 : 0;
   c.workspace = workspace; c.g = g; c.dg = dg; c.k = k; c.rs = r_sigma; c.rk = r_rho; c.stream = stream;
   c.per_image = per_image;
+  c.map_out = map_out;
   if (!st_compiled(r_sigma, r_rho)) return st_forward_generic(c, workspace_bytes);
   return st_dispatch(c, true);
 }
 
+// (srst_st_backward_map: ds = the weighted scratch planes, grad_out = the unit slot, unit_scale 1)
 static int st_backward_entry(const float* ixy, const float* ds, const float* grad_out, int B, int H, int W,
                              const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float* d_img,
-                             void* workspace, size_t workspace_bytes, void* stream, int per_image) {
+                             void* workspace, size_t workspace_bytes, void* stream, int per_image, int unit_scale = 0) {
   if (!ixy || !ds || !grad_out || !g || !dg || !k || !d_img || B <= 0 || H <= 0 || W <= 0) return SRST_E_INVALID;
   if (!srst_st_supported(r_sigma, r_rho)) return SRST_E_UNSUPPORTED;
   StCall c;
@@ -617,6 +638,7 @@ static int st_backward_entry(const float* ixy, const float* ds, const float* gra
   c.vec4 = (W % 4 == 0 && aligned16(d_img) && aligned16(ds)) ? 1 : 0;
   c.g = g; c.dg = dg; c.k = k; c.rs = r_sigma; c.rk = r_rho; c.stream = stream;
   c.per_image = per_image;
+  c.unit_scale = unit_scale;
   if (!st_compiled(r_sigma, r_rho)) return st_backward_generic(c, workspace, workspace_bytes);
   return st_dispatch(c, false);
 }
@@ -657,6 +679,46 @@ int srst_st_backward(const float* ixy, const float* ds, const float* grad_out, i
                      const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float* d_img,
                      void* stream) {
   return srst_st_backward_ws(ixy, ds, grad_out, B, H, W, g, dg, r_sigma, k, r_rho, d_img, nullptr, 0, stream);
+}
+
+int srst_st_forward_map(const float* sr, const float* hr, int B, int H, int W, const float* g, const float* dg,
+                        int r_sigma, const float* k, int r_rho, int normalize, float eps, float* loss_out,
+                        float* map_out, float* ds_sr, float* ds_hr, float* ixy_sr, float* ixy_hr, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+  if (!map_out) return SRST_E_INVALID;
+  return st_forward_entry(sr, hr, B, H, W, g, dg, r_sigma, k, r_rho, normalize, eps, loss_out, ds_sr, ds_hr, ixy_sr,
+                          ixy_hr, workspace, workspace_bytes, stream, 0, map_out);
+}
+
+// workspace of srst_st_backward_map: the weighted ds planes [B,3,H,W], the unit slot, then the generic-radius scratch
+static size_t st_map_ds_bytes(int B, int H, int W) { return ((size_t)B * 3 * H * W * sizeof(float) + 255) / 256 * 256; }
+constexpr size_t kMapUnitBytes = 256;
+
+size_t srst_st_backward_map_workspace_bytes(int B, int H, int W, int r_sigma, int r_rho) {
+  if (B <= 0 || H <= 0 || W <= 0 || !srst_st_supported(r_sigma, r_rho)) return 0;
+  return st_map_ds_bytes(B, H, W) + kMapUnitBytes + srst_st_backward_workspace_bytes(B, H, W, r_sigma, r_rho);
+}
+
+int srst_st_backward_map(const float* ixy, const float* ds, const float* grad_map, int B, int H, int W,
+                         const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float* d_img,
+                         void* workspace, size_t workspace_bytes, void* stream) {
+  if (!ixy || !ds || !grad_map || !g || !dg || !k || !d_img || B <= 0 || H <= 0 || W <= 0) return SRST_E_INVALID;
+  if (!srst_st_supported(r_sigma, r_rho)) return SRST_E_UNSUPPORTED;
+  if (!workspace || !aligned16(workspace) ||
+      workspace_bytes < srst_st_backward_map_workspace_bytes(B, H, W, r_sigma, r_rho))
+    return SRST_E_WORKSPACE;
+  const size_t plane = (size_t)H * W, ds_bytes = st_map_ds_bytes(B, H, W);
+  float* wds = reinterpret_cast<float*>(workspace);
+  float* unit = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + ds_bytes);
+  const bool vec4 = W % 4 == 0 && aligned16(ds) && aligned16(grad_map);
+  const size_t items = (size_t)B * plane / (vec4 ? 4 : 1);
+  const size_t want = (items + kMapNT - 1) / kMapNT, cap = (size_t)sm_count() * 16;
+  const dim3 grid((unsigned)(want < cap ? want : cap));
+  if (vec4) SRST_LAUNCH(st_map_scale_kernel<true>, grid, dim3(kMapNT), 0, stream, ds, grad_map, wds, unit, B, plane);
+  else SRST_LAUNCH(st_map_scale_kernel<false>, grid, dim3(kMapNT), 0, stream, ds, grad_map, wds, unit, B, plane);
+  if (const int e = (int)cudaGetLastError()) return e;
+  return st_backward_entry(ixy, wds, unit, B, H, W, g, dg, r_sigma, k, r_rho, d_img, unit + kMapUnitBytes / sizeof(float),
+                           workspace_bytes - ds_bytes - kMapUnitBytes, stream, 0, 1);
 }
 
 }  // extern "C"

@@ -141,9 +141,15 @@ struct StGenChainParams {
   int B, H, W, normalize;
   float eps, inv_count;
 };
+// MAP: the distance map [B,H,W] (see StFwdMapParams)
+struct StGenChainMapParams : StGenChainParams {
+  float* map_out;
+};
 
-// chain of pixel i (flat over [B][H][W]): adds its distance to lsum, writes its ds_sr / ds_hr
-SRST_DEV void gen_chain_pixel(const StGenChainParams& P, size_t i, size_t plane, float& lsum) {
+// chain of pixel i (flat over [B][H][W]): adds its distance to lsum, writes its ds_sr / ds_hr (and with MAP its
+// distance to map[i])
+template <bool MAP = false>
+SRST_DEV void gen_chain_pixel(const StGenChainParams& P, size_t i, size_t plane, float& lsum, float* map = nullptr) {
   const size_t b = i / plane, o = b * 3 * plane + (i - b * plane);
   const float a = __ldg(P.s1 + o), bb = __ldg(P.s1 + o + plane), c = __ldg(P.s1 + o + 2 * plane);
   const float e = __ldg(P.s2 + o), f = __ldg(P.s2 + o + plane), h = __ldg(P.s2 + o + 2 * plane);
@@ -152,6 +158,7 @@ SRST_DEV void gen_chain_pixel(const StGenChainParams& P, size_t i, size_t plane,
   const float2 d = st_pixel2_raw<true, true>(bcast2(a), bcast2(bb), bcast2(c), bcast2(e), bcast2(f), bcast2(h),
                                             P.normalize != 0, P.eps, G);
   lsum += d.x;
+  if constexpr (MAP) map[i] = d.x;
   if (P.ds_sr) { P.ds_sr[o] = G.da.x; P.ds_sr[o + plane] = G.db.x; P.ds_sr[o + 2 * plane] = G.dc.x; }
   if (P.ds_hr) { P.ds_hr[o] = G.de.x; P.ds_hr[o + plane] = G.df.x; P.ds_hr[o + 2 * plane] = G.dh.x; }
 }
@@ -160,8 +167,11 @@ SRST_DEV void gen_chain_pixel(const StGenChainParams& P, size_t i, size_t plane,
 // workspace, last CTA sums in a fixed order in double and hands the ticket back zeroed).
 // PER_IMG: reduction='none' -- the grid is gridDim.x / B CTAs per image, image-major, each striding over its own
 // image only; loss_out[b] = the mean over image b's pixels (P.inv_count = 1 / (H W)).
-template <bool PER_IMG = false>
-__global__ void __launch_bounds__(kGenNT) gen_chain_kernel(const __grid_constant__ StGenChainParams P) {
+// MAP: also stores every pixel's distance into P.map_out [B,H,W] (the loss and the other outputs are unchanged).
+template <bool PER_IMG = false, bool MAP = false>
+__global__ void __launch_bounds__(kGenNT)
+gen_chain_kernel(const __grid_constant__ std::conditional_t<MAP, StGenChainMapParams, StGenChainParams> P) {
+  static_assert(!(MAP && PER_IMG), "the distance map comes with the batch loss only");
   __shared__ float s_red[kGenNT / 32];
   __shared__ unsigned int s_last;
   const size_t plane = (size_t)P.H * P.W, npix = (size_t)P.B * plane;
@@ -172,8 +182,10 @@ __global__ void __launch_bounds__(kGenNT) gen_chain_kernel(const __grid_constant
     for (size_t i = (size_t)b * plane + (size_t)(blockIdx.x - b * per) * kGenNT + threadIdx.x; i < end; i += (size_t)per * kGenNT)
       gen_chain_pixel(P, i, plane, lsum);
   } else {
-    for (size_t i = (size_t)blockIdx.x * kGenNT + threadIdx.x; i < npix; i += (size_t)gridDim.x * kGenNT)
-      gen_chain_pixel(P, i, plane, lsum);
+    for (size_t i = (size_t)blockIdx.x * kGenNT + threadIdx.x; i < npix; i += (size_t)gridDim.x * kGenNT) {
+      if constexpr (MAP) gen_chain_pixel<true>(P, i, plane, lsum, P.map_out);
+      else gen_chain_pixel(P, i, plane, lsum);
+    }
   }
   lsum = warp_sum(lsum);
   if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = lsum;

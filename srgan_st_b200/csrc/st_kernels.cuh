@@ -29,6 +29,8 @@
 //     and parks each image's smoothed tensor in a thread-private shared-memory slot, so the
 //     per-pixel chain starts with an empty register file (no spills) and is itself a rolled loop.
 #pragma once
+#include <type_traits>
+
 #include "srst_device.cuh"
 
 namespace srst {
@@ -71,6 +73,15 @@ struct StFwdParams {
   float inv_count;
   StTaps<RG, RK> taps;
 };
+
+// MAP forward (srst_st_forward_map): the distance of every pixel also goes to map_out [B,H,W].  A derived type, so
+// that the parameter layout of the other instantiations stays as it is.
+template <int RG, int RK>
+struct StFwdMapParams : StFwdParams<RG, RK> {
+  float* map_out;
+};
+template <int RG, int RK, bool MAP>
+using StFwdParamsT = std::conditional_t<MAP, StFwdMapParams<RG, RK>, StFwdParams<RG, RK>>;
 
 template <int RG, int RK>
 struct StBwdParams {
@@ -400,12 +411,14 @@ SRST_DEV void smooth_h_rowpair_n(const float* row, const Taps& tp, float2 (&out)
   }
 }
 // Chain + stores for one thread's 2 x 4 pixels; returns the sum of the valid distances.
-template <bool WANT_HR>
+// MAP: the distances also go to `map` (image b's [H,W] plane of the map), under the masks of the ds stores.
+template <bool WANT_HR, bool MAP = false>
 SRST_DEV float st_chain_store(const float2 (&S1)[3][4], const float2 (&S2)[3][4], bool norm, float eps,
                               float* __restrict__ ds_sr, float* __restrict__ ds_hr, size_t img_off, int H, int W,
-                              int gy0, int gx0, bool vec4) {
+                              int gy0, int gx0, bool vec4, float* __restrict__ map = nullptr) {
   float lsum = 0.f;
   float2 gs[3][4], gh[3][4];
+  [[maybe_unused]] float2 dm[4];
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     StPixelGrad2 G;
@@ -416,6 +429,7 @@ SRST_DEV float st_chain_store(const float2 (&S1)[3][4], const float2 (&S2)[3][4]
     lsum += (okx && gy0 + 1 < H) ? d.y : 0.f;
     gs[0][j] = G.da; gs[1][j] = G.db; gs[2][j] = G.dc;
     if (WANT_HR) { gh[0][j] = G.de; gh[1][j] = G.df; gh[2][j] = G.dh; }
+    if constexpr (MAP) dm[j] = d;
   }
   if (gx0 >= W) return lsum;
   const size_t plane = (size_t)H * W;
@@ -423,6 +437,19 @@ SRST_DEV float st_chain_store(const float2 (&S1)[3][4], const float2 (&S2)[3][4]
   for (int hf = 0; hf < 2; ++hf) {
     if (gy0 + hf >= H) continue;
     const size_t o = img_off + (size_t)(gy0 + hf) * W + gx0;
+    if constexpr (MAP) {
+      float* m = map + (size_t)(gy0 + hf) * W + gx0;
+      const float m0 = hf ? dm[0].y : dm[0].x, m1 = hf ? dm[1].y : dm[1].x;
+      const float m2 = hf ? dm[2].y : dm[2].x, m3 = hf ? dm[3].y : dm[3].x;
+      if (vec4 && (reinterpret_cast<uintptr_t>(map) & 15u) == 0) {
+        st4(m, make_float4(m0, m1, m2, m3));
+      } else {
+        const float mm[4] = {m0, m1, m2, m3};
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          if (gx0 + j < W) m[j] = mm[j];
+      }
+    }
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
       const float v0 = hf ? gs[c][0].y : gs[c][0].x, v1 = hf ? gs[c][1].y : gs[c][1].x;
@@ -689,10 +716,12 @@ SRST_DEV void st_unit_tensor(float* smem, const float* __restrict__ base, float*
 }
 
 // PER_IMG: reduction='none' -- loss_out[b] is the mean over image b's pixels (P.inv_count = 1 / (H W)) instead of
-// loss_out[0] over the batch; with PX, loss_out[B + b] is image b's mean squared difference over its 3 H W values
-template <class C, bool PX = false, bool WANT_HR = false, bool PER_IMG = false>
+// loss_out[0] over the batch; with PX, loss_out[B + b] is image b's mean squared difference over its 3 H W values.
+// MAP: also stores every pixel's distance into P.map_out [B,H,W] (the loss and the other outputs are unchanged).
+template <class C, bool PX = false, bool WANT_HR = false, bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(C::NT, C::MINB)
-st_forward_kernel(const __grid_constant__ StFwdParams<C::RG, C::RK> P) {
+st_forward_kernel(const __grid_constant__ StFwdParamsT<C::RG, C::RK, MAP> P) {
+  static_assert(!(MAP && (PX || PER_IMG)), "the distance map comes with the batch loss only");
   SRST_DYN_SMEM(float, smem);
   __shared__ float s_red[32];
   __shared__ unsigned int s_last;
@@ -728,8 +757,13 @@ st_forward_kernel(const __grid_constant__ StFwdParams<C::RG, C::RK> P) {
     st_unit_tensor<C, PX>(smem, P.hr + img_off, P.ixy_hr, b, vec4, H, W, y0, x0, P.taps, tid, dvalid, q, seg, S2,
                           PX ? P.sr + img_off : nullptr, &pxsum, 4);
     SRST_STAMP(8);
-    if (dvalid)
-      lsum = st_chain_store<WANT_HR>(S1, S2, norm, P.eps, P.ds_sr, P.ds_hr, img_off, H, W, gy0, gx0, vec4);
+    if (dvalid) {
+      if constexpr (MAP)
+        lsum = st_chain_store<WANT_HR, true>(S1, S2, norm, P.eps, P.ds_sr, P.ds_hr, img_off, H, W, gy0, gx0, vec4,
+                                             P.map_out + (size_t)b * H * W);
+      else
+        lsum = st_chain_store<WANT_HR>(S1, S2, norm, P.eps, P.ds_sr, P.ds_hr, img_off, H, W, gy0, gx0, vec4);
+    }
   } else {
     // SR, then HR, through one copy of the filter code
   #pragma unroll 1
@@ -764,6 +798,11 @@ st_forward_kernel(const __grid_constant__ StFwdParams<C::RG, C::RK> P) {
         const bool okx = gx0 + j < W;
         lsum += (okx && gy0 < H) ? d.x : 0.f;
         lsum += (okx && gy0 + 1 < H) ? d.y : 0.f;
+        if constexpr (MAP) {
+          float* m = P.map_out + (size_t)b * H * W + (size_t)gy0 * W + gx0 + j;
+          if (okx && gy0 < H) m[0] = d.x;
+          if (okx && gy0 + 1 < H) m[W] = d.y;
+        }
         st2(a1, G.da); st2(a1 + 8 * C::NT, G.db); st2(a1 + 16 * C::NT, G.dc);
         if (WANT_HR) { st2(a2, G.de); st2(a2 + 8 * C::NT, G.df); st2(a2 + 16 * C::NT, G.dh); }
       }
@@ -1184,6 +1223,36 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
       if (P.use_tma && tid == 0 && next < ntiles) { fence_async_smem(); issue_s(next); issue_i(next); }
     }
   }  // tile loop
+}
+
+// Backward prepass of the distance map (srst_st_backward_map): out[b][c] = grad_map[b] * ds[b][c] for the three ds
+// planes, and *unit = 1.  The unchanged backward then runs on `out` with `unit` as its upstream gradient and a unit
+// scale, so d_img is the adjoint of grad_map * ds.  VEC4: W % 4 == 0 and all three pointers 16-byte aligned.
+constexpr int kMapNT = 256;
+template <bool VEC4>
+__global__ void __launch_bounds__(kMapNT) st_map_scale_kernel(const float* __restrict__ ds,
+                                                              const float* __restrict__ grad_map, float* __restrict__ out,
+                                                              float* __restrict__ unit, int B, size_t plane) {
+  pdl_wait();  // grad_map may come from the kernel enqueued just before
+  pdl_trigger();
+  if (blockIdx.x == 0 && threadIdx.x == 0) *unit = 1.0f;
+  constexpr int V = VEC4 ? 4 : 1;
+  const size_t n = (size_t)B * plane / V;
+  for (size_t i = (size_t)blockIdx.x * kMapNT + threadIdx.x; i < n; i += (size_t)gridDim.x * kMapNT) {
+    const size_t p = i * V, b = p / plane, o = p + 2 * b * plane;  // o: channel 0 of pixel p in [B][3][H][W]
+    if constexpr (VEC4) {
+      const float4 g = ldg4(grad_map + p);
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        const float4 v = ldg4(ds + o + c * plane);
+        st4(out + o + c * plane, make_float4(g.x * v.x, g.y * v.y, g.z * v.z, g.w * v.w));
+      }
+    } else {
+      const float g = __ldg(grad_map + p);
+#pragma unroll
+      for (int c = 0; c < 3; ++c) out[o + c * plane] = g * __ldg(ds + o + c * plane);
+    }
+  }
 }
 
 }  // namespace srst

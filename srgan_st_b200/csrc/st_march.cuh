@@ -58,6 +58,13 @@ struct StMarchParams {
   StFwdParams<RG, RK> F;
   int nstrips, nchunks, chunk_blocks;  // grid = B * nchunks * nstrips; a chunk = chunk_blocks * 16 rows
 };
+// MAP: the distance map [B,H,W] (see StFwdMapParams)
+template <int RG, int RK>
+struct StMarchMapParams : StMarchParams<RG, RK> {
+  float* map_out;
+};
+template <int RG, int RK, bool MAP>
+using StMarchParamsT = std::conditional_t<MAP, StMarchMapParams<RG, RK>, StMarchParams<RG, RK>>;
 
 template <int TW_, int RG_, int RK_, int CR_ = 8>
 struct StMarchCfg {
@@ -178,10 +185,12 @@ SRST_DEV float2 st_pixel2_raw(float2 a, float2 b, float2 c, float2 e, float2 f, 
 }
 
 // PER_IMG: reduction='none' -- loss_out[b] is the mean over image b's pixels (P.inv_count = 1 / (H W)) instead of
-// loss_out[0] over the batch; with PX, loss_out[B + b] is image b's mean squared difference over its 3 H W values
-template <class C, bool PX = false, bool WANT_HR = false, bool PER_IMG = false>
+// loss_out[0] over the batch; with PX, loss_out[B + b] is image b's mean squared difference over its 3 H W values.
+// MAP: also stores every pixel's distance into MP.map_out [B,H,W] (the loss and the other outputs are unchanged).
+template <class C, bool PX = false, bool WANT_HR = false, bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(C::NT, C::MINB)
-st_forward_march_kernel(const __grid_constant__ StMarchParams<C::RG, C::RK> MP) {
+st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP> MP) {
+  static_assert(!(MAP && (PX || PER_IMG)), "the distance map comes with the batch loss only");
   SRST_DYN_SMEM(float, smem);
   __shared__ float s_red[32];
   __shared__ unsigned int s_last;
@@ -562,6 +571,8 @@ st_forward_march_kernel(const __grid_constant__ StMarchParams<C::RG, C::RK> MP) 
       if (gx < W) {
         float* ps = P.ds_sr ? P.ds_sr + img_off + (size_t)ry * W + gx : nullptr;
         [[maybe_unused]] float* ph = WANT_HR ? P.ds_hr + img_off + (size_t)ry * W + gx : nullptr;
+        [[maybe_unused]] float* pm = nullptr;
+        if constexpr (MAP) pm = MP.map_out + (size_t)b * plane + (size_t)ry * W + gx;
         // all four pixel pairs are evaluated unconditionally (rows past the chunk hold finite filler) so that the
         // compiler can interleave their SFU / FMA dependency chains; only the loss and the stores are masked
 #pragma unroll
@@ -583,6 +594,11 @@ st_forward_march_kernel(const __grid_constant__ StMarchParams<C::RG, C::RK> MP) 
             if (one) { ph[0] = G.de.x; ph[plane] = G.df.x; ph[2 * plane] = G.dh.x; }
             if (two) { ph[W] = G.de.y; ph[plane + W] = G.df.y; ph[2 * plane + W] = G.dh.y; }
             ph += 2 * W;
+          }
+          if constexpr (MAP) {
+            if (one) pm[0] = d.x;
+            if (two) pm[W] = d.y;
+            pm += 2 * W;
           }
         }
       }

@@ -242,6 +242,75 @@ class StructureTensorLoss(nn.Module):
         return r if self.reduction == "mean" else f"{r}, {_reduction_repr(self.reduction)}"
 
 
+class _StructureTensorDistanceFn(torch.autograd.Function):
+    """autograd boundary of the per-pixel distance map (srst_st_forward_map / srst_st_backward_map).  Saves what
+    `_StructureTensorLossFn` saves: per image that needs a gradient, ONE buffer of ds planes followed by Ix, Iy.  The
+    upstream gradient is any [B,H,W] tensor."""
+
+    @staticmethod
+    def forward(ctx, sr, hr, sigma, rho, normalize):
+        lib = _cabi.lib()
+        sr = sr.contiguous()
+        hr = hr.contiguous()
+        B, _, H, W = sr.shape
+        tp = _st_taps(sigma, rho, "structure_tensor_distance")
+        need = ctx.needs_input_grad
+        n_ds, n_ixy, ws_bytes, _ = _st_sizes(B, H, W, tp[2], tp[4])
+        with _on_device(sr.device):
+            stream = _raw_stream(sr.device)
+            loss = torch.empty((), dtype=torch.float32, device=sr.device)
+            dmap = torch.empty((B, H, W), dtype=torch.float32, device=sr.device)
+            saved = [torch.empty(n_ds + n_ixy, dtype=torch.float32, device=sr.device) if n else None for n in need[:2]]
+            ds = [t.data_ptr() if t is not None else None for t in saved]
+            ixy = [p + 4 * n_ds if p is not None else None for p in ds]
+            ws = _workspace("st", sr.device, stream, ws_bytes)
+            rc = lib.srst_st_forward_map(sr.data_ptr(), hr.data_ptr(), B, H, W, tp[0], tp[1], tp[2], tp[3], tp[4],
+                                         int(bool(normalize)), 1e-12, loss.data_ptr(), dmap.data_ptr(), ds[0], ds[1],
+                                         ixy[0], ixy[1], ws.data_ptr(), ws.numel(), stream)
+        if rc:
+            _cabi.check(rc, "srst_st_forward_map")
+        ctx.save_for_backward(saved[0], saved[1])
+        ctx.meta = (tp, B, H, W, n_ds)
+        return dmap
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_map):
+        lib = _cabi.lib()
+        tp, B, H, W, n_ds = ctx.meta
+        if grad_map.dtype != torch.float32 or not grad_map.is_contiguous():   # also the stride-0 ones of .sum() / .mean()
+            grad_map = grad_map.to(torch.float32).contiguous()
+        outs = [None, None]
+        dev = grad_map.device
+        with _on_device(dev):
+            stream = _raw_stream(dev)
+            ws = None
+            for i, saved in enumerate(ctx.saved_tensors):
+                if saved is None or not ctx.needs_input_grad[i]:
+                    continue
+                if ws is None:   # weighted ds planes + unit slot (+ the generic path's planes); the two calls run in order
+                    ws = _workspace("st_map_bwd", dev, stream,
+                                    lib.srst_st_backward_map_workspace_bytes(B, H, W, tp[2], tp[4]))
+                d_img = torch.empty((B, 3, H, W), dtype=torch.float32, device=dev)
+                rc = lib.srst_st_backward_map(saved.data_ptr() + 4 * n_ds, saved.data_ptr(), grad_map.data_ptr(), B, H, W,
+                                              tp[0], tp[1], tp[2], tp[3], tp[4], d_img.data_ptr(), ws.data_ptr(),
+                                              ws.numel(), stream)
+                if rc:
+                    _cabi.check(rc, "srst_st_backward_map")
+                outs[i] = d_img
+        return outs[0], outs[1], None, None, None
+
+
+def structure_tensor_distance(x: torch.Tensor, gt: torch.Tensor, sigma: float = 0.5, rho: float = 2.0,
+                              normalize: bool = True) -> torch.Tensor:
+    """Per-pixel structure-tensor distance between x (SR) and gt (HR), both ``[B,3,H,W]`` fp32 CUDA: the ``[B,H,W]``
+    fp32 map whose mean is ``StructureTensorLoss(sigma, rho, normalize)(x, gt)`` (the map ``compute_distance`` builds
+    before ``st_loss`` takes its mean, reference loss.py:408-409, utils.py:269-279).  Differentiable w.r.t. x, and w.r.t.
+    gt when gt requires grad, under any upstream gradient, e.g. a spatial weighting ``(d * w).sum() / w.sum()``."""
+    _check_pair(x, gt, "structure_tensor_distance")
+    return _StructureTensorDistanceFn.apply(x, gt, sigma, rho, normalize)
+
+
 def structure_tensor_features(img: torch.Tensor, sigma: float = 0.5, rho: float = 2.0):
     """Diagnostic structure-tensor features of ``img`` ``[B,3,H,W]`` (fp32 CUDA), no gradient: a dict with
     ``J`` ``[B,3,H,W]`` (Jxx, Jyy, Jxy as reference utils.py:212-233 names them), ``eigenvalues`` ``[B,2,H,W]`` (small,
