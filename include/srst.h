@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define SRST_VERSION 207 /* major*100 + minor: the major number changes whenever an argument list changes */
+#define SRST_VERSION 208 /* major*100 + minor: the major number changes whenever an argument list changes */
 
 #define SRST_E_INVALID (-1)     /* null pointer / non-positive size / bad enum */
 #define SRST_E_UNSUPPORTED (-2) /* filter radius or patch geometry not compiled in */
@@ -352,6 +352,33 @@ int srst_patch_backward_per_image(int mode, const float* sr, const float* gt, co
                                   int criterion,
                                   float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Per-patch loss map (the element-wise form of the three patch losses: one criterion value per query patch, the
+ * `L1Loss()(p1, sel_p2)` / MSELoss terms of loss.py:139, :222, :371 before their mean), e.g. for spatial weighting or
+ * masking of the loss and for heat maps of the patches that found no good buddy.
+ *   srst_patch_forward_map: the arguments of srst_patch_forward_per_image with map_out (device [B][N] fp32, required)
+ *     after loss_out.  map_out[b*N + n] = the mean over the D criterion terms of query patch n of image b against its
+ *     selected candidate (D = 27 for modes 0 and 2, 9 for mode 1).  loss_out[0] and idx_out are bit-identical to
+ *     srst_bb_forward / srst_gram_forward / srst_pst_forward on the same inputs (same search, same loss grid, same
+ *     reduction order), so loss_out[0] = mean(map_out) up to the order of the summation.
+ *   srst_patch_backward_map: the arguments of srst_patch_backward_per_image with grad_map (device [B][N], any values)
+ *     in place of grad_out: query n of image b contributes with scale grad_map[b*N + n] / D, so d_sr / d_gt = the
+ *     gradient of sum(grad_map * map_out).  Either of d_sr / d_gt may be NULL, not both; d_gt sums with atomicAdd (last
+ *     bits may vary, as for srst_patch_backward_gt).
+ * A NULL map_out / grad_map returns SRST_E_INVALID; every other check, return code and workspace rule is that of the
+ * per-image twins. */
+int srst_patch_forward_map(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                           int B, int H, int W,
+                           const float* g, const float* dg, int r_sigma, const float* k, int r_rho,
+                           float alpha, float beta, int criterion,
+                           int64_t* idx_out, float* loss_out, float* map_out,
+                           void* workspace, size_t workspace_bytes, void* stream);
+int srst_patch_backward_map(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                            const int64_t* idx, const float* grad_map,
+                            int B, int H, int W,
+                            const float* g, const float* dg, int r_sigma, const float* k, int r_rho,
+                            int criterion,
+                            float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Best-Buddy loss with an arbitrary patch geometry: BestBuddyLoss(ksize, pad, stride) of the reference
  * (loss.py:86; F.unfold(kernel_size=ksize, padding=pad, stride=stride) at loss.py:116-129) for everything
@@ -395,6 +422,23 @@ int srst_bbg_backward_per_image(const float* sr, const float* gt, const float* g
                                 int B, int H, int W, int ksize, int pad, int stride, int criterion,
                                 float* d_sr, float* d_gt,
                                 void* workspace, size_t workspace_bytes, void* stream);
+
+/* Per-patch loss map of the arbitrary-geometry path: the arguments, checks and workspace of srst_bbg_forward_per_image /
+ * srst_bbg_backward_per_image, with map_out (device [B][N] fp32, required) after loss_out and grad_map (device [B][N])
+ * in place of grad_out, as for srst_patch_forward_map / srst_patch_backward_map.  D = 3*ksize*ksize, N and the
+ * row-major patch order as F.unfold.  loss_out[0] and idx_out are bit-identical to srst_bbg_forward.  d_sr stays
+ * deterministic: a pixel sums the gradients of the patches that cover it, each with its own weight, in a fixed order.
+ * A NULL map_out / grad_map returns SRST_E_INVALID. */
+int srst_bbg_forward_map(const float* sr, const float* gt, const float* gt2, const float* gt4,
+                         int B, int H, int W, int ksize, int pad, int stride,
+                         float alpha, float beta, int criterion,
+                         int64_t* idx_out, float* loss_out, float* map_out,
+                         void* workspace, size_t workspace_bytes, void* stream);
+int srst_bbg_backward_map(const float* sr, const float* gt, const float* gt2, const float* gt4,
+                          const int64_t* idx, const float* grad_map,
+                          int B, int H, int W, int ksize, int pad, int stride, int criterion,
+                          float* d_sr, float* d_gt,
+                          void* workspace, size_t workspace_bytes, void* stream);
 
 /* The HR pyramid on its own (exposed for tests): out2 [B,3,H/2,W/2], out4 [B,3,H/4,W/4]. */
 int srst_bb_pyramid(const float* gt, int B, int H, int W, float* out2, float* out4, void* stream);

@@ -94,6 +94,13 @@ SIGNATURES = {
     "srst_patch_backward_per_image": (ctypes.c_int, [ctypes.c_int, vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int,
                                                      ctypes.c_int, c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
                                                      ctypes.c_int, vp, vp, vp, ctypes.c_size_t, vp]),
+    "srst_patch_forward_map": (ctypes.c_int, [ctypes.c_int, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                              c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                              ctypes.c_float, ctypes.c_float, ctypes.c_int, vp, vp, vp,
+                                              vp, ctypes.c_size_t, vp]),
+    "srst_patch_backward_map": (ctypes.c_int, [ctypes.c_int, vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int,
+                                               ctypes.c_int, c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_int,
+                                               ctypes.c_int, vp, vp, vp, ctypes.c_size_t, vp]),
     "srst_bbg_supported": (ctypes.c_int, [ctypes.c_int] * 3),
     "srst_bbg_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int] * 6),
     "srst_bbg_num_patches": (ctypes.c_longlong, [ctypes.c_int] * 5),
@@ -111,6 +118,13 @@ SIGNATURES = {
     "srst_bbg_backward_per_image": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                    ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp,
                                                    vp, ctypes.c_size_t, vp]),
+    "srst_bbg_forward_map": (ctypes.c_int, [vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                            ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                            ctypes.c_float, ctypes.c_float, ctypes.c_int, vp, vp, vp,
+                                            vp, ctypes.c_size_t, vp]),
+    "srst_bbg_backward_map": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                             ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp,
+                                             vp, ctypes.c_size_t, vp]),
     "srst_bb_pyramid": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp, vp]),
 }
 

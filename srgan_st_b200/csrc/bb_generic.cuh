@@ -279,11 +279,13 @@ SRST_DEV float bbg_loss_term(const float* sr, const float* gt, const float* gt2,
 
 // one thread per query patch.  PER_IMG: reduction='none' -- ceil(N / BBG_NT) CTAs per image, image-major, so no CTA
 // spans two images; loss_out[b] = the mean over image b's N*D terms.
-template <bool PER_IMG = false>
+// MAP: the scalar grid and reduction (loss_out[0] keeps its bits), and every query's term / D also goes to map_out[B][N].
+template <bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(BBG_NT)
 bbg_loss_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                 const float* __restrict__ gt4, BbgGeom g, const int64_t* __restrict__ idx, int criterion, float* partials,
-                unsigned int* ticket, float* loss_out) {
+                unsigned int* ticket, float* loss_out, float* __restrict__ map_out = nullptr) {
+  static_assert(!(MAP && PER_IMG), "the loss map comes with the batch loss");
   __shared__ float s_red[BBG_NT / 32];
   __shared__ unsigned int s_last;
   const int tid = threadIdx.x;
@@ -296,6 +298,7 @@ bbg_loss_kernel(const float* __restrict__ sr, const float* __restrict__ gt, cons
   } else if (t < (size_t)g.B * g.N) {
     const int b = (int)(t / g.N), i = (int)(t - (size_t)b * g.N);
     acc = bbg_loss_term(sr, gt, gt2, gt4, g, criterion, b, i, (int)idx[t]);
+    if constexpr (MAP) map_out[t] = acc / (float)g.D;
   }
   acc = warp_sum(acc);
   if ((tid & 31) == 0) s_red[tid >> 5] = acc;
@@ -332,8 +335,10 @@ SRST_DEV float bbg_crit_grad(float d, int criterion, float scale) {
 }
 
 // one thread per SR pixel: the patches py in [ceil((y + p - k + 1)/s), floor((y + p)/s)] x likewise px cover it.
-// PER_IMG: reduction='none', grad_out is [B] and image b scales by grad_out[b] / (N D)
-template <bool PER_IMG = false>
+// PER_IMG: reduction='none', grad_out is [B] and image b scales by grad_out[b] / (N D).
+// MAP: the loss map, grad_out is [B][N]: every covering patch q scales by its own grad_out[b N + q] / D, in the same
+// fixed order.
+template <bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(256)
 bbg_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                     const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -345,7 +350,9 @@ bbg_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, 
   const int y = (int)((t / W) % H);
   const int c = (int)((t / ((size_t)W * H)) % 3);
   const int b = (int)(t / ((size_t)3 * W * H));
-  const float scale = __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : g.B) * (float)g.N * (float)g.D);
+  float scale = 0.f;
+  if constexpr (!MAP)
+    scale = __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : g.B) * (float)g.N * (float)g.D);
   const float v = __ldg(sr + t);
   const int ylo = y + g.p - g.k + 1, xlo = x + g.p - g.k + 1;
   const int py0 = ylo <= 0 ? 0 : (ylo + g.s - 1) / g.s, py1 = min((y + g.p) / g.s, g.L[0].ny - 1);
@@ -353,18 +360,21 @@ bbg_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, 
   float out = 0.f;
   for (int py = py0; py <= py1; ++py)
     for (int px = px0; px <= px1; ++px) {
-      int j = (int)idx[(size_t)b * g.N + py * g.L[0].nx + px];
+      const size_t q = (size_t)b * g.N + py * g.L[0].nx + px;
+      int j = (int)idx[q];
       j = min(max(j, 0), g.M - 1);
       const BbgPatch Pc = bbg_candidate(gt, gt2, gt4, g, b, j);
       const float sel = bbg_value(Pc, c, y + g.p - py * g.s, x + g.p - px * g.s);
+      if constexpr (MAP) scale = __ldg(grad_out + q) / (float)g.D;
       out += bbg_crit_grad(v - sel, criterion, scale);
     }
   d_sr[t] = out;
 }
 
 // one thread per (query patch, channel): minus the SR-side gradient lands on the selected candidate's pixels
-// (PER_IMG: reduction='none', grad_out is [B] and image b scales by grad_out[b] / (N D))
-template <bool PER_IMG = false>
+// (PER_IMG: reduction='none', grad_out is [B] and image b scales by grad_out[b] / (N D); MAP: the loss map, grad_out
+// is [B][N] and query i of image b scales by grad_out[b N + i] / D)
+template <bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(256)
 bbg_backward_gt_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                        const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -376,7 +386,8 @@ bbg_backward_gt_kernel(const float* __restrict__ sr, const float* __restrict__ g
   const int b = (int)(bi / g.N), i = (int)(bi - (size_t)b * g.N);
   int j = (int)idx[bi];
   j = min(max(j, 0), g.M - 1);
-  const float scale = __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : g.B) * (float)g.N * (float)g.D);
+  const float scale = MAP ? __ldg(grad_out + bi) / (float)g.D
+                          : __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : g.B) * (float)g.N * (float)g.D);
   const BbgPatch P1 = bbg_patch_of(sr + (size_t)b * 3 * g.L[0].H * g.L[0].W, g.L[0], g.p, g.s, i);
   const BbgPatch Pc = bbg_candidate(gt, gt2, gt4, g, b, j);
   const int l = j < g.L[0].n ? 0 : (j < g.L[0].n + g.L[1].n ? 1 : 2);

@@ -811,19 +811,23 @@ SRST_DEV float bb_loss_term(const float* mats, size_t per_image, const BbGeom& g
   return acc;
 }
 
-// Criterion-gradient scale of a term of image b over `D` elements: grad_out[0] / (B N D) for the batch mean,
-// grad_out[b] / (N D) per image (reduction='none': grad_out is [B]).
-template <bool PER_IMG>
-SRST_DEV float patch_grad_scale(const float* __restrict__ grad_out, int b, int B, int N, float D) {
-  return __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : B) * (float)N * D);
+// Criterion-gradient scale of a term of query i of image b over `D` elements: grad_out[0] / (B N D) for the batch
+// mean, grad_out[b] / (N D) per image (reduction='none': grad_out is [B]), grad_out[b N + i] / D per patch (MAP, the
+// loss map: grad_out is [B][N]).
+template <bool PER_IMG, bool MAP = false>
+SRST_DEV float patch_grad_scale(const float* __restrict__ grad_out, int b, int B, int N, float D, int i = 0) {
+  if constexpr (MAP) return __ldg(grad_out + (size_t)b * N + i) / D;
+  else return __ldg(grad_out + (PER_IMG ? b : 0)) / ((float)(PER_IMG ? 1 : B) * (float)N * D);
 }
 
 // PER_IMG: reduction='none' -- ceil(N / BB_NT) CTAs per image, image-major, so no CTA spans two images;
 // loss_out[b] = the mean over image b's N*D terms.
-template <int D, bool PER_IMG = false>
+// MAP: the scalar grid and reduction (loss_out[0] keeps its bits), and every query's term / D also goes to map_out[B][N].
+template <int D, bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(BB_NT)
 bb_loss_kernel(const float* __restrict__ mats, size_t per_image, BbGeom g, const int64_t* __restrict__ idx,
-               int criterion, float* partials, unsigned int* ticket, float* loss_out) {
+               int criterion, float* partials, unsigned int* ticket, float* loss_out, float* __restrict__ map_out = nullptr) {
+  static_assert(!(MAP && PER_IMG), "the loss map comes with the batch loss");
   __shared__ float s_red[BB_NT / 32];
   __shared__ unsigned int s_last;
   const int tid = threadIdx.x;
@@ -836,6 +840,7 @@ bb_loss_kernel(const float* __restrict__ mats, size_t per_image, BbGeom g, const
   } else if (t < (size_t)g.B * g.N) {
     const int b = (int)(t / g.N), i = (int)(t - (size_t)b * g.N);
     acc = bb_loss_term<D>(mats, per_image, g, b, i, (int)idx[t], criterion);
+    if constexpr (MAP) map_out[t] = acc / (float)D;
   }
   acc = warp_sum(acc);
   if ((tid & 31) == 0) s_red[tid >> 5] = acc;
@@ -878,8 +883,8 @@ SRST_DEV float bb_candidate_value(const float* gt, const float* gt2, const float
   return __ldg(img + ((size_t)c * H + 3 * py + ky) * W + 3 * px + kx);
 }
 
-// PER_IMG: reduction='none', grad_out is [B] (patch_grad_scale)
-template <bool PER_IMG = false>
+// PER_IMG: reduction='none', grad_out is [B]; MAP: the loss map, grad_out is [B][N] (patch_grad_scale)
+template <bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(256)
 bb_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                    const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -898,7 +903,7 @@ bb_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, c
     const int j = (int)idx[(size_t)b * g.N + i];
     const float sel = bb_candidate_value(gt, gt2, gt4, g, b, j, c, y - 3 * py, x - 3 * px);
     const float d = __ldg(sr + t) - sel;
-    const float scale = patch_grad_scale<PER_IMG>(grad_out, b, g.B, g.N, (float)BB_D);
+    const float scale = patch_grad_scale<PER_IMG, MAP>(grad_out, b, g.B, g.N, (float)BB_D, i);
     out = (criterion == 0) ? ((d > 0.f) ? scale : ((d < 0.f) ? -scale : 0.f)) : 2.0f * d * scale;
   }
   d_sr[t] = out;
@@ -937,8 +942,8 @@ __global__ void __launch_bounds__(256) bb_fill_zero_kernel(float* __restrict__ p
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = 0.f;
 }
 
-// BestBuddyLoss: one thread per query patch (PER_IMG: grad_out is [B], patch_grad_scale)
-template <bool PER_IMG = false>
+// BestBuddyLoss: one thread per query patch (PER_IMG: grad_out is [B]; MAP: [B][N]; patch_grad_scale)
+template <bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(256)
 bb_backward_gt_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                       const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -950,7 +955,7 @@ bb_backward_gt_kernel(const float* __restrict__ sr, const float* __restrict__ gt
   float v[BB_D], w[BB_D];
   bb_read_patch(sr + (size_t)b * 3 * g.H * g.W, g.H, g.W, g.n0x, i, v);
   bb_read_candidate(gt, gt2, gt4, g, b, j, w);
-  const float scale = patch_grad_scale<PER_IMG>(grad_out, b, g.B, g.N, (float)BB_D);
+  const float scale = patch_grad_scale<PER_IMG, MAP>(grad_out, b, g.B, g.N, (float)BB_D, i);
 #pragma unroll
   for (int e = 0; e < BB_D; ++e) {
     const float d = w[e] - v[e];
@@ -997,8 +1002,8 @@ bb_pyramid_adjoint_kernel(const float* __restrict__ d2, const float* __restrict_
 // One thread per patch; every pixel covered by a patch belongs to exactly one, the rest stay 0.
 // TO_GT: the same formula with the roles swapped (v = the selected candidate, differentiated; w = the SR patch), the
 // result accumulated into the candidate's level image (d_sr = level 0 = d_gt, d2, d4).
-// PER_IMG: reduction='none', grad_out is [B] (patch_grad_scale)
-template <bool TO_GT = false, bool PER_IMG = false>
+// PER_IMG: reduction='none', grad_out is [B]; MAP: the loss map, grad_out is [B][N] (patch_grad_scale)
+template <bool TO_GT = false, bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(256)
 gram_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                      const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -1018,7 +1023,7 @@ gram_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt,
   }
   bb_gram(v, g1);
   bb_gram(w, gs);
-  const float scale = patch_grad_scale<PER_IMG>(grad_out, b, g.B, g.N, 9.0f);
+  const float scale = patch_grad_scale<PER_IMG, MAP>(grad_out, b, g.B, g.N, 9.0f, i);
   float dG[9];
 #pragma unroll
   for (int k = 0; k < 9; ++k) {
@@ -1047,8 +1052,9 @@ gram_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt,
 //   dJxx = dDxx/q + ddet*Jyy , dJyy = dDyy/q + ddet*Jxx , dJxy = dDxy/q - 2 ddet*Jxy
 // then the adjoint 3x3 smoothing, the product rule dIx = 2 Ix dPxx + Iy dPxy, dIy = 2 Iy dPyy + Ix dPxy,
 // the adjoint derivative filters and the grayscale weights.  One thread per patch.
-// TO_GT: roles swapped and scatter-add into the candidate's level image, as in gram_backward_kernel; PER_IMG: as there
-template <bool TO_GT = false, bool PER_IMG = false>
+// TO_GT: roles swapped and scatter-add into the candidate's level image, as in gram_backward_kernel; PER_IMG, MAP: as
+// there
+template <bool TO_GT = false, bool PER_IMG = false, bool MAP = false>
 __global__ void __launch_bounds__(128)
 pst_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, const float* __restrict__ gt2,
                     const float* __restrict__ gt4, const int64_t* __restrict__ idx, const float* __restrict__ grad_out,
@@ -1069,7 +1075,7 @@ pst_backward_kernel(const float* __restrict__ sr, const float* __restrict__ gt, 
   pst_descriptor(w, tp, dsel);
   PstState S;
   pst_state(v, tp, S);
-  const float scale = patch_grad_scale<PER_IMG>(grad_out, b, g.B, g.N, (float)BB_D);
+  const float scale = patch_grad_scale<PER_IMG, MAP>(grad_out, b, g.B, g.N, (float)BB_D, i);
   float dJ[3][9];
 #pragma unroll
   for (int p = 0; p < 9; ++p) {

@@ -890,13 +890,15 @@ static int zero_fill(float* p, size_t n, void* stream) {
 #endif
 }
 
-// PI: reduction='none' (srst_patch_forward_per_image): loss_out is [B]
-template <int MODE, bool PI = false>
+// PI: reduction='none' (srst_patch_forward_per_image): loss_out is [B].  MAP (srst_patch_forward_map): loss_out[0] as
+// the scalar entry points, and map_out [B][N] the per-query means
+template <int MODE, bool PI = false, bool MAP = false>
 static int bb_forward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W,
                            float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out, void* workspace,
-                           size_t workspace_bytes, void* stream, const PstTaps& tp = PstTaps{}) {
+                           size_t workspace_bytes, void* stream, const PstTaps& tp = PstTaps{}, float* map_out = nullptr) {
+  static_assert(!(PI && MAP), "one output form");
   constexpr int D = BbDesc<MODE>::D;
-  if (!sr || !gt || !idx_out || !loss_out || B <= 0) return SRST_E_INVALID;
+  if (!sr || !gt || !idx_out || !loss_out || (MAP && !map_out) || B <= 0) return SRST_E_INVALID;
   bool dist_l1;
   int e = bb_check(criterion, dist_l1, B, H, W, gt2, gt4);
   if (e) return e;
@@ -931,8 +933,12 @@ static int bb_forward_impl(const float* sr, const float* gt, const float* gt2, c
     return (int)cudaGetLastError();
   }
   const unsigned nl = (unsigned)(((size_t)B * g.N + BB_NT - 1) / BB_NT);
-  SRST_LAUNCH(bb_loss_kernel<D>, dim3(nl), dim3(BB_NT), 0, stream, w.mats, w.per_image, g, idx_out, criterion,
-              w.partials, w.ticket, loss_out);
+  if constexpr (MAP)
+    SRST_LAUNCH((bb_loss_kernel<D, false, true>), dim3(nl), dim3(BB_NT), 0, stream, w.mats, w.per_image, g, idx_out,
+                criterion, w.partials, w.ticket, loss_out, map_out);
+  else
+    SRST_LAUNCH(bb_loss_kernel<D>, dim3(nl), dim3(BB_NT), 0, stream, w.mats, w.per_image, g, idx_out, criterion,
+                w.partials, w.ticket, loss_out);
   return (int)cudaGetLastError();
 }
 
@@ -969,8 +975,8 @@ static int pst_taps(const float* g, const float* dg, int r_sigma, const float* k
   return 0;
 }
 
-// PI: reduction='none' (srst_patch_backward_per_image): grad_out is [B]
-template <int MODE, bool PI = false>
+// PI: reduction='none' (srst_patch_backward_per_image): grad_out is [B]; MAP (srst_patch_backward_map): [B][N]
+template <int MODE, bool PI = false, bool MAP = false>
 static int patch_backward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
                                const float* grad_out, int B, int H, int W, int criterion, float* d_sr, void* workspace,
                                size_t workspace_bytes, void* stream, const PstTaps& tp = PstTaps{}) {
@@ -987,17 +993,17 @@ static int patch_backward_impl(const float* sr, const float* gt, const float* gt
   }
   if constexpr (MODE == 0) {  // one thread per pixel of d_sr
     const size_t total = (size_t)B * 3 * H * W;
-    SRST_LAUNCH(bb_backward_kernel<PI>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
-                grad_out, g, criterion, d_sr);
+    SRST_LAUNCH((bb_backward_kernel<PI, MAP>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4,
+                idx, grad_out, g, criterion, d_sr);
   } else {  // one thread per patch: pixels outside every patch keep a zero gradient
     if ((H % 3 != 0 || W % 3 != 0) && (e = zero_fill(d_sr, (size_t)B * 3 * H * W, stream)) != 0) return e;
     const size_t total = (size_t)B * g.N;
     if constexpr (MODE == 1)
-      SRST_LAUNCH((gram_backward_kernel<false, PI>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2,
-                  gt4, idx, grad_out, g, criterion, d_sr, nullptr, nullptr);
+      SRST_LAUNCH((gram_backward_kernel<false, PI, MAP>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt,
+                  gt2, gt4, idx, grad_out, g, criterion, d_sr, nullptr, nullptr);
     else
-      SRST_LAUNCH((pst_backward_kernel<false, PI>), dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt, gt2,
-                  gt4, idx, grad_out, g, tp, criterion, d_sr, nullptr, nullptr);
+      SRST_LAUNCH((pst_backward_kernel<false, PI, MAP>), dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt,
+                  gt2, gt4, idx, grad_out, g, tp, criterion, d_sr, nullptr, nullptr);
   }
   return (int)cudaGetLastError();
 }
@@ -1042,8 +1048,9 @@ int srst_pst_backward(const float* sr, const float* gt, const float* gt2, const 
 
 }  // extern "C"
 
-// srst_patch_backward_gt, and the d_gt half of srst_patch_backward_per_image (PI: grad_out is [B])
-template <bool PI>
+// srst_patch_backward_gt, and the d_gt half of srst_patch_backward_per_image (PI: grad_out is [B]) and of
+// srst_patch_backward_map (MAP: grad_out is [B][N])
+template <bool PI, bool MAP = false>
 static int patch_backward_gt_impl(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
                                   const int64_t* idx, const float* grad_out, int B, int H, int W, const float* g,
                                   const float* dg, int r_sigma, const float* k, int r_rho, int criterion, float* d_gt,
@@ -1068,14 +1075,14 @@ static int patch_backward_gt_impl(int mode, const float* sr, const float* gt, co
   SRST_LAUNCH(bb_fill_zero_kernel, dim3(fill_grid((n2 + 3) / 4 * 4 + n4, 148)), dim3(256), 0, stream, d2, (n2 + 3) / 4 * 4 + n4);
   const size_t total = (size_t)B * gm.N;
   if (mode == 0)
-    SRST_LAUNCH(bb_backward_gt_kernel<PI>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
-                grad_out, gm, criterion, d_gt, d2, d4);
-  else if (mode == 1)
-    SRST_LAUNCH((gram_backward_kernel<true, PI>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2,
+    SRST_LAUNCH((bb_backward_gt_kernel<PI, MAP>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2,
                 gt4, idx, grad_out, gm, criterion, d_gt, d2, d4);
+  else if (mode == 1)
+    SRST_LAUNCH((gram_backward_kernel<true, PI, MAP>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt,
+                gt2, gt4, idx, grad_out, gm, criterion, d_gt, d2, d4);
   else
-    SRST_LAUNCH((pst_backward_kernel<true, PI>), dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt, gt2,
-                gt4, idx, grad_out, gm, tp, criterion, d_gt, d2, d4);
+    SRST_LAUNCH((pst_backward_kernel<true, PI, MAP>), dim3((unsigned)((total + 127) / 128)), dim3(128), 0, stream, sr, gt,
+                gt2, gt4, idx, grad_out, gm, tp, criterion, d_gt, d2, d4);
   SRST_LAUNCH(bb_pyramid_adjoint_kernel, dim3((unsigned)((n2 + n4 + 255) / 256)), dim3(256), 0, stream, d2, d4, d_gt, B * 3,
               H, W, gm.H2, gm.W2, gm.H4, gm.W4);
   return (int)cudaGetLastError();
@@ -1091,49 +1098,89 @@ int srst_patch_backward_gt(int mode, const float* sr, const float* gt, const flo
                                        d_gt, workspace, workspace_bytes, stream);
 }
 
-int srst_patch_forward_per_image(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4, int B,
-                                 int H, int W, const float* g, const float* dg, int r_sigma, const float* k, int r_rho,
-                                 float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out,
-                                 void* workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// srst_patch_forward_per_image (PI) and srst_patch_forward_map (MAP): `mode` picks the descriptor
+template <bool PI, bool MAP>
+static int patch_forward_mode(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H,
+                              int W, const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float alpha,
+                              float beta, int criterion, int64_t* idx_out, float* loss_out, float* map_out, void* workspace,
+                              size_t workspace_bytes, void* stream) {
   switch (mode) {
     case 0:
-      return bb_forward_impl<0, true>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
-                                      workspace_bytes, stream);
+      return bb_forward_impl<0, PI, MAP>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
+                                         workspace_bytes, stream, PstTaps{}, map_out);
     case 1:
-      return bb_forward_impl<1, true>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
-                                      workspace_bytes, stream);
+      return bb_forward_impl<1, PI, MAP>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
+                                         workspace_bytes, stream, PstTaps{}, map_out);
     case 2: {
       PstTaps tp;
       const int e = pst_taps(g, dg, r_sigma, k, r_rho, tp);
       if (e) return e;
-      return bb_forward_impl<2, true>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
-                                      workspace_bytes, stream, tp);
+      return bb_forward_impl<2, PI, MAP>(sr, gt, gt2, gt4, B, H, W, alpha, beta, criterion, idx_out, loss_out, workspace,
+                                         workspace_bytes, stream, tp, map_out);
     }
     default: return SRST_E_INVALID;
   }
+}
+
+// srst_patch_backward_per_image (PI) and srst_patch_backward_map (MAP): d_sr and / or d_gt in one call
+template <bool PI, bool MAP>
+static int patch_backward_mode(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                               const int64_t* idx, const float* grad_out, int B, int H, int W, const float* g,
+                               const float* dg, int r_sigma, const float* k, int r_rho, int criterion, float* d_sr,
+                               float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
+  if ((!d_sr && !d_gt) || mode < 0 || mode > 2) return SRST_E_INVALID;
+  int e = 0;
+  if (d_sr) {
+    PstTaps tp;
+    if (mode == 2 && (e = pst_taps(g, dg, r_sigma, k, r_rho, tp)) != 0) return e;
+    if (mode == 0) e = patch_backward_impl<0, PI, MAP>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace,
+                                                       workspace_bytes, stream);
+    else if (mode == 1) e = patch_backward_impl<1, PI, MAP>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr,
+                                                            workspace, workspace_bytes, stream);
+    else e = patch_backward_impl<2, PI, MAP>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace,
+                                             workspace_bytes, stream, tp);
+    if (e) return e;
+  }
+  if (d_gt)
+    e = patch_backward_gt_impl<PI, MAP>(mode, sr, gt, gt2, gt4, idx, grad_out, B, H, W, g, dg, r_sigma, k, r_rho, criterion,
+                                        d_gt, workspace, workspace_bytes, stream);
+  return e;
+}
+
+extern "C" {
+
+int srst_patch_forward_per_image(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4, int B,
+                                 int H, int W, const float* g, const float* dg, int r_sigma, const float* k, int r_rho,
+                                 float alpha, float beta, int criterion, int64_t* idx_out, float* loss_out,
+                                 void* workspace, size_t workspace_bytes, void* stream) {
+  return patch_forward_mode<true, false>(mode, sr, gt, gt2, gt4, B, H, W, g, dg, r_sigma, k, r_rho, alpha, beta, criterion,
+                                         idx_out, loss_out, nullptr, workspace, workspace_bytes, stream);
 }
 
 int srst_patch_backward_per_image(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
                                   const int64_t* idx, const float* grad_out, int B, int H, int W, const float* g,
                                   const float* dg, int r_sigma, const float* k, int r_rho, int criterion, float* d_sr,
                                   float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
-  if ((!d_sr && !d_gt) || mode < 0 || mode > 2) return SRST_E_INVALID;
-  int e = 0;
-  if (d_sr) {
-    PstTaps tp;
-    if (mode == 2 && (e = pst_taps(g, dg, r_sigma, k, r_rho, tp)) != 0) return e;
-    if (mode == 0) e = patch_backward_impl<0, true>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace,
-                                                    workspace_bytes, stream);
-    else if (mode == 1) e = patch_backward_impl<1, true>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace,
-                                                         workspace_bytes, stream);
-    else e = patch_backward_impl<2, true>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, criterion, d_sr, workspace,
-                                          workspace_bytes, stream, tp);
-    if (e) return e;
-  }
-  if (d_gt)
-    e = patch_backward_gt_impl<true>(mode, sr, gt, gt2, gt4, idx, grad_out, B, H, W, g, dg, r_sigma, k, r_rho, criterion,
-                                     d_gt, workspace, workspace_bytes, stream);
-  return e;
+  return patch_backward_mode<true, false>(mode, sr, gt, gt2, gt4, idx, grad_out, B, H, W, g, dg, r_sigma, k, r_rho,
+                                          criterion, d_sr, d_gt, workspace, workspace_bytes, stream);
+}
+
+int srst_patch_forward_map(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H,
+                           int W, const float* g, const float* dg, int r_sigma, const float* k, int r_rho, float alpha,
+                           float beta, int criterion, int64_t* idx_out, float* loss_out, float* map_out, void* workspace,
+                           size_t workspace_bytes, void* stream) {
+  return patch_forward_mode<false, true>(mode, sr, gt, gt2, gt4, B, H, W, g, dg, r_sigma, k, r_rho, alpha, beta, criterion,
+                                         idx_out, loss_out, map_out, workspace, workspace_bytes, stream);
+}
+
+int srst_patch_backward_map(int mode, const float* sr, const float* gt, const float* gt2, const float* gt4,
+                            const int64_t* idx, const float* grad_map, int B, int H, int W, const float* g, const float* dg,
+                            int r_sigma, const float* k, int r_rho, int criterion, float* d_sr, float* d_gt,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+  return patch_backward_mode<false, true>(mode, sr, gt, gt2, gt4, idx, grad_map, B, H, W, g, dg, r_sigma, k, r_rho,
+                                          criterion, d_sr, d_gt, workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"
@@ -1166,12 +1213,14 @@ long long srst_bbg_num_patches(int H, int W, int ksize, int pad, int stride) {
 
 }  // extern "C"
 
-// srst_bbg_forward / srst_bbg_forward_per_image (PI: loss_out is [B])
-template <bool PI>
+// srst_bbg_forward / srst_bbg_forward_per_image (PI: loss_out is [B]) / srst_bbg_forward_map (MAP: map_out [B][N])
+template <bool PI, bool MAP = false>
 static int bbg_forward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W,
                             int ksize, int pad, int stride, float alpha, float beta, int criterion, int64_t* idx_out,
-                            float* loss_out, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!sr || !gt || !idx_out || !loss_out || B <= 0) return SRST_E_INVALID;
+                            float* loss_out, void* workspace, size_t workspace_bytes, void* stream,
+                            float* map_out = nullptr) {
+  static_assert(!(PI && MAP), "one output form");
+  if (!sr || !gt || !idx_out || !loss_out || (MAP && !map_out) || B <= 0) return SRST_E_INVALID;
   bool dist_l1;
   int e = bb_criterion(criterion, dist_l1);
   if (e) return e;
@@ -1198,13 +1247,17 @@ static int bbg_forward_impl(const float* sr, const float* gt, const float* gt2, 
     return (int)cudaGetLastError();
   }
   const unsigned nl = (unsigned)(((size_t)B * g.N + BBG_NT - 1) / BBG_NT);
-  SRST_LAUNCH(bbg_loss_kernel<false>, dim3(nl), dim3(BBG_NT), 0, stream, sr, gt, gt2, gt4, g, idx_out, criterion, w.partials,
-              w.ticket, loss_out);
+  if constexpr (MAP)
+    SRST_LAUNCH((bbg_loss_kernel<false, true>), dim3(nl), dim3(BBG_NT), 0, stream, sr, gt, gt2, gt4, g, idx_out, criterion,
+                w.partials, w.ticket, loss_out, map_out);
+  else
+    SRST_LAUNCH(bbg_loss_kernel<false>, dim3(nl), dim3(BBG_NT), 0, stream, sr, gt, gt2, gt4, g, idx_out, criterion,
+                w.partials, w.ticket, loss_out);
   return (int)cudaGetLastError();
 }
 
-// srst_bbg_backward / srst_bbg_backward_per_image (PI: grad_out is [B])
-template <bool PI>
+// srst_bbg_backward / srst_bbg_backward_per_image (PI: grad_out is [B]) / srst_bbg_backward_map (MAP: [B][N])
+template <bool PI, bool MAP = false>
 static int bbg_backward_impl(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
                              const float* grad_out, int B, int H, int W, int ksize, int pad, int stride, int criterion,
                              float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
@@ -1219,8 +1272,8 @@ static int bbg_backward_impl(const float* sr, const float* gt, const float* gt2,
   if ((e = bbg_prepare(gt, gt2, gt4, B, H, W, g, workspace, workspace_bytes, w, stream)) != 0) return e;
   const size_t n0 = (size_t)B * 3 * H * W;
   if (d_sr) {
-    SRST_LAUNCH(bbg_backward_kernel<PI>, dim3((unsigned)((n0 + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
-                grad_out, g, criterion, d_sr);
+    SRST_LAUNCH((bbg_backward_kernel<PI, MAP>), dim3((unsigned)((n0 + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4,
+                idx, grad_out, g, criterion, d_sr);
     if ((e = (int)cudaGetLastError()) != 0) return e;
   }
   if (d_gt) {
@@ -1228,8 +1281,8 @@ static int bbg_backward_impl(const float* sr, const float* gt, const float* gt2,
     SRST_LAUNCH(bb_fill_zero_kernel, dim3(fill_grid(n0, 592)), dim3(256), 0, stream, d_gt, n0);
     SRST_LAUNCH(bb_fill_zero_kernel, dim3(fill_grid((n2 + 3) / 4 * 4 + n4, 148)), dim3(256), 0, stream, w.d2, (n2 + 3) / 4 * 4 + n4);
     const size_t total = (size_t)B * g.N * 3;
-    SRST_LAUNCH(bbg_backward_gt_kernel<PI>, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2, gt4, idx,
-                grad_out, g, criterion, d_gt, w.d2, w.d4);
+    SRST_LAUNCH((bbg_backward_gt_kernel<PI, MAP>), dim3((unsigned)((total + 255) / 256)), dim3(256), 0, stream, sr, gt, gt2,
+                gt4, idx, grad_out, g, criterion, d_gt, w.d2, w.d4);
     SRST_LAUNCH(bb_pyramid_adjoint_kernel, dim3((unsigned)((n2 + n4 + 255) / 256)), dim3(256), 0, stream, w.d2, w.d4, d_gt,
                 B * 3, H, W, g.L[1].H, g.L[1].W, g.L[2].H, g.L[2].W);
     if ((e = (int)cudaGetLastError()) != 0) return e;
@@ -1265,6 +1318,20 @@ int srst_bbg_backward_per_image(const float* sr, const float* gt, const float* g
                                 float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
   return bbg_backward_impl<true>(sr, gt, gt2, gt4, idx, grad_out, B, H, W, ksize, pad, stride, criterion, d_sr, d_gt,
                                  workspace, workspace_bytes, stream);
+}
+
+int srst_bbg_forward_map(const float* sr, const float* gt, const float* gt2, const float* gt4, int B, int H, int W,
+                         int ksize, int pad, int stride, float alpha, float beta, int criterion, int64_t* idx_out,
+                         float* loss_out, float* map_out, void* workspace, size_t workspace_bytes, void* stream) {
+  return bbg_forward_impl<false, true>(sr, gt, gt2, gt4, B, H, W, ksize, pad, stride, alpha, beta, criterion, idx_out,
+                                       loss_out, workspace, workspace_bytes, stream, map_out);
+}
+
+int srst_bbg_backward_map(const float* sr, const float* gt, const float* gt2, const float* gt4, const int64_t* idx,
+                          const float* grad_map, int B, int H, int W, int ksize, int pad, int stride, int criterion,
+                          float* d_sr, float* d_gt, void* workspace, size_t workspace_bytes, void* stream) {
+  return bbg_backward_impl<false, true>(sr, gt, gt2, gt4, idx, grad_map, B, H, W, ksize, pad, stride, criterion, d_sr, d_gt,
+                                        workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

@@ -492,11 +492,12 @@ class _PatchLossFn(torch.autograd.Function):
     and, through the gather of the selected candidates, w.r.t. gt (reference loss.py:135-139, :219-222, :369-371); the
     argmin is not.  `loss_cls` is the module class: its _plan / _fwd / _bwd make the C ABI calls that differ per loss.
     `args` holds what they take from the module (weights, criterion, taps, geometry), fixed at forward time: a module
-    changed between forward and backward does not change the gradient.  `per_image`: reduction='none' -- the loss and
-    the upstream gradient are [B], and _fwd_none / _bwd_none make the calls."""
+    changed between forward and backward does not change the gradient.  `form` is the output: "mean" (a 0-dim batch
+    mean), "none" (reduction='none': the loss and the upstream gradient are [B], _fwd_none / _bwd_none make the calls)
+    or "map" (loss_map: one value per query patch, [B,N], _fwd_map / _bwd_map)."""
 
     @staticmethod
-    def forward(ctx, sr, gt, loss_cls, args, pyramid, per_image=False):
+    def forward(ctx, sr, gt, loss_cls, args, pyramid, form="mean"):
         sr = sr.contiguous()
         gt = gt.contiguous()
         B, _, H, W = sr.shape
@@ -505,13 +506,19 @@ class _PatchLossFn(torch.autograd.Function):
             stream = _raw_stream(sr.device)
             gt2, gt4 = _hr_pyramid(gt, pyramid)
             idx = torch.empty((B, n), dtype=torch.int64, device=sr.device)
-            loss = torch.empty((B,) if per_image else (), dtype=torch.float32, device=sr.device)
-            fwd = loss_cls._fwd_none if per_image else loss_cls._fwd
-            fwd(args, sr, gt, gt2, gt4, idx, loss, _workspace(kind, sr.device, stream, nbytes), stream)
+            ws = _workspace(kind, sr.device, stream, nbytes)
+            if form == "map":
+                out = torch.empty((B, n), dtype=torch.float32, device=sr.device)
+                loss_cls._fwd_map(args, sr, gt, gt2, gt4, idx, torch.empty((), dtype=torch.float32, device=sr.device),
+                                  out, ws, stream)
+            else:
+                out = torch.empty((B,) if form == "none" else (), dtype=torch.float32, device=sr.device)
+                fwd = loss_cls._fwd_none if form == "none" else loss_cls._fwd
+                fwd(args, sr, gt, gt2, gt4, idx, out, ws, stream)
         ctx.save_for_backward(sr, gt, gt2, gt4, idx)
-        ctx.meta = (loss_cls, args, kind, nbytes, per_image)
+        ctx.meta = (loss_cls, args, kind, nbytes, form)
         ctx.mark_non_differentiable(idx)
-        return loss, idx
+        return out, idx
 
     @staticmethod
     @once_differentiable
@@ -520,13 +527,13 @@ class _PatchLossFn(torch.autograd.Function):
         if not (need_sr or need_gt):
             return None, None, None, None, None, None
         sr, gt, gt2, gt4, idx = ctx.saved_tensors
-        loss_cls, args, kind, nbytes, per_image = ctx.meta
-        grad_out = grad_out.to(torch.float32).contiguous()   # also the stride-0 [B] of .sum() / .mean()
+        loss_cls, args, kind, nbytes, form = ctx.meta
+        grad_out = grad_out.to(torch.float32).contiguous()   # also the stride-0 [B] / [B,N] of .sum() / .mean()
         with _on_device(sr.device):
             stream = _raw_stream(sr.device)
             d_sr = torch.empty_like(sr) if need_sr else None
             d_gt = torch.empty_like(gt) if need_gt else None
-            bwd = loss_cls._bwd_none if per_image else loss_cls._bwd
+            bwd = {"mean": loss_cls._bwd, "none": loss_cls._bwd_none, "map": loss_cls._bwd_map}[form]
             bwd(args, sr, gt, gt2, gt4, idx, grad_out, d_sr, d_gt, _workspace(kind, sr.device, stream, nbytes), stream)
         return d_sr, d_gt, None, None, None, None
 
@@ -535,14 +542,16 @@ class _PatchLoss(nn.Module):
     """What BestBuddyLoss, GramLoss and PatchwiseStructureTensorLoss share: the reference's constructor arguments
     `alpha`, `beta`, `ksize`, `dist_norm`, `criterion`, the `pyramid` and `reduction` choices, the call through
     _PatchLossFn, and ``last_indices``, the argmin indices ``[B,N]`` (int64) of the most recent call.  A subclass supplies
-    the C ABI calls (_args, _fwd, _bwd; _MODE and _taps_of for the per-image entry points) and checks its patch geometry
-    (_check_geometry).
+    the C ABI calls (_args, _fwd, _bwd; _MODE and _taps_of for the per-image and loss-map entry points) and checks its
+    patch geometry (_check_geometry).
 
     ``reduction='none'`` returns ``[B]``: entry b is the mean over image b's criterion terms, i.e. the reference module
-    applied to ``(x[b:b+1], gt[b:b+1])``; the search and ``last_indices`` are the same as with 'mean'."""
+    applied to ``(x[b:b+1], gt[b:b+1])``; the search and ``last_indices`` are the same as with 'mean'.
+
+    ``loss_map(x, gt)`` returns the element-wise form, one value per query patch (see there)."""
 
     _criterion_error = "%s criterion has not been implmented."   # the reference's message (loss.py:113, :178)
-    _MODE = 0   # `mode` of srst_patch_forward_per_image / srst_patch_backward_per_image
+    _MODE = 0   # `mode` of the srst_patch_*_per_image / srst_patch_*_map entry points
 
     def __init__(self, alpha, beta, ksize, dist_norm, criterion, pyramid, pad=0, stride=3, reduction="mean"):
         super().__init__()
@@ -577,11 +586,26 @@ class _PatchLoss(nn.Module):
     def forward(self, x, gt):
         _check_pair(x, gt, type(self).__name__)
         if self.reduction == "none":
-            loss, idx = _PatchLossFn.apply(x, gt, type(self), self._args(), self.pyramid, True)
+            loss, idx = _PatchLossFn.apply(x, gt, type(self), self._args(), self.pyramid, "none")
         else:
             loss, idx = _PatchLossFn.apply(x, gt, type(self), self._args(), self.pyramid)
         self.last_indices = idx
         return loss
+
+    def loss_map(self, x, gt):
+        """The per-patch loss map, an fp32 ``[B, ny, nx]`` tensor on the query patch grid (F.unfold's row-major order;
+        ``ny, nx = H // 3, W // 3`` for the default 3x3 / stride-3 geometry).  Entry ``[b, i, j]`` is the mean over the
+        D criterion terms of query patch (i, j) of image b against its selected candidate: the reference's
+        ``criterion(reduction='none')(p1, sel_p2).mean(-1)`` (loss.py:139, :222, :371) before its mean.  So
+        ``loss_map(x, gt).mean()`` is the 'mean' loss and its per-image means are the 'none' losses, whatever
+        ``self.reduction`` says.  Differentiable w.r.t. x, and w.r.t. gt when gt requires grad, under any ``[B, ny, nx]``
+        upstream gradient: spatial weighting or masking of the loss, heat maps of the patches without a good buddy.
+        The search, its checks and errors and ``last_indices`` are those of ``forward``."""
+        _check_pair(x, gt, type(self).__name__)
+        args = self._args()
+        m, idx = _PatchLossFn.apply(x, gt, type(self), args, self.pyramid, "map")
+        self.last_indices = idx
+        return m.view(x.shape[0], *self._grid(args, x.shape[2], x.shape[3]))
 
     def extra_repr(self) -> str:
         return _reduction_repr(self.reduction)
@@ -608,6 +632,30 @@ class _PatchLoss(nn.Module):
                                                        _ptr(grad_out), B, H, W, *cls._taps_of(args)[:5], args[2], _ptr(d_sr),
                                                        _ptr(d_gt), _ptr(ws), ws.numel(), stream)
         _cabi.check(rc, "srst_patch_backward_per_image")
+
+    @classmethod
+    def _fwd_map(cls, args, sr, gt, gt2, gt4, idx, loss, out, ws, stream):
+        """loss_map forward of the default 3x3 / stride-3 patch grid: out is [B,N], loss the (unused) batch mean."""
+        alpha, beta, crit = args[:3]
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_patch_forward_map(cls._MODE, _ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W,
+                                                *cls._taps_of(args)[:5], alpha, beta, crit, _ptr(idx), _ptr(loss), _ptr(out),
+                                                _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_patch_forward_map")
+
+    @classmethod
+    def _bwd_map(cls, args, sr, gt, gt2, gt4, idx, grad_map, d_sr, d_gt, ws, stream):
+        """loss_map backward: grad_map is [B,N]; one call fills d_sr and d_gt, either of which may be None."""
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_patch_backward_map(cls._MODE, _ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx),
+                                                 _ptr(grad_map), B, H, W, *cls._taps_of(args)[:5], args[2], _ptr(d_sr),
+                                                 _ptr(d_gt), _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_patch_backward_map")
+
+    @classmethod
+    def _grid(cls, args, H, W):
+        """(ny, nx), the query patch grid of the default 3x3 / stride-3 geometry."""
+        return H // 3, W // 3
 
     @classmethod
     def _plan(cls, args, B, H, W):
@@ -668,6 +716,13 @@ class BestBuddyLoss(_PatchLoss):
                              f"ksize={ks}, pad={pad}, stride={st} patch (F.unfold would raise too)")
         return n, "bbg", nbytes
 
+    @classmethod
+    def _grid(cls, args, H, W):
+        if args[3] is None:
+            return super()._grid(args, H, W)
+        ks, pad, st = args[3]
+        return (H + 2 * pad - ks) // st + 1, (W + 2 * pad - ks) // st + 1   # F.unfold
+
     @staticmethod
     def _fwd(args, sr, gt, gt2, gt4, idx, loss, ws, stream):
         alpha, beta, crit, geom = args
@@ -718,6 +773,26 @@ class BestBuddyLoss(_PatchLoss):
         rc = _cabi.lib().srst_bbg_backward_per_image(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_out), B,
                                                      H, W, *geom, crit, _ptr(d_sr), _ptr(d_gt), _ptr(ws), ws.numel(), stream)
         _cabi.check(rc, "srst_bbg_backward_per_image")
+
+    @classmethod
+    def _fwd_map(cls, args, sr, gt, gt2, gt4, idx, loss, out, ws, stream):
+        alpha, beta, crit, geom = args
+        if geom is None:
+            return super()._fwd_map(args, sr, gt, gt2, gt4, idx, loss, out, ws, stream)
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_bbg_forward_map(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), B, H, W, *geom, alpha, beta, crit,
+                                              _ptr(idx), _ptr(loss), _ptr(out), _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_bbg_forward_map")
+
+    @classmethod
+    def _bwd_map(cls, args, sr, gt, gt2, gt4, idx, grad_map, d_sr, d_gt, ws, stream):
+        crit, geom = args[2:]
+        if geom is None:
+            return super()._bwd_map(args, sr, gt, gt2, gt4, idx, grad_map, d_sr, d_gt, ws, stream)
+        B, _, H, W = sr.shape
+        rc = _cabi.lib().srst_bbg_backward_map(_ptr(sr), _ptr(gt), _ptr(gt2), _ptr(gt4), _ptr(idx), _ptr(grad_map), B, H, W,
+                                               *geom, crit, _ptr(d_sr), _ptr(d_gt), _ptr(ws), ws.numel(), stream)
+        _cabi.check(rc, "srst_bbg_backward_map")
 
 
 class GramLoss(_PatchLoss):
