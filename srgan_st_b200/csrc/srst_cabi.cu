@@ -54,9 +54,11 @@ using Fwd2 = StFwdCfg<24, 96, 8, 4, 2, 8, 3, 0>;   // Fwd1 with three CTAs per S
 using March96 = StMarchCfg<96, 2, 8>;
 using March112 = StMarchCfg<112, 2, 8>;
 constexpr int kNumFwdCfg = 5, kFwdMarch96 = 3, kFwdMarch112 = 4;
-//                       TH  TW  RS   NT RG RK MINB CSD PIPE
+//                       TH  TW  RS   NT RG RK MINB CSD PIPE XFULL
 using Bwd0 = StBwdCfg<28, 56, 16, 256, 2, 8, 2, 8, true>;  // large images: persistent CTAs, the next tile's boxes prefetched
-using Bwd1 = StBwdCfg<12, 96, 8, 224, 2, 8, 2, 8, true>;   // full-width strips of 96-wide crops, persistent
+// cfg 1: full-width strips of crops (W <= 96, no x halo); the strip height is picked from the batch (crop_bwd)
+using Bwd1 = StBwdCfg<12, 96, 8, 224, 2, 8, 2, 8, true, true>;     // persistent 12-row strips
+using Bwd1W = StBwdCfg<24, 96, 14, 192, 2, 8, 2, 8, false, true>;  // 24-row strips, one tile per CTA
 constexpr int kNumBwdCfg = 2;
 
 constexpr int kMinFwdTH = 16, kMinFwdTW = 48;  // finest forward work split (workspace sizing): 16-row chunks, 48-wide tiles
@@ -259,10 +261,11 @@ static int launch_st_march(const StFwdParamsT<C::RG, C::RK, MAP>& F, void* strea
 
 template <class C, bool PX = false, bool PI = false>
 static int launch_st_backward(StBwdParams<C::RG, C::RK>& P, void* stream) {
+  if (C::XFULL && P.W > C::TW) return SRST_E_SHAPE;  // the tile layout assumes one tile in x
   static const bool tma_env = env_int_once("SRST_ST_BWD_TMA", 1) != 0;
   const int Hp = (P.H + 1) / 2;
   P.use_tma = (tma_env && P.vec4 && aligned16(P.ixy) &&
-               make_plane_map(&P.ds_map, P.ds, (long long)P.B * 3, P.H, P.W, C::VW, C::SH, 3) &&
+               make_plane_map(&P.ds_map, P.ds, (long long)P.B * 3, P.H, P.W, C::SW, C::SH, 3) &&
                make_plane_map(&P.ixy_map, P.ixy, (long long)P.B * 2, Hp, 2 * P.W, C::PI, C::EH / 2, 2)) ? 1 : 0;
   P.tiles_x = (P.W + C::TW - 1) / C::TW;
   P.tiles_y = (P.H + C::TH - 1) / C::TH;
@@ -302,7 +305,8 @@ static int pick_march_cfg(int W) {
 static int pick_bwd_cfg(int B, int H, int W) {
   const int forced = forced_bwd();
   if (forced >= 0 && forced < kNumBwdCfg) return forced;
-  // measured on B200 (profiles/r02_tile_sweep.log): full-width 12x96 strips on 96-wide crops, the 28x56 tile on large images
+  // measured on B200 (profiles/r02_tile_sweep.log, r07_bwd_crop_sweep.log): full-width strips on 96-wide crops, the 28x56
+  // tile on large images
   (void)B; (void)H;
   return W <= 96 ? 1 : 0;
 }
@@ -471,6 +475,17 @@ static int st_forward_rr(const StCall& c) {
   }
 }
 
+// Crop-width backward (cfg 1, W <= 96).  12-row strips while they fit one round of the resident CTAs (16 x 96 rows:
+// 128 strips on 296 slots); beyond that the 24-row strips, whose taller tiles stage and filter fewer halo rows per
+// output row: one round instead of two at 64 x 96 rows, and less work per row at 1024 (measured on B200:
+// profiles/r07_bwd_crop_sweep.log).
+template <bool PX>
+static int crop_bwd(StBwdParams<2, 8>& P, const StCall& c) {
+  const long long slots = (long long)sm_count() * Bwd1::MINB;
+  if ((long long)c.B * ((c.H + Bwd1::TH - 1) / Bwd1::TH) <= slots) return tiled_bwd<Bwd1, PX>(P, c);
+  return tiled_bwd<Bwd1W, PX>(P, c);
+}
+
 template <int RG, int RK>
 static int st_backward_rr(const StCall& c) {
   static thread_local StBwdParams<RG, RK> P;
@@ -483,11 +498,11 @@ static int st_backward_rr(const StCall& c) {
   P.taps = cached_taps<RG, RK>(c.g, c.dg, c.rs, c.k, c.rk);
   if constexpr (RG == 2 && RK == 8) {
     if (c.px_other) {  // the fused Pixel term is compiled into the two default tile shapes
-      if (c.W <= 96) return tiled_bwd<Bwd1, true>(P, c);
+      if (c.W <= Bwd1::TW) return crop_bwd<true>(P, c);
       return tiled_bwd<Bwd0, true>(P, c);
     }
-    if (pick_bwd_cfg(c.B, c.H, c.W) == 1) return tiled_bwd<Bwd1, false>(P, c);
-    return tiled_bwd<Bwd0, false>(P, c);
+    if (c.W <= Bwd1::TW && pick_bwd_cfg(c.B, c.H, c.W) == 1) return crop_bwd<false>(P, c);
+    return tiled_bwd<Bwd0, false>(P, c);  // cfg 1 forced on an image wider than its strips runs cfg 0
   } else {
     using G = StBwdCfg<24, 64, (24 + 2 * RG) / 2, 256, RG, RK, (RK <= 8 ? 2 : 1), 4>;
     return c.px_other ? tiled_bwd<G, true>(P, c) : tiled_bwd<G, false>(P, c);

@@ -974,7 +974,7 @@ st_features_kernel(const __grid_constant__ StFeatParams<C::RG, C::RK> P) {
 // ------------------------------------------------------------------------------------------------
 // Backward
 // ------------------------------------------------------------------------------------------------
-template <int TH_, int TW_, int RS_, int NT_, int RG_, int RK_, int MINB_, int CSD_ = 8, bool PIPE_ = false>
+template <int TH_, int TW_, int RS_, int NT_, int RG_, int RK_, int MINB_, int CSD_ = 8, bool PIPE_ = false, bool XFULL_ = false>
 struct StBwdCfg {
   static constexpr int TH = TH_, TW = TW_, RS = RS_, NT = NT_, RG = RG_, RK = RK_, MINB = MINB_;
   // PIPE: persistent CTAs that loop over tiles and fetch the NEXT tile's ds box as soon as the vertical pass has
@@ -982,25 +982,35 @@ struct StBwdCfg {
   // of the warp time when every CTA waits for its own tile first -- hides behind the rest of the current tile.
   // dIx|dIy then need their own region instead of re-using the ds staging.
   static constexpr bool PIPE = PIPE_;
+  // XFULL: for images no wider than the tile (W <= TW, one tile in x, x0 == 0).  Every x-halo column is then outside
+  // the image, where ds, Ix and Iy -- and so E, dIx and dIy -- are zero: only the TW image columns of ds and Ix, Iy
+  // are staged, the vertical pass and the product rule run on them alone, and the zero columns the horizontal window
+  // (RK each side of V) and the adjoint derivative filter (RG each side of dIx|dIy) read are written by the kernel.
+  static constexpr bool XFULL = XFULL_;
   static constexpr int CSD = CSD_;  // output columns per phase-D' item: 8 reads a 24-column window per 8 outputs
                                     // (3x shared-memory amplification) instead of 20 per 4 (5x)
   static constexpr int HXE = round_up4(RG);  // x halo of the E region (where dIx, dIy are needed)
   static constexpr int HXK = round_up4(RK);
   static constexpr int EH = TH + 2 * RG, EW = TW + 2 * HXE, PE = smem_pitch(2 * EW);
-  static constexpr int VW = EW + 2 * HXK, PV = smem_pitch(2 * VW);  // vertical-pass output
+  static constexpr int VW = (XFULL ? TW : EW) + 2 * HXK, PV = smem_pitch(2 * VW);  // vertical-pass output
   static constexpr int SH = EH + 2 * RK;                            // staged ds rows
   static constexpr int NSEG = EH / RS;
-  // saved Ix, Iy tile: TMA box of EH/2 row pairs x EWB columns (x 2 floats); EWB = EW + 2 makes the
+  // x extent of the product rule (E columns EC0..EC0+ECW-1, the rest of the E region is zero), of the staged ds box
+  // (SW columns from tile column -SX, landing at V column SX0) and of the saved Ix, Iy box (from tile column -IX)
+  static constexpr int EC0 = XFULL ? HXE : 0, ECW = XFULL ? TW : EW;
+  static constexpr int SW = XFULL ? TW : VW, SX = XFULL ? 0 : HXE + HXK, SX0 = XFULL ? HXK : 0, IX = XFULL ? 0 : HXE;
+  static constexpr int VE = XFULL ? HXE : 0;  // V column of E column e's window start: e - VE
+  // saved Ix, Iy tile: TMA box of EH/2 row pairs x EWB columns (x 2 floats); EWB = ECW + 2 makes the
   // pitch 2*EWB == 4 mod 8 floats (conflict-free LDS.128 across row pairs) and a multiple of 16 bytes
-  static constexpr int EWB = EW + 2, PI = 2 * EWB;
+  static constexpr int EWB = ECW + 2, PI = 2 * EWB;
   static constexpr int BW_LO = (HXE - RG) / 2 * 2, BW_HI = (HXE + 4 + RG + 1) / 2 * 2, BWIN = BW_HI - BW_LO;
   static constexpr int DW_LO = (HXK - RK) / 2 * 2, DW_HI = (HXK + CSD + RK + 1) / 2 * 2, DWIN = DW_HI - DW_LO;
-  using MapD = ItemMap<EH / 2, EW / CSD, CSD>;  // horizontal pass + product rule
-  using MapE = ItemMap<TH / 2, TW / 4, 4>;      // adjoint derivative filters + stores
-  // smem: X: staged ds planes [3][SH][VW] row-major (TMA destination), later dIx|dIy (the staging is
+  using MapD = ItemMap<EH / 2, ECW / CSD, CSD>;  // horizontal pass + product rule
+  using MapE = ItemMap<TH / 2, TW / 4, 4>;       // adjoint derivative filters + stores
+  // smem: X: staged ds planes [3][SH][SW] row-major (TMA destination), later dIx|dIy (the staging is
   // dead once the vertical pass has consumed it) | I: saved Ix, Iy [2][EH/2][PI] (TMA destination) | V (3 planes)
   static constexpr int V_FLOATS = (EH / 2) * PV, I_FLOATS = (EH / 2) * PI, DI_FLOATS = (EH / 2) * PE;
-  static constexpr int S_FLOATS = SH * VW;
+  static constexpr int S_FLOATS = SH * SW;
   static constexpr int X_FLOATS = PIPE ? 3 * S_FLOATS : cmax(2 * DI_FLOATS, 3 * S_FLOATS);
   static constexpr int I_OFF = (X_FLOATS + 31) / 32 * 32;               // 128-byte aligned (TMA destination)
   static constexpr int V_OFF = (I_OFF + 2 * I_FLOATS + 31) / 32 * 32;
@@ -1011,7 +1021,9 @@ struct StBwdCfg {
   static_assert(EH % RS == 0 && RS % 2 == 0 && TH % 2 == 0 && TW % 4 == 0 && RG % 2 == 0 && RK % 2 == 0,
                 "bad backward tile");
   static_assert(NT % 32 == 0 && NT <= 1024, "bad backward block size");
-  static_assert((CSD == 4 || CSD == 8) && EW % CSD == 0, "bad phase-D' item width");
+  static_assert((CSD == 4 || CSD == 8) && ECW % CSD == 0, "bad phase-D' item width");
+  // MINB CTAs per SM: 228 KB of shared memory per SM on sm_100, 1 KB of it reserved per CTA
+  static_assert(MINB * (SMEM_BYTES + 1024) <= 228 * 1024, "shared memory does not allow MINB CTAs per SM");
 };
 
 // PER_IMG: reduction='none' -- grad_out (and with PX grad_px) is [B] and the tile of image b scales by grad_out[b] / (H W)
@@ -1020,7 +1032,7 @@ template <class C, bool PX = false, bool PER_IMG = false>
 __global__ void __launch_bounds__(C::NT, C::MINB)
 st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
   SRST_DYN_SMEM(float, smem);
-  float* sS = smem;                     // staged ds [3][SH][VW]
+  float* sS = smem;                     // staged ds [3][SH][SW]
   float* sdI0 = smem + C::DI_OFF;       // dIx [EH/2][PE]: over the (dead) staging, or its own region when pipelined
   float* sdI1 = sdI0 + C::DI_FLOATS;    // dIy
   float* sI0 = smem + C::I_OFF;         // saved Ix [EH/2][PI]
@@ -1041,13 +1053,13 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
     const int tx_ = t % P.tiles_x, r_ = t / P.tiles_x;
     const int ty_ = r_ % P.tiles_y, b_ = r_ / P.tiles_y;
     tma_expect(&s_mbar, pipe ? kBytesS : kBytesS + kBytesI);
-    tma_load_3d(&s_mbar, sS, &P.ds_map, tx_ * C::TW - C::HXE - C::HXK, ty_ * C::TH - C::RG - C::RK, b_ * 3, C::VW, C::SH, 3);
+    tma_load_3d(&s_mbar, sS, &P.ds_map, tx_ * C::TW - C::SX, ty_ * C::TH - C::RG - C::RK, b_ * 3, C::SW, C::SH, 3);
   };
   auto issue_i = [&](int t) {
     const int tx_ = t % P.tiles_x, r_ = t / P.tiles_x;
     const int ty_ = r_ % P.tiles_y, b_ = r_ / P.tiles_y;
     if (pipe) tma_expect(&s_mbar_i, kBytesI);
-    tma_load_3d(pipe ? &s_mbar_i : &s_mbar, sI0, &P.ixy_map, 2 * (tx_ * C::TW - C::HXE), (ty_ * C::TH - C::RG) / 2, b_ * 2,
+    tma_load_3d(pipe ? &s_mbar_i : &s_mbar, sI0, &P.ixy_map, 2 * (tx_ * C::TW - C::IX), (ty_ * C::TH - C::RG) / 2, b_ * 2,
                 C::PI, C::EH / 2, 2);
   };
 
@@ -1067,9 +1079,10 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
   const int b = trow / P.tiles_y;
   const int y0 = ty * C::TH, x0 = tx * C::TW;
   const size_t img_off = (size_t)b * 3 * plane;
-  const int xv0 = x0 - C::HXE - C::HXK;  // first staged / V column
-  const int yv0 = y0 - C::RG - C::RK;    // first staged row
-  const int xe0 = x0 - C::HXE;           // first E-region column
+  const int xv0 = x0 - C::HXE - C::HXK + C::VE;  // first V column
+  const int xs0 = x0 - C::SX;                     // first staged column (V column SX0)
+  const int yv0 = y0 - C::RG - C::RK;             // first staged row
+  const int xi0 = x0 - C::IX;                     // first staged Ix, Iy column (E column EC0)
   const int qe0 = (y0 - C::RG) / 2;      // first E-region row pair (y0 - RG is even; may be -RG/2)
 
   // Stage the three ds planes (+halo) and the saved Ix, Iy tile.  Preferred path: two TMA box copies
@@ -1079,17 +1092,17 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
     tma_wait(&s_mbar, parity);
   } else {
     const float* dsb = P.ds + img_off;
-    for (int it = tid; it < 3 * C::SH * C::VW; it += C::NT) {
-      const int vx = it % C::VW, rc = it / C::VW;
+    for (int it = tid; it < 3 * C::SH * C::SW; it += C::NT) {
+      const int sx = it % C::SW, rc = it / C::SW;
       const int r = rc % C::SH, c = rc / C::SH;
-      const int gy = yv0 + r, gx = xv0 + vx;
+      const int gy = yv0 + r, gx = xs0 + sx;
       sS[it] = (gy >= 0 && gy < H && gx >= 0 && gx < W) ? __ldg(dsb + c * plane + (size_t)gy * W + gx) : 0.f;
     }
     const int Hp = (H + 1) >> 1;
     for (int it = tid; it < 2 * (C::EH / 2) * C::PI; it += C::NT) {
       const int e = it % C::PI, rc = it / C::PI;
       const int qq = rc % (C::EH / 2), pl = rc / (C::EH / 2);
-      const int gp = qe0 + qq, gx = xe0 + (e >> 1);
+      const int gp = qe0 + qq, gx = xi0 + (e >> 1);
       sI0[it] = (gp >= 0 && gp < Hp && gx >= 0 && gx < W) ? __ldg(P.ixy + ixy_offset(b, pl, Hp, W, gp, gx) + (e & 1)) : 0.f;
     }
     __syncthreads();
@@ -1098,7 +1111,7 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
   // Phase C': vertical rho-pass of the three staged ds planes; a lane owns one column and RS rows.
   // The adjoint of the zero-padded symmetric smoothing is the same zero-padded smoothing.
   {
-    const int c_lo = max(0, -xv0), c_hi = min(C::VW, W - xv0);
+    const int c_lo = max(0, -xv0), c_hi = min(C::SX0 + C::SW, W - xv0);
     const int ncol = c_hi - c_lo;
     const int nclr = C::VW - ncol;
     for (int it = tid; it < nclr * (C::EH / 2); it += C::NT) {
@@ -1115,10 +1128,10 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
       float2 acc[C::RS / 2];
 #pragma unroll
       for (int j = 0; j < C::RS / 2; ++j) acc[j] = make_float2(0.f, 0.f);
-      const float* p = sS + (c * C::SH + seg * C::RS) * C::VW + vx;
+      const float* p = sS + (c * C::SH + seg * C::RS) * C::SW + vx - C::SX0;
 #pragma unroll
       for (int r = 0; r < C::RS + 2 * C::RK; ++r) {
-        const float v = p[r * C::VW];
+        const float v = p[r * C::SW];
 #pragma unroll
         for (int jp = 0; jp < C::RS / 2; ++jp) {
           const int u = r - 2 * jp;
@@ -1138,20 +1151,29 @@ st_backward_kernel(const __grid_constant__ StBwdParams<C::RG, C::RK> P) {
 
   // Phase D': horizontal rho-pass -> E = K*ds at the E-region pixels, then the product rule
   //   dIx = 2 Ix Exx + Iy Exy ,  dIy = 2 Iy Eyy + Ix Exy      (adjoint of utils.py:225-229)
+  if constexpr (C::XFULL) {  // the E columns outside the image: dIx = dIy = 0
+    constexpr int NZ = C::EW - C::ECW;
+    for (int it = tid; it < 2 * NZ * (C::EH / 2); it += C::NT) {
+      const int pl = it / (NZ * (C::EH / 2)), r = it - pl * (NZ * (C::EH / 2));
+      const int q = r / NZ, u = r - q * NZ;
+      const int e = u < C::EC0 ? u : C::ECW + u;
+      st2((pl ? sdI1 : sdI0) + q * C::PE + 2 * e, make_float2(0.f, 0.f));
+    }
+  }
   for (int it = tid; it < C::MapD::SLOTS; it += C::NT) {
     int q, seg;
     if (!C::MapD::decode(it, q, seg)) continue;
-    const int ex0 = C::CSD * seg;
+    const int ex0 = C::EC0 + C::CSD * seg, ix0 = C::CSD * seg;
     float2 E[3][C::CSD];
 #pragma unroll
     for (int c = 0; c < 3; ++c)
       smooth_h_rowpair_n<C::RK, C::CSD, C::DWIN, C::HXK - C::DW_LO>(
-          sV + c * C::V_FLOATS + q * C::PV + 2 * (ex0 + C::DW_LO), tp, E[c]);
+          sV + c * C::V_FLOATS + q * C::PV + 2 * (ex0 - C::VE + C::DW_LO), tp, E[c]);
     float* o0 = sdI0 + q * C::PE + 2 * ex0;
     float* o1 = sdI1 + q * C::PE + 2 * ex0;
 #pragma unroll
     for (int m = 0; m < C::CSD / 2; ++m) {  // two columns per LDS.128 / STS.128
-      const float4 ixv = ld4(sI0 + q * C::PI + 2 * ex0 + 4 * m), iyv = ld4(sI1 + q * C::PI + 2 * ex0 + 4 * m);
+      const float4 ixv = ld4(sI0 + q * C::PI + 2 * ix0 + 4 * m), iyv = ld4(sI1 + q * C::PI + 2 * ix0 + 4 * m);
       const float2 ix[2] = {make_float2(ixv.x, ixv.y), make_float2(ixv.z, ixv.w)};
       const float2 iy[2] = {make_float2(iyv.x, iyv.y), make_float2(iyv.z, iyv.w)};
       float2 dx[2], dy[2];
