@@ -50,8 +50,10 @@ using Fwd0 = StFwdCfg<32, 64, 16, 4, 2, 8, 3, 0, true>;  // large images, 256 th
 using Fwd1 = StFwdCfg<24, 96, 8, 4, 2, 8, 2, 0>;   // full-width strip of a 96-wide crop (no horizontal halo), 288 threads, unrolled
 using Fwd2 = StFwdCfg<24, 96, 8, 4, 2, 8, 3, 0>;   // Fwd1 with three CTAs per SM (72 registers): multi-wave batches of 96-wide crops
 // cfg 3, 4: the row-marching kernel (st_march.cuh), 96- and 112-column strips -- the default whenever TMA can
-// fetch the images; the tiled shapes above remain for unaligned tensors and as the fall-back
+// fetch the images; the tiled shapes above remain for unaligned tensors and as the fall-back.  Cfg 3 runs the crop
+// layout (March96X: no x halo) on images no wider than 96 columns.
 using March96 = StMarchCfg<96, 2, 8>;
+using March96X = StMarchCfg<96, 2, 8, 8, true>;
 using March112 = StMarchCfg<112, 2, 8>;
 constexpr int kNumFwdCfg = 5, kFwdMarch96 = 3, kFwdMarch112 = 4;
 //                       TH  TW  RS   NT RG RK MINB CSD PIPE XFULL
@@ -228,8 +230,9 @@ static int launch_st_march(const StFwdParamsT<C::RG, C::RK, MAP>& F, void* strea
   static thread_local StMarchParamsT<C::RG, C::RK, MAP> MP_tls;
   auto& MP = MP_tls;  // a plain reference: the emulation's kernel threads must see THIS thread's instance
   if (!F.vec4) return kMarchUnusable;
-  if (!make_plane_map(&MP.sr_map, F.sr, (long long)F.B * 3, F.H, F.W, C::GW, C::RS, 3) ||
-      !make_plane_map(&MP.hr_map, F.hr, (long long)F.B * 3, F.H, F.W, C::GW, C::RS, 3))
+  if (C::XFULL && F.W > C::TW) return SRST_E_SHAPE;  // the crop layout has one strip, at x = 0
+  if (!make_plane_map(&MP.sr_map, F.sr, (long long)F.B * 3, F.H, F.W, C::BW, C::RS, 3) ||
+      !make_plane_map(&MP.hr_map, F.hr, (long long)F.B * 3, F.H, F.W, C::BW, C::RS, 3))
     return kMarchUnusable;
   MP.F = F;
   if constexpr (MAP) MP.map_out = F.map_out;
@@ -454,7 +457,9 @@ static int st_forward_rr(const StCall& c) {
     const int mcfg = pick_march_cfg(c.W);
     if (mcfg >= 0) {
       int e;
-      if (mcfg == kFwdMarch96) e = c.px ? march_fwd<March96, true>(P, c) : march_fwd<March96, false>(P, c);
+      if (mcfg == kFwdMarch96 && c.W <= March96X::TW)
+        e = c.px ? march_fwd<March96X, true>(P, c) : march_fwd<March96X, false>(P, c);
+      else if (mcfg == kFwdMarch96) e = c.px ? march_fwd<March96, true>(P, c) : march_fwd<March96, false>(P, c);
       else e = c.px ? march_fwd<March112, true>(P, c) : march_fwd<March112, false>(P, c);
       if (e != kMarchUnusable) return e;
     }

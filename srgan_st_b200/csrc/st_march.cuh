@@ -53,7 +53,7 @@ SRST_DEV void march_stamp(bool who, int slot) {
 
 template <int RG, int RK>
 struct StMarchParams {
-  SrstTmap sr_map;  // sr viewed as [B*3][H][W]; box [3][16][GW]
+  SrstTmap sr_map;  // sr viewed as [B*3][H][W]; box [3][16][BW]
   SrstTmap hr_map;
   StFwdParams<RG, RK> F;
   int nstrips, nchunks, chunk_blocks;  // grid = B * nchunks * nstrips; a chunk = chunk_blocks * 16 rows
@@ -66,14 +66,25 @@ struct StMarchMapParams : StMarchParams<RG, RK> {
 template <int RG, int RK, bool MAP>
 using StMarchParamsT = std::conditional_t<MAP, StMarchMapParams<RG, RK>, StMarchParams<RG, RK>>;
 
-template <int TW_, int RG_, int RK_, int CR_ = 8>
+// XFULL: crop layout, for images no wider than the strip (W <= TW, so x0 == 0).  Every x-halo column is outside
+// the image, so its gray values and gradients are zeros: the raw box and the gray conversion cover the TW image
+// columns only, the gradient items the NSEGH image segments only, and the zero columns that the edge windows read
+// (gray: GXH per side, Ix / Iy: RK per side) are written once per CTA.  The gradient and horizontal items are
+// mapped so that a warp holds 4 consecutive row pairs (xitem): a warp whose rows are all outside the image skips
+// the arithmetic of both passes.
+template <int TW_, int RG_, int RK_, int CR_ = 8, bool XFULL_ = false>
 struct StMarchCfg {
+  static constexpr bool XFULL = XFULL_;
   static constexpr int TW = TW_, RG = RG_, RK = RK_;
   static constexpr int CR = CR_, CQ = CR_ / 2;       // rows / row pairs of a block that one consumer thread owns (8 or 4 rows)
   static constexpr int RS = 16, NQ = 8;             // rows / row pairs per block
-  static constexpr int GXH = round_up4(RK + RG);    // x halo of the gray rows; a multiple of 4: TMA wants the first box column 16-byte aligned
-  static constexpr int GOFF = GXH - RK - RG;        // gray columns left of the first gradient window
-  static constexpr int GW = TW + 2 * GXH;           // width of the raw box and of the gray rows
+  // x halo of the gray rows; a multiple of 4: TMA wants the first box column 16-byte aligned, and the crop
+  // layout's gray rows start 16-byte aligned too (its halo is the RG zero columns of the edge windows)
+  static constexpr int GXH = XFULL ? round_up4(RG) : round_up4(RK + RG);
+  static constexpr int GOFF = GXH - RK - RG;        // gray columns left of the window of gradient segment 0 (x0 - RK ..)
+  static constexpr int GW = TW + 2 * GXH;           // width of the gray rows
+  static constexpr int BX = XFULL ? 0 : -GXH;       // first raw box column relative to x0
+  static constexpr int BW = XFULL ? TW : GW;        // width of the raw box
   static constexpr int GP = NQ + RG;                // gray row pairs held: RG carried from the previous block + 8 new
   static constexpr int PG = smem_pitch(2 * GW);
   static constexpr int DW = TW + 2 * RK, PD = smem_pitch(2 * DW);  // Ix, Iy rows (x halo RK)
@@ -83,10 +94,10 @@ struct StMarchCfg {
   static constexpr int HWIN = 8 + 2 * RK;           // Ix, Iy window of a horizontal item
   static constexpr int NIN = RK + CQ;               // ring row pairs a consumer reads for its CQ output row pairs
   static constexpr int NP = 2 * NQ * NSEGB;         // producers: one gradient item each (2 images x 8 row pairs x segments)
-  static constexpr int NH = 2 * NQ * NSEGH;         // horizontal items (the first NH producers)
+  static constexpr int NH = 2 * NQ * NSEGH;         // horizontal items (the first NH producers; XFULL: gradient items too)
   static constexpr int NC = (RS / CR) * TW;         // consumers: column x row part of the block
   static constexpr int NT = NP + NC;
-  static constexpr int RAW_IMG = 3 * RS * GW;       // one TMA box
+  static constexpr int RAW_IMG = 3 * RS * BW;       // one TMA box
   static constexpr int GRAY_IMG = GP * PG, D_PLANE = NQ * PD, H_PLANE = 2 * NQ * PH;
   static constexpr int GRAY_OFF = (2 * RAW_IMG + 31) / 32 * 32;
   static constexpr int D_OFF = GRAY_OFF + 4 * GRAY_IMG;   // two gray buffers (block parity) x two images
@@ -97,8 +108,46 @@ struct StMarchCfg {
   static_assert(CR == 8 || CR == 4, "march: consumer rows");
   static_assert(RG % 2 == 0 && RK == 8, "march: radii (two ring blocks cover 16 + 2 RK rows; 8-column items aligned to the strip)");
   static_assert(TW % 16 == 0 && NP % 32 == 0 && NC % 32 == 0 && NT <= 1024, "march: strip width");
-  static_assert(GW % 4 == 0 && GW <= 256 && (RAW_IMG * 4) % 128 == 0 && GOFF % 2 == 0, "march: TMA box");
+  static_assert(BW % 4 == 0 && BW <= 256 && (RAW_IMG * 4) % 128 == 0 && GOFF % 2 == 0, "march: TMA box");
   static_assert(NH <= NP && NP - NH == 32 && TW / 2 <= 64, "march: horizontal items; one copy warp, two float4 per lane and row pair");
+
+  // Crop layout item map: item i < NH -> row pair q, image, image segment seg (columns 8 seg ..).  A warp holds row
+  // pairs 4h .. 4h+3 (h = warp / XWH) of 8 consecutive (image, segment) pairs; a quarter-warp holds those 4 row
+  // pairs of 2 adjacent segments of one image.
+  static constexpr int XWH = NH / 64;  // warps per half block
+  __host__ __device__ static constexpr void xitem(int i, int& q, int& img, int& seg) {
+    const int w = i >> 5, l = i & 31;
+    q = 4 * (w / XWH) + (l & 3);
+    const int c = 8 * (w % XWH) + 2 * (l >> 3) + ((l >> 2) & 1);
+    img = c / NSEGH;
+    seg = c % NSEGH;
+  }
+  // 16-byte bank group of every LDS.128 / STS.128 address of the crop items (the window steps move all lanes of a
+  // quarter-warp alike): gray window (gradient), Ix / Iy row (gradient store, horizontal window), ring row (store).
+  // A quarter-warp is one shared-memory wavefront when its 8 lanes hit 8 distinct groups.
+  __host__ __device__ static constexpr bool xitem_conflict_free() {
+    for (int g = 0; g < NH / 8; ++g)
+      for (int a = 0; a < 2 * 4; ++a) {  // address kind x ring / gray parity
+        unsigned seen = 0;
+        for (int l = 0; l < 8; ++l) {
+          int q = 0, img = 0, seg = 0;
+          xitem(8 * g + l, q, img, seg);
+          const int par = a & 1;
+          int off = 0;
+          switch (a >> 1) {
+            case 0: off = (par * 2 + img) * GRAY_IMG + q * PG + 2 * (8 * (seg + RK / 8) + GOFF); break;
+            case 1: off = img * 2 * D_PLANE + q * PD + 2 * (8 * (seg + RK / 8)); break;
+            case 2: off = img * 2 * D_PLANE + q * PD + 2 * (8 * seg); break;
+            default: off = img * 3 * H_PLANE + (8 * par + q) * PH + 2 * (8 * seg); break;
+          }
+          if (off % 4 != 0) return false;
+          seen |= 1u << ((off / 4) % 8);
+        }
+        if (seen != 0xffu) return false;
+      }
+    return true;
+  }
+  static_assert(!XFULL || (NQ == 8 && NSEGH % 4 == 0 && GXH >= RG), "march crop layout: 4 row pairs x 8 items per warp");
 };
 
 // The per-pixel chain on RAW tensors: same mathematics as st_pixel2 with the normalisation folded in.  With
@@ -191,6 +240,7 @@ template <class C, bool PX = false, bool WANT_HR = false, bool PER_IMG = false, 
 __global__ void __launch_bounds__(C::NT, C::MINB)
 st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP> MP) {
   static_assert(!(MAP && (PX || PER_IMG)), "the distance map comes with the batch loss only");
+  static_assert(!C::XFULL || C::xitem_conflict_free(), "march crop layout: a quarter-warp's 16-byte accesses share a bank group");
   SRST_DYN_SMEM(float, smem);
   __shared__ float s_red[32];
   __shared__ unsigned int s_last;
@@ -233,21 +283,21 @@ st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP
   // loaded directly while the first box is in flight)
   auto issue_raw = [&](int k) {
     tma_expect(&s_mbar, (unsigned)(2 * C::RAW_IMG * sizeof(float)));
-    tma_load_3d(&s_mbar, sRaw, &MP.sr_map, x0 - C::GXH, hb(k) + RG, b * 3, C::GW, C::RS, 3);
-    tma_load_3d(&s_mbar, sRaw + C::RAW_IMG, &MP.hr_map, x0 - C::GXH, hb(k) + RG, b * 3, C::GW, C::RS, 3);
+    tma_load_3d(&s_mbar, sRaw, &MP.sr_map, x0 + C::BX, hb(k) + RG, b * 3, C::BW, C::RS, 3);
+    tma_load_3d(&s_mbar, sRaw + C::RAW_IMG, &MP.hr_map, x0 + C::BX, hb(k) + RG, b * 3, C::BW, C::RS, 3);
   };
   [[maybe_unused]] float pxsum = 0.f;
   // raw box of block k -> gray row pairs RG .. RG+7 of gray buffer k&1; item = image x row pair x 4 columns
   auto convert = [&](int k) {
-    constexpr int C4 = C::GW / 4;
+    constexpr int C4 = C::BW / 4;
     float* gbuf = sGray + (k & 1) * 2 * C::GRAY_IMG;
     for (int it = tid; it < 2 * NQ * C4; it += C::NP) {
       const int c4 = it % C4, rr = it / C4;
       const int q = rr % NQ, img = rr / NQ;
-      const float* r0 = sRaw + img * C::RAW_IMG + (2 * q) * C::GW + 4 * c4;
-      const float4 R0 = ld4(r0), G0 = ld4(r0 + C::RS * C::GW), B0 = ld4(r0 + 2 * C::RS * C::GW);
-      const float4 R1 = ld4(r0 + C::GW), G1 = ld4(r0 + C::GW + C::RS * C::GW), B1 = ld4(r0 + C::GW + 2 * C::RS * C::GW);
-      float* o = gbuf + img * C::GRAY_IMG + (RG + q) * C::PG + 8 * c4;
+      const float* r0 = sRaw + img * C::RAW_IMG + (2 * q) * C::BW + 4 * c4;
+      const float4 R0 = ld4(r0), G0 = ld4(r0 + C::RS * C::BW), B0 = ld4(r0 + 2 * C::RS * C::BW);
+      const float4 R1 = ld4(r0 + C::BW), G1 = ld4(r0 + C::BW + C::RS * C::BW), B1 = ld4(r0 + C::BW + 2 * C::RS * C::BW);
+      float* o = gbuf + img * C::GRAY_IMG + (RG + q) * C::PG + 8 * c4 + 2 * (C::GXH + C::BX);
       st4(o, make_float4(gray_of(R0.x, G0.x, B0.x), gray_of(R1.x, G1.x, B1.x), gray_of(R0.y, G0.y, B0.y),
                          gray_of(R1.y, G1.y, B1.y)));
       st4(o + 4, make_float4(gray_of(R0.z, G0.z, B0.z), gray_of(R1.z, G1.z, B1.z), gray_of(R0.w, G0.w, B0.w),
@@ -261,11 +311,11 @@ st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP
         const int c2 = it % C2, r = it / C2;
         const int gy = ry0 + r, gx = x0 + 2 * c2;
         if (gy < y0 || gy >= y1 || gx >= W) continue;
-        const float* ps = sRaw + r * C::GW + C::GXH + 2 * c2;
+        const float* ps = sRaw + r * C::BW - C::BX + 2 * c2;
         float acc = 0.f;
 #pragma unroll
         for (int ch = 0; ch < 3; ++ch) {
-          const float2 u = ld2(ps + ch * C::RS * C::GW), v = ld2(ps + C::RAW_IMG + ch * C::RS * C::GW);
+          const float2 u = ld2(ps + ch * C::RS * C::BW), v = ld2(ps + C::RAW_IMG + ch * C::RS * C::BW);
           const float d0 = u.x - v.x, d1 = u.y - v.y;
           acc = fmaf(d0, d0, acc);
           acc = fmaf(d1, d1, acc);
@@ -282,11 +332,11 @@ st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP
     // Block 0 (its RG carried row pairs and its 8 new ones: image rows hb(0) - RG .. hb(0) + RG + 15) comes straight
     // from global memory while the box of block 1 is in flight; item = row pair x 4 columns of BOTH images, spread
     // over ALL threads of the CTA (the consumers have nothing else to do yet).
-    constexpr int C4 = C::GW / 4;
+    constexpr int C4 = C::BW / 4;
     for (int it = tid; it < C::GP * C4; it += C::NT) {
       const int c4 = it % C4, pr = it / C4;
-      const int gx = x0 - C::GXH + 4 * c4;
-      const bool xin = gx >= 0 && gx < W;  // x0 - GXH and W are multiples of 4: a float4 is all-in or all-out
+      const int gx = x0 + C::BX + 4 * c4;
+      const bool xin = gx >= 0 && gx < W;  // x0 + BX and W are multiples of 4: a float4 is all-in or all-out
       float4 v[2][2][3];                   // [image][row of the pair][channel]
       bool ok[2];
 #pragma unroll
@@ -305,7 +355,7 @@ st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP
 #pragma unroll
       for (int img = 0; img < 2; ++img) {
         const float4 *a0 = v[img][0], *a1 = v[img][1];
-        float* o = sGray + img * C::GRAY_IMG + pr * C::PG + 8 * c4;
+        float* o = sGray + img * C::GRAY_IMG + pr * C::PG + 8 * c4 + 2 * (C::GXH + C::BX);
         st4(o, make_float4(gray_of(a0[0].x, a0[1].x, a0[2].x), gray_of(a1[0].x, a1[1].x, a1[2].x),
                            gray_of(a0[0].y, a0[1].y, a0[2].y), gray_of(a1[0].y, a1[1].y, a1[2].y)));
         st4(o + 4, make_float4(gray_of(a0[0].z, a0[1].z, a0[2].z), gray_of(a1[0].z, a1[1].z, a1[2].z),
@@ -334,6 +384,23 @@ st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP
         }
       }
     }
+    if constexpr (C::XFULL) {
+      // the zero columns of the edge windows, which nothing else writes: gray columns -GXH .. -1 and TW .. TW+GXH-1
+      // of every gray row pair (both buffers, both images), Ix / Iy columns -RK .. -1 and TW .. TW+RK-1
+      constexpr int GZ = C::GXH / 2, DZ = RK / 2;  // float4 per row pair and side
+      constexpr int NG = 4 * C::GP * 2 * GZ, ND = 4 * NQ * 2 * DZ;
+      for (int it = tid; it < NG + ND; it += C::NT) {
+        float* o;
+        if (it < NG) {
+          const int r = it / (2 * GZ), u = it % (2 * GZ);
+          o = sGray + r * C::PG + (u < GZ ? 4 * u : 2 * (C::GXH + C::TW) + 4 * (u - GZ));
+        } else {
+          const int r = (it - NG) / (2 * DZ), u = (it - NG) % (2 * DZ);
+          o = sD + r * C::PD + (u < DZ ? 4 * u : 2 * (RK + C::TW) + 4 * (u - DZ));
+        }
+        st4(o, make_float4(0.f, 0.f, 0.f, 0.f));
+      }
+    }
   }
   __syncthreads();
 
@@ -355,9 +422,19 @@ st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP
     for (int k = 0; k <= NB; ++k) {
       {
         // gradients of block k: Ix, Iy on 8 row pairs x DW columns of both images; zero outside the image (the
-        // reference zero-pads the PRODUCTS, utils.py:225-230); strip-interior items save them for the backward
-        const int q = tid & 7, rest = tid >> 3;
-        const int seg = rest % C::NSEGB, img = rest / C::NSEGB;
+        // reference zero-pads the PRODUCTS, utils.py:225-230); strip-interior items save them for the backward.
+        // Crop layout: the image columns only (segments 1 .. NSEGH of the DW columns), on the first NH producers.
+        if (!C::XFULL || tid < C::NH) {
+        int q, seg, img;
+        if constexpr (C::XFULL) {
+          C::xitem(tid, q, img, seg);
+          seg += RK / 8;
+        } else {
+          q = tid & 7;
+          const int rest = tid >> 3;
+          seg = rest % C::NSEGB;
+          img = rest / C::NSEGB;
+        }
         const int gy = hb(k) + 2 * q, gx0 = x0 - RK + 8 * seg;
         float2 Ix[8], Iy[8];
         if (gy + 1 >= 0 && gy < H && gx0 + 7 >= 0 && gx0 < W && MARCH_ON(3)) {
@@ -384,6 +461,7 @@ st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP
         for (int j = 0; j < 8; j += 2) {
           st4(o0 + 2 * j, make_float4(Ix[j].x, Ix[j].y, Ix[j + 1].x, Ix[j + 1].y));
           st4(o1 + 2 * j, make_float4(Iy[j].x, Iy[j].y, Iy[j + 1].x, Iy[j + 1].y));
+        }
         }
         MSTAMP(tid == 0, 2 + 6 * k);  // gradients done
         // gray rows of block k+1 into the other gray buffer (its box was requested one half-step ago)
@@ -467,8 +545,15 @@ st_forward_march_kernel(const __grid_constant__ StMarchParamsT<C::RG, C::RK, MAP
         // products + horizontal rho-pass of block k -> ring row pairs 8*(k&1) ..; item = image x row pair x 8 columns.
         // Scatter form: window column j contributes k[j - o] to output column o, so Ix, Iy are read once.
         if (tid < C::NH && MARCH_ON(2)) {
-          const int q = tid & 7, rest = tid >> 3;
-          const int seg = rest % C::NSEGH, img = rest / C::NSEGH;
+          int q, seg, img;
+          if constexpr (C::XFULL) {
+            C::xitem(tid, q, img, seg);
+          } else {
+            q = tid & 7;
+            const int rest = tid >> 3;
+            seg = rest % C::NSEGH;
+            img = rest / C::NSEGH;
+          }
           const float* pix = sD + (img * 2) * C::D_PLANE + q * C::PD + 2 * (8 * seg);
           const float* piy = pix + C::D_PLANE;
           float2 acc[3][8];

@@ -3,6 +3,8 @@
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -DSRST_MARCH_ABL -DMB_TW=112 \
 //        -I srgan_st_b200/csrc -o tools/_bin/march_bench_112 tools/march_bench.cu -lcuda
 //   tools/_bin/march_bench_112 B H W [chunk_blocks] [mask ...]
+// -DMB_XFULL=1 (with MB_TW=96): the crop layout (images no wider than 96 columns).  -DSRST_MARCH_STAMPS and MB_STAMPS=1
+// in the environment: phase time stamps of one launch, medians over all CTAs and per chunk index.
 // mask bits: 1 chain, 2 vertical, 4 horizontal, 8 gradient, 16 convert, 32 ds stores, 64 ixy stores (set = skipped)
 #include <cstdio>
 #include <cstdlib>
@@ -16,7 +18,10 @@ using namespace srst;
 #ifndef MB_CR
 #define MB_CR 8
 #endif
-using C = StMarchCfg<MB_TW, 2, 8, MB_CR>;
+#ifndef MB_XFULL
+#define MB_XFULL 0
+#endif
+using C = StMarchCfg<MB_TW, 2, 8, MB_CR, MB_XFULL != 0>;
 static bool make_map(CUtensorMap* map, const float* base, long long planes, int rows, int cols, int bw, int bh, int bp) {
   const cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)planes};
   const cuuint64_t strides[2] = {(cuuint64_t)cols * 4, (cuuint64_t)cols * rows * 4};
@@ -29,6 +34,7 @@ static bool make_map(CUtensorMap* map, const float* base, long long planes, int 
 int main(int argc, char** argv) {
   const int B = argc > 1 ? atoi(argv[1]) : 1, H = argc > 2 ? atoi(argv[2]) : 1356, W = argc > 3 ? atoi(argv[3]) : 2040;
   int cb_forced = argc > 4 ? atoi(argv[4]) : 0;
+  if (C::XFULL && W > C::TW) { printf("the crop layout needs W <= %d\n", C::TW); return 1; }
   const size_t n = (size_t)B * 3 * H * W;
   const int NPOOL = (int)(400e6 / (2.0 * n * 4)) + 2;  // > 2x L2 of inputs
   std::vector<float*> sr(NPOOL), hr(NPOOL);
@@ -46,7 +52,7 @@ int main(int argc, char** argv) {
   int sms = 148; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0);
   for (int p = 0; p < NPOOL; ++p) {
     auto& MP = MPs[p];
-    if (!make_map(&MP.sr_map, sr[p], (long long)B * 3, H, W, C::GW, C::RS, 3) || !make_map(&MP.hr_map, hr[p], (long long)B * 3, H, W, C::GW, C::RS, 3)) { printf("map failed\n"); return 1; }
+    if (!make_map(&MP.sr_map, sr[p], (long long)B * 3, H, W, C::BW, C::RS, 3) || !make_map(&MP.hr_map, hr[p], (long long)B * 3, H, W, C::BW, C::RS, 3)) { printf("map failed\n"); return 1; }
     auto& F = MP.F;
     F.sr = sr[p]; F.hr = hr[p]; F.ds_sr = ds; F.ds_hr = nullptr; F.ixy_sr = ixy; F.ixy_hr = nullptr;
     F.ticket = (unsigned*)ws; F.partials = ws + 4; F.px_partials = nullptr; F.loss_out = loss;
@@ -72,7 +78,7 @@ int main(int argc, char** argv) {
   auto kern = st_forward_march_kernel<C, false, false>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES);
   const int grid = B * MPs[0].nstrips * MPs[0].nchunks;
-  printf("TW=%d B=%d %dx%d: grid %d (strips %d, chunks %d of %d blocks), %d threads, %zu B smem\n", C::TW, B, H, W, grid,
+  printf("TW=%d%s B=%d %dx%d: grid %d (strips %d, chunks %d of %d blocks), %d threads, %zu B smem\n", C::TW, C::XFULL ? " (crop layout)" : "", B, H, W, grid,
          MPs[0].nstrips, MPs[0].nchunks, MPs[0].chunk_blocks, C::NT, C::SMEM_BYTES);
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   const int iters = 40;
@@ -102,12 +108,29 @@ int main(int argc, char** argv) {
     std::vector<long long> hst((size_t)grid * 128);
     cudaMemcpy(hst.data(), d, hst.size() * 8, cudaMemcpyDeviceToHost);
     long long t0 = 0; for (int c = 0; c < grid; ++c) if (hst[(size_t)c * 128] && (!t0 || hst[(size_t)c * 128] < t0)) t0 = hst[(size_t)c * 128];
+    // CTA c works on chunk (c / nstrips) % nchunks of its strip (the grid is image-major, then chunk, then strip)
+    const int nch = MPs[1].nchunks, nst = MPs[1].nstrips;
     for (int sl = 0; sl < 128; ++sl) {
       std::vector<double> v;
-      for (int c = 0; c < grid; ++c) if (hst[(size_t)c * 128 + sl]) v.push_back((hst[(size_t)c * 128 + sl] - t0) * 1e-3);
+      std::vector<std::vector<double>> vc(nch);
+      for (int c = 0; c < grid; ++c)
+        if (hst[(size_t)c * 128 + sl]) {
+          const double t = (hst[(size_t)c * 128 + sl] - t0) * 1e-3;
+          v.push_back(t);
+          vc[(c / nst) % nch].push_back(t);
+        }
       if (v.empty()) continue;
       std::sort(v.begin(), v.end());
-      printf("  %s slot %2d: median %7.2f us  min %7.2f  max %7.2f  (n=%zu)\n", sl < 64 ? "P" : "C", sl & 63, v[v.size() / 2], v.front(), v.back(), v.size());
+      printf("  %s slot %2d: median %7.2f us  min %7.2f  max %7.2f  (n=%zu)", sl < 64 ? "P" : "C", sl & 63, v[v.size() / 2], v.front(), v.back(), v.size());
+      if (nch > 1 && nch <= 8) {
+        printf("  per chunk:");
+        for (auto& u : vc) {
+          if (u.empty()) { printf("      -"); continue; }
+          std::sort(u.begin(), u.end());
+          printf(" %7.2f", u[u.size() / 2]);
+        }
+      }
+      printf("\n");
     }
   }
 #endif
